@@ -20,6 +20,14 @@ Output: ONE JSON line on rank 0.
                MSD forward/backward, two AdamW updates; gradient all-reduce over NCCL when N > 1)
 
 --workload train makes the training step the primary metric of the line (same keys).
+
+--dump-outputs DIR writes, after the timed steps, what the primary metric's last timed step returned to its caller as
+DIR/<name>.npy (float32; rank 0's shard): the Generator workloads' waveform `y_g_hat`; with --workload train the
+training step's `y_g_hat` and losses.  An array above DUMP_ARRAY_BYTES keeps a fixed, seeded selection of whole batch
+items (DUMP_SEED).  The inputs depend only on the arguments, so two builds can be compared output for output: the
+Generator's waveform repeats bit for bit, while the training step's reductions are not bit-reproducible and its
+outputs drift apart over the warm-up + --steps AdamW updates (two runs of one build on a B200, 10 timed steps: losses
+within 0.6 %, waveform within 3e-3 absolute).
 """
 from __future__ import annotations
 
@@ -58,6 +66,29 @@ def shard_range(n_items: int, rank: int, world: int):
     base, rem = divmod(n_items, world)
     lo = rank * base + min(rank, rem)
     return lo, lo + base + (1 if rank < rem else 0)
+
+
+DUMP_ARRAY_BYTES = 16 << 20   # the default line's waveform is 64 MiB: 16 of its 64 items
+DUMP_SEED = 0
+
+
+def dump_sample(t: torch.Tensor) -> torch.Tensor:
+    """t as float32 on the host; above DUMP_ARRAY_BYTES only a seeded choice of whole items along dim 0, in order."""
+    t = t.detach().float()
+    if t.dim() > 0 and t.numel() * 4 > DUMP_ARRAY_BYTES:
+        keep = max(1, DUMP_ARRAY_BYTES // (t[0].numel() * 4))
+        items = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(DUMP_SEED))[:keep].sort().values
+        t = t[items.to(t.device)]
+    return t.cpu()
+
+
+def write_outputs(path: str, arrays) -> None:
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), t.numpy())
+    total = sum(t.numel() * 4 for t in arrays.values())
+    print(f"bench.py: wrote {len(arrays)} arrays ({total / 2**20:.1f} MiB) to {path}", file=sys.stderr)
 
 
 def _dist_on() -> bool:
@@ -370,8 +401,9 @@ def measure_mel(dev, steps: int):
                          "frac": gbs / peaks["hbm_gbs"], "algorithmic_bytes_per_frame": 1344, "traffic": None}}
 
 
-def measure_train(dev, rank, world, steps: int, warmup: int, batch: int = TRAIN["batch"]):
-    """Time the full training step.  Returns a dict with device-resident and end-to-end numbers (max over ranks)."""
+def measure_train(dev, rank, world, steps: int, warmup: int, batch: int = TRAIN["batch"], keep_outputs: bool = False):
+    """Time the full training step.  Returns a dict with device-resident and end-to-end numbers (max over ranks);
+    keep_outputs: also what the last timed step returned (dump_sample of each tensor) under "outputs"."""
     import hifigan_b200 as H
     from hifigan_b200 import _lib
     from hifigan_b200.configs import load_config
@@ -411,6 +443,8 @@ def measure_train(dev, rank, world, steps: int, warmup: int, batch: int = TRAIN[
     barrier()
     ms = e0.elapsed_time(e1) / steps
     launches = _lib.launch_count() - n0
+    # the graph's static outputs: copied before the end-to-end steps below replay into them
+    outputs = {k: dump_sample(v) for k, v in out.items()} if keep_outputs else None
     # end to end: the step's three inputs come from pinned host memory, the logged losses go back to the host
     host_loss = torch.empty(2, dtype=torch.float32).pin_memory()
     f0e, f1e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -445,7 +479,7 @@ def measure_train(dev, rank, world, steps: int, warmup: int, batch: int = TRAIN[
             "segments": sum_over_ranks(float(batch)), "launches_per_step": per_step, "graphed": graphed,
             "h2d": (host_x.numel() + host_y.numel() + host_ymel.numel()) * 4, "d2h": 8, "warmup": n_warm,
             "slice_order": list(ts.D.order),
-            "losses": [float(v) for v in host_loss.tolist()]}
+            "losses": [float(v) for v in host_loss.tolist()], "outputs": outputs}
 
 
 def train_summary(r, world):
@@ -473,10 +507,13 @@ def run_train(args, rank, world, local_rank):
     dev = torch.device("cuda", local_rank)
     sampler = ClockSampler(local_rank)
     sampler.start()
-    r = measure_train(dev, rank, world, args.steps, args.warmup, args.per_gpu_batch or TRAIN["batch"])
+    r = measure_train(dev, rank, world, args.steps, args.warmup, args.per_gpu_batch or TRAIN["batch"],
+                      keep_outputs=bool(args.dump_outputs) and rank == 0)
     clocks = sampler.stop()
     if rank != 0:
         return
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, r["outputs"])
     t = train_summary(r, world)
     line = {"metric": t["metric"], "value": t["value"], "unit": t["unit"], "n_gpus": world, "steps": args.steps,
             "warmup": r["warmup"], "ms_per_step": t["ms_per_step"], "higher_is_better": True,
@@ -572,11 +609,13 @@ def run_ours(args, rank, world, local_rank):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(args.steps):
-            eng.forward(x, time_convs=True)
+            y = eng.forward(x, time_convs=True)
             conv_ms.append(eng.last_conv_events)
         e1.record()
         barrier()
         launches = _lib.launch_count() - launches0
+        # the engine-owned buffer: copied before the end-to-end calls below write it again
+        outputs = {"y_g_hat": dump_sample(y)} if args.dump_outputs and rank == 0 else None
         ms = e0.elapsed_time(e1) / args.steps
         conv_ms = sum(a.elapsed_time(b) for a, b in conv_ms) / args.steps
         # ---------------- end-to-end through the public API with host buffers
@@ -610,11 +649,13 @@ def run_ours(args, rank, world, local_rank):
         G._drop_engines()
         torch.cuda.empty_cache()
         try:
-            train = train_summary(measure_train(dev, rank, world, max(5, min(args.steps, 20)), 3), world)
+            train = train_summary(measure_train(dev, rank, world, args.steps, args.warmup), world)
         except Exception as e:  # noqa: BLE001  (the headline number must survive a failure of the secondary one)
             train = {"error": f"{type(e).__name__}: {e}"}
     if rank != 0:
         return
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
     peaks = measured_peaks()
     n_conv = launches // args.steps - 2  # every launch of a step except ncl_to_nlc and conv_post
     conv_flops = samples * (FLOP_PER_SAMPLE[ver] - CONV_POST_FLOP_PER_SAMPLE[ver])
@@ -669,7 +710,13 @@ def main():
     ap.add_argument("--per-gpu-batch", type=int, default=0,
                     help="--workload train: segments per GPU (default 16 = BASELINE configs[2]; configs[3]'s global "
                          "batch 128 is 64 / 32 / 16 at 2 / 4 / 8 GPUs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step returned as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what --impl ours computed")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

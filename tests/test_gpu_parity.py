@@ -774,3 +774,31 @@ def test_randomised_shapes_sweep():
                          text=True, cwd=root, timeout=900)
     assert out.returncode == 0, out.stdout[-3000:] + out.stderr[-2000:]
     assert "failures: 0" in out.stdout
+
+
+def test_bench_dump_outputs_is_what_the_generator_returns(H, tmp_path):
+    """`bench.py --dump-outputs DIR` after `--steps 2` of the cfg1 workload (V1, 1 x 80 x 256 mel from seed 0, weights
+    from seed 1234, weight_norm folded) writes the waveform a caller of Generator gets for the same input."""
+    import json
+    import subprocess
+    import sys
+    from hifigan_b200.configs import load_config
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dump = tmp_path / "dump"
+    cmd = [sys.executable, os.path.join(root, "bench.py"), "--workload", "cfg1", "--steps", "2", "--warmup", "1",
+           "--no-cpu-baseline", "--dump-outputs", str(dump)]
+    out = subprocess.run(cmd, capture_output=True, text=True, cwd=root, timeout=600)
+    assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
+    lines = [l for l in out.stdout.splitlines() if l.startswith("{")]
+    assert len(lines) == 1 and json.loads(lines[0])["steps"] == 2
+    assert sorted(os.listdir(dump)) == ["y_g_hat.npy"]
+    got = np.load(dump / "y_g_hat.npy")
+    torch.manual_seed(1234)
+    G = H.Generator(load_config("v1")).cuda().eval()
+    G.remove_weight_norm()
+    torch.manual_seed(0)
+    x = torch.randn(1, 80, 256)
+    with torch.no_grad():
+        ref = G(x.cuda()).cpu().numpy()
+    assert got.dtype == np.float32 and got.shape == ref.shape == (1, 1, 65536)
+    assert np.abs(got - ref).max() <= 1e-6

@@ -236,7 +236,7 @@ def test_segment_sampler_fine_tuning_draw_rule_matches_reference():
     assert picks == want
 
 
-def test_reference_style_top_level_imports():
+def test_reference_style_top_level_imports(tmp_path):
     """`src/`-on-PYTHONPATH spelling of the reference (inference.py:9-11) resolves to this package."""
     import subprocess
     import sys
@@ -244,7 +244,7 @@ def test_reference_style_top_level_imports():
             "from models import Generator; from utils import get_padding; "
             "import hifigan_b200; assert Generator is hifigan_b200.Generator; print('ok')")
     env = dict(os.environ, PYTHONPATH=os.path.join(ROOT, "hifi-gan_b200", "compat") + os.pathsep + ROOT)
-    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, cwd="/tmp")
+    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, cwd=tmp_path)
     assert out.returncode == 0 and out.stdout.strip().endswith("ok"), out.stderr
 
 
@@ -375,6 +375,25 @@ def test_bench_reference_arm_contract(workload):
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     other = subprocess.run(cmd + ["--gpus", "2"], capture_output=True, text=True, cwd=ROOT, timeout=600, env=env)
     assert other.returncode == 0 and not [l for l in other.stdout.splitlines() if l.startswith("{")]
+
+
+def test_bench_dump_sample_is_seeded_and_bounded(tmp_path):
+    """`bench.py --dump-outputs`: an output above DUMP_ARRAY_BYTES keeps the same whole items, in batch order, on every
+    call (the default line's 64 x 262 144-sample waveform -> 16 items); smaller outputs and scalars are kept whole;
+    the files hold exactly what was kept, as float32."""
+    import bench
+    y = torch.randn(64, 1, 262144)
+    a, b = bench.dump_sample(y), bench.dump_sample(y.clone())
+    assert a.shape == (16, 1, 262144) and a.dtype == torch.float32 and torch.equal(a, b)
+    items = [i for i in range(64) if any(torch.equal(y[i], r) for r in a)]
+    assert len(items) == 16 and torch.equal(y[items], a)
+    small, loss = torch.randn(16, 1, 8192, dtype=torch.float64), torch.tensor(2.5)
+    assert torch.equal(bench.dump_sample(small), small.float()) and bench.dump_sample(loss).shape == ()
+    bench.write_outputs(str(tmp_path / "out"), {"y_g_hat": a, "loss": bench.dump_sample(loss)})
+    assert sorted(os.listdir(tmp_path / "out")) == ["loss.npy", "y_g_hat.npy"]
+    got = np.load(tmp_path / "out" / "y_g_hat.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, a.numpy())
+    assert np.load(tmp_path / "out" / "loss.npy") == np.float32(2.5)
 
 
 def test_epoch_learning_rate_matches_torch_exponential_lr():
