@@ -19,16 +19,25 @@ parameter gradients.
 """
 from __future__ import annotations
 
+import itertools
 from typing import List, Optional
 
 import torch
 
 from . import _lib
-from .models import _stream
+from .models import _avgpool, _loss_mean, _stream
 
 
-def _needs_autograd(x: torch.Tensor, module: torch.nn.Module) -> bool:
-    return torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in module.parameters()))
+def _engine(module: torch.nn.Module, device, build):
+    """The module's autograd-path engine (`build()` makes one).  Its job tables hold raw pointers to the parameters
+    and buffers, so it is rebuilt whenever their storage moved: `.to()`, `p.data = ...`, FlatParams re-pointing them."""
+    key = (device,) + tuple(t.data_ptr() for t in itertools.chain(module.parameters(), module.buffers()))
+    eng = module.__dict__.get("_hg_autograd")
+    if eng is None or eng.storage_key != key:
+        eng = build()
+        eng.storage_key = key
+        module.__dict__["_hg_autograd"] = eng
+    return eng
 
 
 def _grads_out(flat, params, needs) -> list:
@@ -43,11 +52,8 @@ def _grads_out(flat, params, needs) -> list:
 class _GeneratorFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, gen, *params):
-        tr = gen.__dict__.get("_hg_autograd")
-        if tr is None or tr.device != x.device:
-            from .train import GeneratorTrainer
-            tr = GeneratorTrainer(gen, x.device, bind=False)
-            gen.__dict__["_hg_autograd"] = tr
+        from .train import GeneratorTrainer
+        tr = _engine(gen, x.device, lambda: GeneratorTrainer(gen, x.device, bind=False))
         y = tr.forward(x.detach())
         tr.call_id = getattr(tr, "call_id", 0) + 1
         ctx.tr, ctx.call_id, ctx.in_shape = tr, tr.call_id, tuple(x.shape)
@@ -83,50 +89,53 @@ _SLOTS = 4
 
 
 class _DiscEngine:
-    """Per-module state of the autograd path: the sub-discriminator trainer (kernel sequences, workspaces) and a
-    private flat gradient buffer."""
+    """Per-module state of a DiscriminatorP / DiscriminatorS: the sub-discriminator trainer (kernel sequences,
+    workspaces), a private flat gradient buffer and the ring of call slots."""
 
     def __init__(self, disc, device):
         from .train import FlatParams, _SubDiscTrainer
-        self.device = device
         self.flat = FlatParams(disc, device, bind=False)
-        self.sd = _SubDiscTrainer(disc, device)
+        self.sd = _SubDiscTrainer(disc, device, self.flat)
         self.next_slot = 0
         self.slot_call = [0] * _SLOTS
         self.calls = 0
 
 
+def _disc_run(disc, x: torch.Tensor, differentiable: bool):
+    """One call of a sub-discriminator: claim the next ring slot, run the forward, export the feature maps and
+    assemble the logits.  Returns (feature maps fp32 [B,C,H,p] + logits [B,1,H,p],
+    (engine, slot, call id, G, W, x2d))."""
+    eng = _engine(disc, x.device, lambda: _DiscEngine(disc, x.device))
+    sd = eng.sd
+    L = _lib.lib()
+    b, c, t = x.shape
+    if c != 1:
+        raise ValueError("discriminators take [B,1,T] audio")
+    x2d = x.detach().reshape(b, t).contiguous().float()
+    slot = eng.next_slot
+    eng.next_slot = (slot + 1) % _SLOTS
+    eng.calls += 1
+    eng.slot_call[slot] = eng.calls
+    G, W = sd.forward_single(x2d, slot, dgrad=differentiable)
+    period, st = sd.period, _stream()
+    outs = []
+    for (h, rows, ch), act in zip(G["geo"], G["act"]):
+        f = torch.empty(b, ch, h, period, dtype=torch.float32, device=x.device)
+        _lib.check(L.hg_disc_export_fmap(act.data_ptr(), b, period, h, rows, ch, f.data_ptr(), st),
+                   "hg_disc_export_fmap")
+        outs.append(f)
+    h_last = G["geo"][-1][0]
+    post = G["logit"].view(b, period, h_last).permute(0, 2, 1).contiguous().unsqueeze(1)     # [B,1,H,p]
+    outs.append(post)
+    return tuple(outs), (eng, slot, eng.calls, G, W, x2d)
+
+
 class _DiscFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, disc, *params):
-        eng = disc.__dict__.get("_hg_autograd")
-        if eng is None or eng.device != x.device:
-            eng = _DiscEngine(disc, x.device)
-            disc.__dict__["_hg_autograd"] = eng
-        sd = eng.sd
-        L = _lib.lib()
-        b, c, t = x.shape
-        if c != 1:
-            raise ValueError("discriminators take [B,1,T] audio")
-        x2d = x.detach().reshape(b, t).contiguous().float()
-        slot = eng.next_slot
-        eng.next_slot = (slot + 1) % _SLOTS
-        eng.calls += 1
-        eng.slot_call[slot] = eng.calls
-        G, W = sd.forward_single(x2d, slot)
-        period, st = sd.period, _stream()
-        outs = []
-        for (h, rows, ch), act in zip(G["geo"], G["act"]):
-            f = torch.empty(b, ch, h, period, dtype=torch.float32, device=x.device)
-            _lib.check(L.hg_disc_export_fmap(act.data_ptr(), b, period, h, rows, ch, f.data_ptr(), st),
-                       "hg_disc_export_fmap")
-            outs.append(f)
-        h_last = G["geo"][-1][0]
-        post = G["logit"].view(b, period, h_last).permute(0, 2, 1).contiguous().unsqueeze(1)     # [B,1,H,p]
-        outs.append(post)
-        ctx.eng, ctx.slot, ctx.call, ctx.G, ctx.W, ctx.x2d = eng, slot, eng.calls, G, W, x2d
+        outs, (ctx.eng, ctx.slot, ctx.call, ctx.G, ctx.W, ctx.x2d) = _disc_run(disc, x, True)
         ctx.set_materialize_grads(False)
-        return tuple(outs)
+        return outs
 
     @staticmethod
     def backward(ctx, *douts):
@@ -169,9 +178,10 @@ class _DiscFn(torch.autograd.Function):
         return (None if dy is None else dy.view(b, 1, t), None) + tuple(grads)
 
 
-def disc_forward(disc, x: torch.Tensor):
-    """(flattened logits, feature maps fp32 [B,C,H,p]) of one DiscriminatorP / DiscriminatorS call, differentiable"""
-    outs = _DiscFn.apply(x, disc, *disc.parameters())
+def disc_forward(disc, x: torch.Tensor, differentiable: bool):
+    """(flattened logits, feature maps fp32 [B,C,H,p]) of one DiscriminatorP / DiscriminatorS call; through autograd
+    when `differentiable`, otherwise the same forward without the data-gradient banks"""
+    outs = _DiscFn.apply(x, disc, *disc.parameters()) if differentiable else _disc_run(disc, x, False)[0]
     fmap = list(outs)
     return torch.flatten(fmap[-1], 1, -1), fmap
 
@@ -181,13 +191,8 @@ class _AvgPoolFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x):
-        b, c, t = x.shape
-        xin = x.detach().reshape(b * c, t).contiguous().float()
-        out = torch.empty(b * c, t // 2 + 1, dtype=torch.float32, device=x.device)
-        _lib.check(_lib.lib().hg_avgpool_4_2_2_fwd(xin.data_ptr(), b * c, t, out.data_ptr(), _stream()),
-                   "hg_avgpool_4_2_2_fwd")
-        ctx.shape = (b, c, t)
-        return out.view(b, c, -1)
+        ctx.shape = tuple(x.shape)
+        return _avgpool(x)
 
     @staticmethod
     def backward(ctx, dout):
@@ -211,12 +216,9 @@ class _MeanFn(torch.autograd.Function):
     def forward(ctx, a, b, mode, c):
         a32 = a.detach().contiguous().float()
         b32 = None if b is None else b.detach().contiguous().float()
-        acc = torch.zeros(1, dtype=torch.float32, device=a.device)
-        _lib.check(_lib.lib().hg_loss_sum(a32.data_ptr(), 0 if b32 is None else b32.data_ptr(), a32.numel(), mode, c,
-                                          acc.data_ptr(), _stream()), "hg_loss_sum")
         ctx.a, ctx.b, ctx.mode, ctx.c = a32, b32, mode, c
         ctx.a_shape, ctx.b_shape = a.shape, (None if b is None else b.shape)
-        return acc[0] / a32.numel()
+        return _loss_mean(a32, b32, mode, c)
 
     @staticmethod
     def backward(ctx, dout):

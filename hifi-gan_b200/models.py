@@ -55,6 +55,11 @@ def _require_cuda(x: torch.Tensor, what: str) -> None:
         raise RuntimeError(f"{what}: hifigan_b200 has no CPU path; move the tensor to a B200 (got {x.device})")
 
 
+def _wants_grad(x: torch.Tensor, module: nn.Module) -> bool:
+    """whether torch autograd records this call of `module` on `x`"""
+    return torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in module.parameters()))
+
+
 def _g_v(m: nn.Module) -> Tuple[Optional[torch.Tensor], torch.Tensor]:
     """(g, v) while weight_norm is attached, (None, weight) after remove_weight_norm."""
     if hasattr(m, "weight_g"):
@@ -265,7 +270,7 @@ class _StandaloneBlockMixin:
 
     def forward(self, x: torch.Tensor) -> torch.Tensor:
         _require_cuda(x, type(self).__name__)
-        if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters())):
+        if _wants_grad(x, self):
             raise NotImplementedError(f"{type(self).__name__} on its own is an inference surface (call it under "
                                       "torch.no_grad()); it is differentiable as part of Generator")
         L = _lib.lib()
@@ -681,7 +686,7 @@ class Generator(torch.nn.Module):
         if x.dim() != 3 or x.shape[1] != self.conv_pre.in_channels:
             raise ValueError(f"expected [B,{self.conv_pre.in_channels},F], got {tuple(x.shape)}")
         if lengths is not None:
-            if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters())):
+            if _wants_grad(x, self):
                 raise NotImplementedError("ragged batches are an inference feature: call under torch.no_grad()")
             ln = torch.as_tensor(lengths).to(device=x.device, dtype=torch.int32).contiguous()
             if ln.shape != (x.shape[0],) or int(ln.min()) < 1 or int(ln.max()) > x.shape[2]:
@@ -689,7 +694,7 @@ class Generator(torch.nn.Module):
             # frames past an item's end must read as zero padding at conv_pre's input
             mask = torch.arange(x.shape[2], device=x.device)[None, None, :] < ln[:, None, None]
             return self._engine(x.device).forward(x * mask, lengths=ln).clone()
-        if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters())):
+        if _wants_grad(x, self):
             # differentiable call (an UPSTREAM-style `loss.backward()` loop): one autograd.Function over the training
             # forward (every conv input kept) and the hand-written backward — autograd.py
             from . import autograd
@@ -721,32 +726,10 @@ class Generator(torch.nn.Module):
 # forward pass runs on libhifigan_b200.so: Cin = 1 and Cout = 1 ends on CUDA-core kernels (hg_disc_*), every
 # wide layer on the tcgen05 implicit-GEMM kernel (hg_conv1d_general_fwd) — strided layers through residue
 # boxes, grouped layers as per-group N tiles (narrow groups merged into block-diagonal 32-wide ones).
-# Activations live as bf16 [B*period][rows][C]: one independent 1-D sequence per period column.
+# Activations live as bf16 [B*period][rows][C]: one independent 1-D sequence per period column.  Every call, with or
+# without autograd recording, runs on the module's engine (autograd.py: _SubDiscTrainer.forward_single), so a
+# discriminator computes the same numbers in both modes.
 # --------------------------------------------------------------------------------------------------
-def _effective_weight(m: nn.Module) -> torch.Tensor:
-    """fp32 conv weight of a weight_norm / spectral_norm / plain module, computed on the module's device.
-    weight_norm: g * v / ||v|| (dim 0).  spectral_norm: W / sigma with ONE power iteration per call in
-    train mode, updating the `weight_u` / `weight_v` buffers in place exactly like
-    torch.nn.utils.spectral_norm (eps 1e-12) — the reference relies on that call-by-call behaviour
-    (SURVEY.md Appendix B.11); eval mode uses the stored buffers.
-    (Weight preparation is a handful of tiny device ops per layer, not the conv hot path.)"""
-    with torch.no_grad():
-        if hasattr(m, "weight_g"):
-            v, g = m.weight_v, m.weight_g
-            dims = tuple(range(1, v.dim()))
-            return (v * (g / v.pow(2).sum(dim=dims, keepdim=True).sqrt())).float()
-        if hasattr(m, "weight_orig"):
-            w = m.weight_orig
-            wm = w.flatten(1)
-            u, v = m.weight_u, m.weight_v
-            if m.training:
-                v.copy_(torch.nn.functional.normalize(torch.mv(wm.t(), u), dim=0, eps=1e-12))
-                u.copy_(torch.nn.functional.normalize(torch.mv(wm, v), dim=0, eps=1e-12))
-            sigma = torch.dot(u, torch.mv(wm, v))
-            return (w / sigma).float()
-        return m.weight.float()
-
-
 def _round_up(n: int, m: int) -> int:
     return (n + m - 1) // m * m
 
@@ -775,112 +758,26 @@ class _DiscLayer:
         self.order = list(order)
 
     def pack(self, w: torch.Tensor) -> torch.Tensor:
-        """w fp32 [cout][cin/groups][k] -> bf16 [k (kernel order)][cout][cin_tile]."""
-        cout, cin_g, k = w.shape
-        w = w[:, :, self.order]
-        if self.groups > 1 and self.merge > 1:
-            full = w.new_zeros(cout, self.cin_tile, k)
-            cout_g = cout // self.groups
-            slot = (torch.arange(cout, device=w.device) // cout_g) % self.merge   # position inside the merged tile
-            idx = slot.unsqueeze(1) * cin_g + torch.arange(cin_g, device=w.device).unsqueeze(0)  # [cout][cin_g]
-            full.scatter_(1, idx.unsqueeze(2).expand(-1, -1, k), w)
-            w = full
-        return w.permute(2, 0, 1).contiguous().to(torch.bfloat16)
+        """w fp32 contiguous [cout][cin/groups][k] on the device -> bf16 [k (kernel order)][cout][cin_tile]
+        (hg_pack_disc_weight)."""
+        out = torch.empty(self.k, self.cout, self.cin_tile, dtype=torch.bfloat16, device=w.device)
+        _lib.check(_lib.lib().hg_pack_disc_weight(w.data_ptr(), self.cout, self.cin, self.groups, self.merge, self.k,
+                                                  self.stride, self.pad, out.data_ptr(), 0, _stream()),
+                   "hg_pack_disc_weight")
+        return out
 
 
-def _param_key(m: nn.Module):
-    ts = [getattr(m, n, None) for n in ("weight_g", "weight_v", "weight_orig", "weight", "bias")]
-    return tuple((t.data_ptr(), t._version) for t in ts if isinstance(t, torch.Tensor))
+class _SubDiscriminator(torch.nn.Module):
+    """forward() of DiscriminatorP / DiscriminatorS: y fp32 [B,1,T] -> (logits [B, H*p], feature maps fp32
+    [B,C,H,p])."""
+
+    def forward(self, x):
+        _require_cuda(x, f"{type(self).__name__}.forward")
+        from . import autograd
+        return autograd.disc_forward(self, x, _wants_grad(x, self))
 
 
-def _disc_weights(owner: nn.Module, idx: int, m: nn.Module, build):
-    """Per-layer cache of the GEMM-ready weight: rebuilt when a parameter changed, and on every call for a
-    spectral-norm layer in train mode (its power iteration must advance call by call)."""
-    cache = owner.__dict__.setdefault("_hg_wcache", {})
-    live_sn = hasattr(m, "weight_orig") and m.training
-    key = None if live_sn else _param_key(m)
-    hit = cache.get(idx)
-    if hit is not None and key is not None and hit[0] == key:
-        return hit[1]
-    val = build()
-    cache[idx] = (key, val)
-    return val
-
-
-def _disc_forward(L, owner: nn.Module, y: torch.Tensor, period: int, first, mids, last, mods):
-    """Shared body of DiscriminatorP / DiscriminatorS.  y fp32 [B,1,T] -> (logits [B, H*p], fmaps fp32 NCHW-like).
-    first = (k, stride, pad, cout), mids = [_DiscLayer], last = (k,), mods = conv modules in order."""
-    b, c, t = y.shape
-    if c != 1:
-        raise ValueError("discriminators take [B,1,T] audio")
-    dev = y.device
-    yin = y.reshape(b, t).contiguous().float()
-    st = _stream()
-    k0, s0, p0, c0 = first
-    h = (t + period - 1) // period
-    if (h * period - t) >= t:
-        raise RuntimeError("reflect padding needs n_pad < t (reference F.pad behaviour)")
-    h = (h + 2 * p0 - k0) // s0 + 1
-    nseq = b * period
-    # geometry + zero-initialised activation buffers (rows past the valid length are the next conv's zero
-    # padding and are never written), cached per input shape
-    ws_cache = owner.__dict__.setdefault("_hg_ws", {})
-    ws = ws_cache.get((b, t, dev))
-    if ws is None:
-        geo, hh = [], h
-        rows = _round_up(hh, mids[0].stride)
-        geo.append((hh, rows, c0))
-        for li, layer in enumerate(mids):
-            hh = (hh + 2 * layer.pad - layer.k) // layer.stride + 1
-            nxt = mids[li + 1].stride if li + 1 < len(mids) else 1
-            geo.append((hh, _round_up(hh, nxt), layer.cout))
-        ws = [(torch.zeros(nseq, r_, c_, dtype=torch.bfloat16, device=dev), h_, r_, c_) for h_, r_, c_ in geo]
-        if len(ws_cache) >= 4:
-            ws_cache.pop(next(iter(ws_cache)))
-        ws_cache[(b, t, dev)] = ws
-    w0, b0 = _disc_weights(owner, 0, mods[0], lambda: (_effective_weight(mods[0]).reshape(c0, k0).contiguous(),
-                                                         mods[0].bias.detach().float().contiguous()))
-    act, h, rows, _ = ws[0]
-    _lib.check(L.hg_disc_first_conv_fwd(yin.data_ptr(), w0.data_ptr(), b0.data_ptr(), b, t, period, k0, s0, p0, c0,
-                                        rows, act.data_ptr(), LRELU_SLOPE, st), "hg_disc_first_conv_fwd")
-    for li, layer in enumerate(mids):
-        m = mods[1 + li]
-
-        def build(m=m, layer=layer):
-            w = _effective_weight(m)
-            return layer.pack(w.reshape(w.shape[0], w.shape[1], layer.k)), m.bias.detach().float().contiguous()
-
-        w, bias = _disc_weights(owner, 1 + li, m, build)
-        out, h_out, rows_out, _ = ws[1 + li]
-        _lib.check(L.hg_conv1d_general_fwd(act.data_ptr(), w.data_ptr(), bias.data_ptr(), nseq, rows, layer.cin, h_out,
-                                           rows_out, layer.groups_eff, layer.cout, layer.k, layer.stride, layer.pad,
-                                           out.data_ptr(), LRELU_SLOPE, 0, 0, 0, st), "hg_conv1d_general_fwd")
-        act, h, rows = out, h_out, rows_out
-    mp, kp, c_last = mods[-1], last[0], ws[-1][3]
-    wp, bp = _disc_weights(owner, len(mods) - 1, mp, lambda: (_effective_weight(mp).reshape(c_last, kp).contiguous(),
-                                                               mp.bias.detach().float().contiguous()))
-    post = torch.empty(nseq, h, dtype=torch.float32, device=dev)
-    _lib.check(L.hg_disc_last_conv_fwd(act.data_ptr(), wp.data_ptr(), bp.data_ptr(), nseq, h, rows, c_last, kp,
-                                       post.data_ptr(), st), "hg_disc_last_conv_fwd")
-    fmap = []
-    for a_, h_, rows_, c_ in ws:
-        f = torch.empty(b, c_, h_, period, dtype=torch.float32, device=dev)
-        _lib.check(L.hg_disc_export_fmap(a_.data_ptr(), b, period, h_, rows_, c_, f.data_ptr(), st), "hg_disc_export_fmap")
-        fmap.append(f)
-    post = post.view(b, period, h).permute(0, 2, 1).contiguous().unsqueeze(1)  # [B,1,H,p]
-    fmap.append(post)
-    return torch.flatten(post, 1, -1), fmap
-
-
-def _check_disc_input(x: torch.Tensor, what: str) -> None:
-    _require_cuda(x, what)
-
-
-def _disc_wants_grad(x: torch.Tensor, disc: nn.Module) -> bool:
-    return torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in disc.parameters()))
-
-
-class DiscriminatorP(torch.nn.Module):
+class DiscriminatorP(_SubDiscriminator):
     def __init__(self, period, kernel_size=5, stride=3, use_spectral_norm=False):
         super().__init__()
         self.period = period
@@ -891,22 +788,6 @@ class DiscriminatorP(torch.nn.Module):
         layers.append(norm_f(Conv2d(1024, 1024, (kernel_size, 1), 1, padding=(2, 0))))
         self.convs = nn.ModuleList(layers)
         self.conv_post = norm_f(Conv2d(1024, 1, (3, 1), 1, padding=(1, 0)))
-
-    def forward(self, x):
-        _check_disc_input(x, "DiscriminatorP.forward")
-        if _disc_wants_grad(x, self):
-            from . import autograd
-            return autograd.disc_forward(self, x)
-        convs = list(self.convs)
-        first = (convs[0].kernel_size[0], convs[0].stride[0], convs[0].padding[0], convs[0].out_channels)
-        mids = self.__dict__.get("_hg_layers")
-        if mids is None:
-            mids = [_DiscLayer(m.in_channels, m.out_channels, m.kernel_size[0], m.stride[0], m.padding[0], 1)
-                    for m in convs[1:]]
-            self.__dict__["_hg_layers"] = mids
-        out, fmap = _disc_forward(_lib.lib(), self, x, self.period, first, mids, (self.conv_post.kernel_size[0],),
-                                  convs + [self.conv_post])
-        return out, fmap
 
 
 class MultiPeriodDiscriminator(torch.nn.Module):
@@ -924,7 +805,7 @@ class MultiPeriodDiscriminator(torch.nn.Module):
         return y_d_rs, y_d_gs, fmap_rs, fmap_gs
 
 
-class DiscriminatorS(torch.nn.Module):
+class DiscriminatorS(_SubDiscriminator):
     _SPEC = [(1, 128, 15, 1, 1, 7), (128, 128, 41, 2, 4, 20), (128, 256, 41, 2, 16, 20),
              (256, 512, 41, 4, 16, 20), (512, 1024, 41, 4, 16, 20), (1024, 1024, 41, 1, 16, 20),
              (1024, 1024, 5, 1, 1, 2)]
@@ -937,21 +818,18 @@ class DiscriminatorS(torch.nn.Module):
         self.conv_post = norm_f(Conv1d(1024, 1, 3, 1, padding=1))
 
     def forward(self, x):
-        _check_disc_input(x, "DiscriminatorS.forward")
-        if _disc_wants_grad(x, self):
-            from . import autograd
-            out, fmap = autograd.disc_forward(self, x)
-            return out, [f.squeeze(-1) for f in fmap]
-        convs = list(self.convs)
-        first = (convs[0].kernel_size[0], convs[0].stride[0], convs[0].padding[0], convs[0].out_channels)
-        mids = self.__dict__.get("_hg_layers")
-        if mids is None:
-            mids = [_DiscLayer(m.in_channels, m.out_channels, m.kernel_size[0], m.stride[0], m.padding[0], m.groups)
-                    for m in convs[1:]]
-            self.__dict__["_hg_layers"] = mids
-        out, fmap = _disc_forward(_lib.lib(), self, x, 1, first, mids, (self.conv_post.kernel_size[0],),
-                                  convs + [self.conv_post])
+        out, fmap = super().forward(x)
         return out, [f.squeeze(-1) for f in fmap]   # [B,C,T,1] -> the reference's [B,C,T]
+
+
+def _avgpool(x: torch.Tensor) -> torch.Tensor:
+    """AvgPool1d(4, 2, padding=2) over the last dimension (hg_avgpool_4_2_2_fwd): [..., T] -> fp32 [..., T // 2 + 1]"""
+    t = x.shape[-1]
+    xin = x.detach().reshape(-1, t).contiguous().float()
+    out = torch.empty(*x.shape[:-1], t // 2 + 1, dtype=torch.float32, device=x.device)
+    _lib.check(_lib.lib().hg_avgpool_4_2_2_fwd(xin.data_ptr(), xin.shape[0], t, out.data_ptr(), _stream()),
+               "hg_avgpool_4_2_2_fwd")
+    return out
 
 
 class MultiScaleDiscriminator(torch.nn.Module):
@@ -967,16 +845,11 @@ class MultiScaleDiscriminator(torch.nn.Module):
         if torch.is_grad_enabled() and x.requires_grad:
             from . import autograd
             return autograd.avgpool(x)
-        b, c, t = x.shape
-        xin = x.reshape(b * c, t).contiguous().float()
-        out = torch.empty(b * c, t // 2 + 1, dtype=torch.float32, device=x.device)
-        _lib.check(_lib.lib().hg_avgpool_4_2_2_fwd(xin.data_ptr(), b * c, t, out.data_ptr(), _stream()),
-                   "hg_avgpool_4_2_2_fwd")
-        return out.view(b, c, -1)
+        return _avgpool(x)
 
     def forward(self, y, y_hat):
-        _check_disc_input(y, "MultiScaleDiscriminator.forward")
-        _check_disc_input(y_hat, "MultiScaleDiscriminator.forward")
+        _require_cuda(y, "MultiScaleDiscriminator.forward")
+        _require_cuda(y_hat, "MultiScaleDiscriminator.forward")
         y_d_rs, y_d_gs, fmap_rs, fmap_gs = [], [], [], []
         for i, d in enumerate(self.discriminators):
             if i != 0:
@@ -988,6 +861,14 @@ class MultiScaleDiscriminator(torch.nn.Module):
         return y_d_rs, y_d_gs, fmap_rs, fmap_gs
 
 
+def _loss_mean(a32: torch.Tensor, b32: Optional[torch.Tensor], mode: int, c: float) -> torch.Tensor:
+    """mean |a - b| (mode 0) or mean (c - a)^2 (mode 1) of contiguous fp32 device tensors (hg_loss_sum)"""
+    acc = torch.zeros(1, dtype=torch.float32, device=a32.device)
+    _lib.check(_lib.lib().hg_loss_sum(a32.data_ptr(), 0 if b32 is None else b32.data_ptr(), a32.numel(), mode, c,
+                                      acc.data_ptr(), _stream()), "hg_loss_sum")
+    return acc[0] / a32.numel()
+
+
 def _device_mean(a: torch.Tensor, b: Optional[torch.Tensor], mode: int, c: float) -> torch.Tensor:
     """mean |a-b| (mode 0) or mean (c-a)^2 (mode 1) through hg_loss_sum; differentiable (hg_loss_grad) when an
     argument carries autograd history.  No CPU path."""
@@ -996,12 +877,7 @@ def _device_mean(a: torch.Tensor, b: Optional[torch.Tensor], mode: int, c: float
     if torch.is_grad_enabled() and (a.requires_grad or (b is not None and b.requires_grad)):
         from . import autograd
         return autograd.device_mean(a, b, mode, c)
-    a32 = a.detach().contiguous().float()
-    b32 = None if b is None else b.detach().contiguous().float()
-    acc = torch.zeros(1, dtype=torch.float32, device=a.device)
-    _lib.check(_lib.lib().hg_loss_sum(a32.data_ptr(), 0 if b32 is None else b32.data_ptr(), a32.numel(), mode, c,
-                                      acc.data_ptr(), _stream()), "hg_loss_sum")
-    return acc[0] / a32.numel()
+    return _loss_mean(a.detach().contiguous().float(), None if b is None else b.detach().contiguous().float(), mode, c)
 
 
 def feature_loss(fmap_r, fmap_g):

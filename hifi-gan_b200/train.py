@@ -23,16 +23,8 @@ import torch.nn as nn
 from . import _lib
 from .meldataset import mel_spectrogram, torch_mels
 from .models import (LRELU_SLOPE, DiscriminatorP, DiscriminatorS, Generator, MultiPeriodDiscriminator,
-                     MultiScaleDiscriminator, ResBlock1, _DiscLayer, _PackedConv, _conv, _device_mean,
-                     _effective_weight, _g_v, _pad_ch, _round_up, _stream, discriminator_loss, feature_loss,
-                     generator_loss)
-
-
-def _gb(param: torch.Tensor) -> torch.Tensor:
-    """The buffer this library writes `param`'s gradient into (a view of its network's flat gradient buffer, set by
-    FlatParams).  TrainStep binds it as `param.grad` as well; the autograd path (autograd.py) keeps it private and
-    hands copies to torch."""
-    return param._hg_grad
+                     MultiScaleDiscriminator, ResBlock1, _DiscLayer, _PackedConv, _avgpool, _conv, _device_mean,
+                     _g_v, _pad_ch, _round_up, _stream, discriminator_loss, feature_loss, generator_loss)
 
 
 def _p(x) -> int:
@@ -75,8 +67,8 @@ class FlatParams:
     state_dict() / load_state_dict() keep working — they copy through the views."""
 
     def __init__(self, module: nn.Module, device, bind: bool = True):
-        """bind=False (the autograd path): only the flat GRADIENT buffer is created and attached to the parameters as
-        `_hg_grad`; parameters, `.grad` and the optimizer state stay torch's."""
+        """bind=False (the autograd path): only the flat GRADIENT buffer is created; parameters, `.grad` and the
+        optimizer state stay torch's."""
         self.module = module
         self.bound = bind
         ps = [p for p in module.parameters()]
@@ -89,11 +81,11 @@ class FlatParams:
         self.numel = off
         self.g = torch.zeros(off, dtype=torch.float32, device=device)
         self.params = ps
+        self._grads = {id(p): self.g[o:o + s].view(p.shape) for p, o, s in zip(ps, self.offsets, self.sizes)}
         if not bind:
-            for p, o, s in zip(ps, self.offsets, self.sizes):
+            for p in ps:
                 if p.device != self.g.device or p.dtype != torch.float32 or not p.is_contiguous():
                     raise RuntimeError("hifigan_b200: parameters must be contiguous fp32 tensors on the CUDA device")
-                p._hg_grad = self.g[o:o + s].view(p.shape)
             return
         self.p = torch.zeros(off, dtype=torch.float32, device=device)
         self.m = torch.zeros(off, dtype=torch.float32, device=device)
@@ -106,8 +98,12 @@ class FlatParams:
                 view = self.p[o:o + s].view(p.shape)
                 view.copy_(p.detach().to(device=device, dtype=torch.float32))
                 p.data = view
-                p.grad = self.g[o:o + s].view(p.shape)
-                p._hg_grad = p.grad
+                p.grad = self._grads[id(p)]
+
+    def grad(self, param: torch.Tensor) -> torch.Tensor:
+        """the view of the flat gradient buffer the library writes `param`'s gradient into (bound as `param.grad`
+        when bind=True; the autograd path keeps it private and hands copies to torch)"""
+        return self._grads[id(param)]
 
     def adamw(self, lr: float, betas=(0.8, 0.99), eps: float = 1e-8, weight_decay: float = 0.01,
               grad_scale: float = 1.0) -> None:
@@ -245,8 +241,8 @@ class _GenLayerGrad:
     Every kernel here ACCUMULATES: GeneratorTrainer.backward zeroes the flat packed-gradient buffer and the flat
     parameter-gradient buffer first, so no per-layer memset / copy nodes are needed."""
 
-    def __init__(self, pc: _PackedConv, device, need_dgrad: bool = True):
-        self.pc = pc
+    def __init__(self, pc: _PackedConv, device, flat: FlatParams, need_dgrad: bool = True):
+        self.pc, self.flat = pc, flat
         rows = pc.w.shape[1]
         self.rows = rows
         self.wd = torch.empty(pc.taps, pc.cin_p, rows, dtype=torch.bfloat16, device=device) if need_dgrad else None
@@ -273,16 +269,16 @@ class _GenLayerGrad:
                       ints=(pc.taps, self.rows, pc.cin_p, tc, tn))
         m = pc.module
         g, v = _g_v(m)
-        dg = None if g is None else _gb(g)
+        dv, dg = self.flat.grad(v), None if g is None else self.flat.grad(g)
         if pc.kind == "conv":
-            table.add(finish, batched.FINISH_ROW, pc.cout, pc.cin * pc.taps * 4, self.dwp, g, v, _gb(v), dg,
+            table.add(finish, batched.FINISH_ROW, pc.cout, pc.cin * pc.taps * 4, self.dwp, g, v, dv, dg,
                       ints=(0, pc.cout, pc.cin, pc.taps, self.rows, pc.cin_p, pc.cout, 1, 0, 0, 0, 0, 1),
                       tab=range(pc.taps))
         else:
             k = m.kernel_size[0]
             nshift, smin = c_int(), c_int()
             _lib.check(_lib.lib().hg_convtr1d_geometry(k, pc.stride, m.padding[0], byref(nshift), byref(smin)))
-            table.add(finish, batched.FINISH_ROW, pc.cin, pc.cout * k * 4, self.dwp, g, v, _gb(v), dg,
+            table.add(finish, batched.FINISH_ROW, pc.cin, pc.cout * k * 4, self.dwp, g, v, dv, dg,
                       ints=(1, pc.cin, pc.cout, k, pc.stride * pc.cout_p, pc.cin_p, 0, 1, pc.stride, m.padding[0],
                             smin.value, pc.cout_p, 1))
 
@@ -296,7 +292,7 @@ class _GenLayerGrad:
         """pointer of bias.grad when the producer of this layer's output gradient can add its fp32 column sums
         straight into it (no channel padding: c output columns == cout), else 0 -> bias_grad() runs afterwards"""
         b = self.pc.module.bias
-        return _gb(b).data_ptr() if (b is not None and c == self.pc.cout) else 0
+        return self.flat.grad(b).data_ptr() if (b is not None and c == self.pc.cout) else 0
 
     def bias_grad(self, L, dy, batch: int, t: int, c: int) -> None:
         """bias.grad (+)= column sums of dy [B][t][c] — only for layers with channel padding (V2's 16-channel stage);
@@ -305,12 +301,13 @@ class _GenLayerGrad:
         if b is None or self.bias_dst(c):
             return
         if c == self.pc.cout:
-            _lib.check(L.hg_colsum_bf16(_p(dy), batch, t, t, c, 1, _gb(b).data_ptr(), _stream()), "hg_colsum_bf16")
+            _lib.check(L.hg_colsum_bf16(_p(dy), batch, t, t, c, 1, self.flat.grad(b).data_ptr(), _stream()),
+                       "hg_colsum_bf16")
         else:
             if self.db is None:
                 self.db = torch.zeros(c, dtype=torch.float32, device=dy.device)
             _lib.check(L.hg_colsum_bf16(_p(dy), batch, t, t, c, 0, self.db.data_ptr(), _stream()), "hg_colsum_bf16")
-            _gb(b).add_(self.db[: self.pc.cout])
+            self.flat.grad(b).add_(self.db[: self.pc.cout])
 
     def dgrad(self, L, dy, batch: int, t: int, out, mask=None, slope: float = LRELU_SLOPE, res0=None, res1=None,
               res2=None, scale: float = 1.0, bias_dsts=()) -> None:
@@ -327,29 +324,33 @@ class _GenLayerGrad:
         pc = self.pc
         m = pc.module
         g, v = _g_v(m)
-        gp, dgp = (0, 0) if g is None else (g.data_ptr(), _gb(g).data_ptr())
+        gp, dgp = (0, 0) if g is None else (g.data_ptr(), self.flat.grad(g).data_ptr())
+        dvp = self.flat.grad(v).data_ptr()
         if pc.kind == "conv":
             _lib.check(L.hg_wgrad_finish_conv(self.dwp.data_ptr(), pc.cout, pc.cin, pc.taps, self.rows, pc.cin_p,
-                                              pc.cout, 1, None, v.data_ptr(), gp, 1, _gb(v).data_ptr(), dgp,
+                                              pc.cout, 1, None, v.data_ptr(), gp, 1, dvp, dgp,
                                               _stream()), "hg_wgrad_finish_conv")
         else:
             _lib.check(L.hg_wgrad_finish_convtr(self.dwp.data_ptr(), pc.cin, pc.cout, m.kernel_size[0], pc.stride,
                                                 m.padding[0], pc.cin_p, pc.cout_p, v.data_ptr(), gp, 1,
-                                                _gb(v).data_ptr(), dgp, _stream()), "hg_wgrad_finish_convtr")
+                                                dvp, dgp, _stream()), "hg_wgrad_finish_convtr")
 
 
-def _route_weight_grad(L, m: nn.Module, dw: torch.Tensor, d0: int, rest: int, accumulate: bool = False) -> None:
-    """dw fp32 (dense, parameter layout, first d0*rest elements of `dw`) -> the module's parameter gradients."""
+def _route_weight_grad(L, flat: FlatParams, m: nn.Module, dw: torch.Tensor, d0: int, rest: int,
+                       accumulate: bool = False) -> None:
+    """dw fp32 (dense, parameter layout, first d0*rest elements of `dw`) -> the module's parameter gradients in
+    `flat`'s gradient buffer."""
     g, v = _g_v(m)
     if g is not None:
         _lib.check(L.hg_weight_norm_bwd(dw.data_ptr(), v.data_ptr(), g.data_ptr(), d0, rest, 1 if accumulate else 0,
-                                        _gb(v).data_ptr(), _gb(g).data_ptr(), _stream()), "hg_weight_norm_bwd")
+                                        flat.grad(v).data_ptr(), flat.grad(g).data_ptr(), _stream()),
+                   "hg_weight_norm_bwd")
     else:
         src = dw[: d0 * rest].view(v.shape)
         if accumulate:
-            _gb(v).add_(src)
+            flat.grad(v).add_(src)
         else:
-            _gb(v).copy_(src)
+            flat.grad(v).copy_(src)
 
 
 class GeneratorTrainer:
@@ -363,9 +364,9 @@ class GeneratorTrainer:
         gen._drop_engines()
         self.eng = gen._engine(device)
         e = self.eng
-        self.g_pre = _GenLayerGrad(e.pre, device, need_dgrad=not bind)
-        self.g_ups = [_GenLayerGrad(pc, device) for pc in e.ups]
-        self.g_blocks = [[_GenLayerGrad(pc, device) for pc in blk] for blk in e.blocks]
+        self.g_pre = _GenLayerGrad(e.pre, device, self.flat, need_dgrad=not bind)
+        self.g_ups = [_GenLayerGrad(pc, device, self.flat) for pc in e.ups]
+        self.g_blocks = [[_GenLayerGrad(pc, device, self.flat) for pc in blk] for blk in e.blocks]
         layers = [self.g_pre] + self.g_ups + [x for b in self.g_blocks for x in b]
         self.dwp_flat = torch.zeros(sum(gl.dwp_numel for gl in layers), dtype=torch.float32, device=device)
         off = 0
@@ -593,8 +594,8 @@ class GeneratorTrainer:
 
         def post_grads():
             cin, k = post.in_channels, post.kernel_size[0]
-            _route_weight_grad(L, post, self.post_dw[:cin].contiguous(), 1, cin * k)
-            _gb(post.bias).copy_(self.post_db)      # flat.g was zeroed: plain stores here
+            _route_weight_grad(L, self.flat, post, self.post_dw[:cin].contiguous(), 1, cin * k)
+            self.flat.grad(post.bias).copy_(self.post_db)      # flat.g was zeroed: plain stores here
         self._side(L, self.W_LANE, main, post_grads)
         for i in reversed(range(len(e.ups))):
             st = stages[i]
@@ -656,7 +657,8 @@ class _DiscBwdLayer:
         self.w = torch.empty(self.nshift, s * layer.cin, self.cout_tile, dtype=torch.bfloat16, device=device)
 
     def pack(self, w_eff: torch.Tensor, w_fwd_packed=None) -> None:
-        """w_eff fp32 [cout][cin/groups][k] (effective weight) -> the data-gradient filter bank (hg_pack_disc_weight)"""
+        """w_eff fp32 [cout][cin/groups][k] (effective weight) -> the data-gradient filter bank (hg_pack_disc_weight).
+        w_fwd_packed is not read: the bank is derived from w_eff alone."""
         layer = self.layer
         _lib.check(_lib.lib().hg_pack_disc_weight(w_eff.data_ptr(), layer.cout, layer.cin, layer.groups, layer.merge,
                                                   layer.k, layer.stride, layer.pad, 0, self.w.data_ptr(), _stream()),
@@ -690,11 +692,12 @@ class _SubDiscTrainer:
 
     W_CHAINS = 4
 
-    def __init__(self, disc: nn.Module, device, boost: int = 0):
-        """boost: added to the CUDA stream priorities of every lane of this sub-discriminator (negative = more urgent):
+    def __init__(self, disc: nn.Module, device, flat: FlatParams, boost: int = 0):
+        """flat: the FlatParams whose gradient buffer receives this sub-discriminator's parameter gradients.
+        boost: added to the CUDA stream priorities of every lane of this sub-discriminator (negative = more urgent):
         the sub-discriminator with the longest chain (the spectral-norm scale) is the step's critical path, so its
         kernels — its weight-gradient lane included — are placed ahead of the other sub-discriminators'."""
-        self.disc, self.device = disc, device
+        self.disc, self.device, self.flat = disc, device, flat
         self.period = getattr(disc, "period", 1)
         convs = list(disc.convs)
         self.mods = convs + [disc.conv_post]
@@ -743,7 +746,6 @@ class _SubDiscTrainer:
     def invalidate(self) -> None:
         """the parameters changed (optimizer update / load_state_dict): re-fold and re-pack on next use"""
         self.fwd_valid = self.dgrad_valid = False
-        self.disc.__dict__.pop("_hg_wcache", None)      # the module API's own pack cache (inference-side forward)
 
     # ---- weights -------------------------------------------------------------------------------------------
     def _scratch_of(self, chain: int) -> torch.Tensor:
@@ -827,8 +829,8 @@ class _SubDiscTrainer:
                 pos = [0] * layer.k
                 for q, j in enumerate(layer.order):
                     pos[j] = q
-                t.add("finish", batched.FINISH_ROW, layer.cout, cin_g * layer.k * 4, self.dwps[li - 1], g, v, _gb(v),
-                      _gb(g), ints=(0, layer.cout, cin_g, layer.k, layer.cout, layer.cin_tile,
+                t.add("finish", batched.FINISH_ROW, layer.cout, cin_g * layer.k * 4, self.dwps[li - 1], g, v,
+                      self.flat.grad(v), self.flat.grad(g), ints=(0, layer.cout, cin_g, layer.k, layer.cout, layer.cin_tile,
                                     layer.cout // layer.groups, layer.merge, 0, 0, 0, 0, 1), tab=pos)
         self._tables[part] = t.finalize()
         return t
@@ -1147,26 +1149,27 @@ class _SubDiscTrainer:
             self.dgrad_valid = True
 
     # ---- one module call under torch autograd (autograd.py): forward with its own activation / weight slot ---------
-    def forward_single(self, x2d: torch.Tensor, slot: int):
+    def forward_single(self, x2d: torch.Tensor, slot: int, dgrad: bool = True):
         """x2d fp32 [B, T] -> (G, W) of call slot `slot`: activations, logits, the weights this call used (a train-mode
-        spectral-norm layer advances its power iteration per call, like the reference's hook) and their
-        data-gradient banks.  Everything on the current stream."""
+        spectral-norm layer advances its power iteration per call, like the reference's hook) and, with `dgrad`
+        (the call can be differentiated), their data-gradient banks.  Everything on the current stream."""
         L = _lib.lib()
         nb, t = x2d.shape
         G = self._geometry(nb, t, slot)
         W = self._prepare_weights(slot)
-        tb = self._table(slot)
-        if tb.has("dgrad"):
-            tb.launch("dgrad")
-        for i in self.untiled:
-            self._bwd_bank(slot)[i].pack(W["eff"][1 + i])
+        if dgrad:
+            tb = self._table(slot)
+            if tb.has("dgrad"):
+                tb.launch("dgrad")
+            for i in self.untiled:
+                self._bwd_bank(slot)[i].pack(W["eff"][1 + i])
         self._forward_part(L, G, W, x2d, 0, nb, t)
         return G, W
 
     def backward_single(self, G, W, slot: int, x2d: torch.Tensor, dlogit: torch.Tensor, pre_adds, want_wgrad: bool,
                         dy_audio) -> None:
         """Backward of forward_single's call: dlogit fp32 [B*period][h] (internal order), pre_adds[l] bf16 gradient at
-        feature map l in the internal layout (or None) -> parameter gradients ADDED into the _gb buffers (want_wgrad)
+        feature map l in the internal layout (or None) -> parameter gradients ADDED into self.flat (want_wgrad)
         and / or the audio gradient ADDED into dy_audio fp32 [B][T]."""
         L = _lib.lib()
         nb, t = x2d.shape
@@ -1228,7 +1231,7 @@ class _SubDiscTrainer:
         fm_r_last = act_last[seq0 - nr:].data_ptr() if fm else 0
         # every data-gradient launch of the discriminator step also sums the bias gradient of the layer whose output
         # it differentiates, in fp32, straight into the flat gradient buffer (zeroed in run_phases)
-        bias_of = (lambda li: _gb(self.mods[li].bias).data_ptr()) if want_wgrad else (lambda li: 0)
+        bias_of = (lambda li: self.flat.grad(self.mods[li].bias).data_ptr()) if want_wgrad else (lambda li: 0)
         _lib.check(L.hg_disc_last_conv_bwd(act_last[seq0:].data_ptr(), W["wp"].data_ptr(), G["dlogit"][seq0:].data_ptr(),
                                            nseq, h_last, rows_last, c_last, self.kpost, LRELU_SLOPE, fm_r_last,
                                            nfm[nl] if fm else 0.0, _p(pre[nl]), G["grad"][-1][seq0:].data_ptr(), 0, 0,
@@ -1276,7 +1279,8 @@ class _SubDiscTrainer:
                         _lib.check(L.hg_wgrad_finish_conv(self.dwps[li].data_ptr(), layer.cout, cin_g, layer.k,
                                                           layer.cout, layer.cin_tile, layer.cout // layer.groups,
                                                           layer.merge, order, v.data_ptr(), g.data_ptr(), 1,
-                                                          _gb(v).data_ptr(), _gb(g).data_ptr(), st), "hg_wgrad_finish_conv")
+                                                          self.flat.grad(v).data_ptr(), self.flat.grad(g).data_ptr(),
+                                                          st), "hg_wgrad_finish_conv")
                 side(layer_grads, nl - li)
             bwd[li].dgrad(L, d_out, nseq, h_out, rows_out, rows_in, a_in[seq0:],
                           a_in[seq0 - nr:] if fm else None, nfm[li] if fm else 0.0, G["grad"][li][seq0:], _stream(),
@@ -1304,12 +1308,11 @@ class _SubDiscTrainer:
                                                 G["grad"][0][seq0:].data_ptr(), bn, self.t, period, k0, s0, p0, c0,
                                                 geo[0][1], 0, 0, _p(dy_audio), _stream()), "hg_disc_first_conv_bwd")
 
-    @staticmethod
-    def _bias(m: nn.Module, db: torch.Tensor, accumulate: bool) -> None:
+    def _bias(self, m: nn.Module, db: torch.Tensor, accumulate: bool) -> None:
         if accumulate:
-            _gb(m.bias).add_(db)
+            self.flat.grad(m.bias).add_(db)
         else:
-            _gb(m.bias).copy_(db)
+            self.flat.grad(m.bias).copy_(db)
 
     def _route(self, L, m: nn.Module, dw: torch.Tensor, d0: int, rest: int, W, li: int, accumulate: bool) -> None:
         if hasattr(m, "weight_orig"):
@@ -1317,10 +1320,10 @@ class _SubDiscTrainer:
             u, v, sigma, snws = W["sn"][li]
             _lib.check(L.hg_spectral_norm_bwd(dw.data_ptr(), W["eff"][li].data_ptr(), u.data_ptr(), v.data_ptr(),
                                               sigma.data_ptr(), d0, rest, 1 if accumulate else 0,
-                                              _gb(m.weight_orig).data_ptr(), snws.data_ptr(), _stream()),
+                                              self.flat.grad(m.weight_orig).data_ptr(), snws.data_ptr(), _stream()),
                        "hg_spectral_norm_bwd")
         else:
-            _route_weight_grad(L, m, dw, d0, rest, accumulate)
+            _route_weight_grad(L, self.flat, m, dw, d0, rest, accumulate)
 
 
 class DiscriminatorTrainer:
@@ -1330,16 +1333,15 @@ class DiscriminatorTrainer:
         self.mpd, self.msd, self.device = mpd, msd, device
         holder = nn.ModuleList([mpd, msd])        # optimizer order of the reference: chain(msd, mpd) — order is free
         self.flat = FlatParams(holder, device)
-        for d in list(mpd.discriminators) + list(msd.discriminators):
-            d.__dict__.pop("_hg_wcache", None)
         # scheduling: the scale discriminators' chains (k = 41 grouped convs, spectral norm) are long and narrow, the
         # period discriminators' short and wide; the scales' lanes outrank the periods' so that they are done by the
         # time the periods fill the GPU (HG_DISC_BOOST="a,b,c" sets the three boosts, "0" disables; measured
         # -2,-1,-1: 11.86 ms, 0,0,0: 11.98, -2,-1,0: 12.12, -2,-2,-2: 12.9 in round 2)
         env = os.environ.get("HG_DISC_BOOST", "")
         boosts = [0, 0, 0] if env == "0" else [int(v) for v in env.split(",")] if "," in env else [-2, -1, -1]
-        self.subs_p = [_SubDiscTrainer(d, device) for d in mpd.discriminators]
-        self.subs_s = [_SubDiscTrainer(d, device, boosts[min(i, 2)]) for i, d in enumerate(msd.discriminators)]
+        self.subs_p = [_SubDiscTrainer(d, device, self.flat) for d in mpd.discriminators]
+        self.subs_s = [_SubDiscTrainer(d, device, self.flat, boosts[min(i, 2)])
+                       for i, d in enumerate(msd.discriminators)]
         self.subs = self.subs_p + self.subs_s
         self.nslots = 12
         # raw loss sums of the discriminator-step forward / of the generator-step forward
@@ -1364,18 +1366,12 @@ class DiscriminatorTrainer:
 
     def _inputs(self, y: torch.Tensor, y_hat: torch.Tensor) -> int:
         """(real ++ generated) audio and its AvgPool1d(4,2,2) pyramid for the scale discriminators"""
-        L = _lib.lib()
         b = y.shape[0]
         ycat = torch.cat([y.reshape(b, -1), y_hat.reshape(b, -1)], 0).contiguous().float()
         self.b, self.t = b, ycat.shape[1]
         self.pooled = [ycat]
-        cur = ycat
         for i in range(1, len(self.subs_s)):
-            t = cur.shape[1]
-            nxt = torch.empty(2 * b, t // 2 + 1, dtype=torch.float32, device=self.device)
-            _lib.check(L.hg_avgpool_4_2_2_fwd(cur.data_ptr(), 2 * b, t, nxt.data_ptr(), _stream()), "hg_avgpool_4_2_2_fwd")
-            self.pooled.append(nxt)
-            cur = nxt
+            self.pooled.append(_avgpool(self.pooled[-1]))
         return b
 
     def _input_of(self, i: int) -> torch.Tensor:
