@@ -107,7 +107,6 @@ _SIGNATURES = {
     "hg_last_error": (c_char_p, []),
     "hg_abi_version": (c_int, []),
     "hg_launch_count": (c_int64, []),
-    "hg_set_cta_limit": (c_int, [c_int]),
     "hg_timestamp": (c_int, [c_void_p, c_void_p]),
     "hg_pack_conv1d_weight": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "hg_convtr1d_geometry": (c_int, [c_int, c_int, c_int, POINTER(c_int), POINTER(c_int)]),
@@ -151,7 +150,6 @@ _SIGNATURES = {
                                 c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     "hg_conv1d_wgrad": (c_int, [c_void_p, c_void_p] + [c_int] * 11 + [c_void_p, c_int, c_void_p]),
     "hg_unpack_wgrad_conv": (c_int, [c_void_p] + [c_int] * 7 + [POINTER(c_int), c_void_p, c_void_p]),
-    "hg_unpack_wgrad_convtr": (c_int, [c_void_p] + [c_int] * 7 + [c_void_p, c_void_p]),
     "hg_wgrad_finish_conv": (c_int, [c_void_p] + [c_int] * 7 + [POINTER(c_int), c_void_p, c_void_p, c_int, c_void_p,
                                                                   c_void_p, c_void_p]),
     "hg_wgrad_finish_convtr": (c_int, [c_void_p] + [c_int] * 7 + [c_void_p, c_void_p, c_int, c_void_p, c_void_p,
@@ -173,7 +171,6 @@ _SIGNATURES = {
     "hg_avgpool_4_2_2_bwd": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "hg_loss_grad": (c_int, [c_void_p, c_void_p, ctypes.c_longlong, c_int, c_float, c_float, c_float, c_void_p,
                              c_void_p, c_void_p]),
-    "hg_l1_sum_bf16": (c_int, [c_void_p, c_void_p, ctypes.c_longlong, c_void_p, c_void_p]),
     "hg_adamw_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, ctypes.c_longlong, c_float, c_float, c_float,
                               c_float, c_float, c_int, c_void_p, c_void_p, c_float, c_void_p]),
 }
@@ -195,7 +192,7 @@ def lib() -> ctypes.CDLL:
                 fn = getattr(handle, name)
                 fn.restype = res
                 fn.argtypes = args
-            if handle.hg_abi_version() != 2:
+            if handle.hg_abi_version() != 3:
                 raise HgError("libhifigan_b200.so ABI mismatch")
             _lib = handle
     return _lib

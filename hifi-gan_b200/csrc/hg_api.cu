@@ -37,12 +37,6 @@ extern "C" int hg_timestamp(uint64_t* dst, void* stream) {
   return HG_OK;
 }
 
-extern "C" int hg_set_cta_limit(int max_ctas) {
-  const int old = hg::t_cta_limit;
-  hg::t_cta_limit = max_ctas > 0 ? max_ctas : 0;
-  return old;
-}
-
 static PFN_cuTensorMapEncodeTiled_v12000 get_encode_fn() {
   static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
   if (fn) return fn;

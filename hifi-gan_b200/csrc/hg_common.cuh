@@ -347,11 +347,6 @@ struct PerDeviceOnce {
     return true;
   }
 };
-
-// hg_set_cta_limit: cap on the persistent grids of the conv kernels launched by this host thread (0 = one CTA per SM).
-// Lets a caller run independent kernel chains side by side on disjoint SM subsets (the MRF branches of a stage).
-inline thread_local int t_cta_limit = 0;
-inline int cap_ctas(int n) { return (t_cta_limit > 0 && t_cta_limit < n) ? t_cta_limit : n; }
 }  // namespace hg
 
 // host-side: cuTensorMapEncodeTiled through the runtime's driver entry point (no -lcuda needed)

@@ -996,13 +996,12 @@ int conv_forward(const void* x, const void* w_packed, const float* bias, int bat
 
   const size_t smem_bytes = 1024 + static_cast<size_t>(a_slots) * p.a_slot_bytes + w_bytes_total +
                             sizeof(Barriers) + colsum_bytes;
-  const int sms = hg::cap_ctas(g_num_sms);
-  const int grid = p.num_tiles < sms ? p.num_tiles : sms;
+  const int grid = p.num_tiles < g_num_sms ? p.num_tiles : g_num_sms;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (pair) {
     const size_t smem2 = 1024 + static_cast<size_t>(a_slots) * p.a_slot_bytes + w_bytes_total + sizeof(Barriers2) +
                          colsum_bytes;
-    const int grid2 = sms >= 2 ? (sms & ~1) : 2;     // whole CTA pairs
+    const int grid2 = g_num_sms;     // whole CTA pairs: `pair` requires an even SM count
     rc = (n_tile == 256) ? launch2<256>(tm_x, tm_w, p, smem2, grid2, st)
                          : launch2<128>(tm_x, tm_w, p, smem2, grid2, st);
     if (rc) return rc;

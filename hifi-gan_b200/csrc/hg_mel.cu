@@ -1,20 +1,16 @@
 // hg_mel.cu — mel_spectrogram (src/meldataset.py:56-85) as ONE fused kernel:
 //   reflect-pad -> frame x periodic Hann -> rFFT(1024) -> |X|^2 -> HTK mel (sparse) -> log(clamp(.,1e-5))
 // The reference goes through torchaudio.transforms.MelSpectrogram (meldataset.py:59-71): >= 6 library
-// launches and three HBM round trips of the [B,513,F] spectrum.  Here a block of 512 threads owns 16
-// consecutive frames: the 4864-sample input window and the constant tables (window, twiddles, CSR filterbank)
-// are brought into shared memory with one round of cp.async copies, each 64-thread group runs a 512-point
-// complex Stockham FFT (radix 8 x 8 x 8) per frame on the even/odd packed samples (two frames per group, the
-// group's two warps meeting on their own named barrier), un-packs the real spectrum, accumulates the
-// triangular mel filters from the CSR table and the block writes [80][16] outputs with 64-byte contiguous runs.
+// launches and three HBM round trips of the [B,513,F] spectrum.  n_fft == 1024 runs mel_kernel2 (one warp per two
+// frames, the FFT in registers), any other n_fft the direct-DFT mel_dft_kernel, and the backward mel_bwd_kernel
+// (64-thread groups running a 512-point complex Stockham FFT, radix 8 x 8 x 8, on the even/odd packed samples).
 //
 // The per-thread phases are __host__ __device__ so tests can run the exact same arithmetic on the CPU
-// (hg_mel_emulate_host below) — there is no GPU in the development container.
+// (hg_mel_emulate_host, hg_mel_bwd_emulate_host below) — there is no GPU in the development container.
 #include "hg_common.cuh"
 
 #include <atomic>
 #include <cmath>
-#include <cstdlib>
 #include <vector>
 
 #include "../../include/hifigan_b200.h"
@@ -45,9 +41,7 @@ namespace {
 constexpr int kNfft = 1024;
 constexpr int kHalf = 512;
 constexpr int kFramesPerBlock = 16;
-constexpr int kGroups = 8;
 constexpr int kGroupThreads = 64;
-constexpr int kMelThreads = kGroups * kGroupThreads;
 constexpr int kPadLen = kHalf + kHalf / 16;  // PADI(511) + 1 = 543 -> 544
 
 __host__ __device__ __forceinline__ int padi(int i) { return i + (i >> 4); }
@@ -115,37 +109,6 @@ __host__ __device__ __forceinline__ void fft_pass(int j, int ns, const cpx* __re
   for (int r = 0; r < 8; ++r) out[padi(j0 + r * ns)] = v[r];
 }
 
-// real-FFT un-packing + power for bins k = tid, tid+64, ... (0..512); z = FFT512 of packed samples
-__host__ __device__ __forceinline__ void unpack_power(int tid, const cpx* __restrict__ z,
-                                                      float* __restrict__ power,
-                                                      const float2* __restrict__ tw1024) {
-  for (int k = tid; k <= kHalf; k += kGroupThreads) {
-    const cpx zk = z[padi(k & (kHalf - 1))];
-    cpx zc = z[padi((kHalf - k) & (kHalf - 1))];
-    zc.y = -zc.y;
-    const cpx e = cpx{0.5f * (zk.x + zc.x), 0.5f * (zk.y + zc.y)};
-    const cpx d = csub(zk, zc);
-    const cpx o = cpx{0.5f * d.y, -0.5f * d.x};  // (zk - zc) / (2i)
-    const float2 w = tw1024[k];
-    const cpx x = cadd(e, cmul(o, cpx{w.x, w.y}));
-    power[k] = x.x * x.x + x.y * x.y;
-  }
-}
-
-__host__ __device__ __forceinline__ void mel_project(int tid, int num_mels,
-                                                     const float* __restrict__ power,
-                                                     const int* __restrict__ mel_start,
-                                                     const int* __restrict__ mel_off,
-                                                     const float* __restrict__ mel_w,
-                                                     float* __restrict__ out_col, int out_stride) {
-  for (int m = tid; m < num_mels; m += kGroupThreads) {
-    const int s = mel_start[m], o = mel_off[m], n = mel_off[m + 1] - o;
-    float acc = 0.f;
-    for (int i = 0; i < n; ++i) acc += mel_w[o + i] * power[s + i];
-    out_col[m * out_stride] = logf(fmaxf(acc, 1e-5f));
-  }
-}
-
 __host__ __device__ __forceinline__ int reflect_index(int i, int t) {
   if (i < 0) i = -i;
   if (i >= t) i = 2 * (t - 1) - i;
@@ -161,44 +124,10 @@ __device__ __forceinline__ void atomic_max_f32(float* addr, float v) {
   else atomicMin(reinterpret_cast<unsigned int*>(addr), __float_as_uint(v));
 }
 
-struct MelArgs {
-  const float* y;
-  float* out;
-  float* minmax;
-  int batch, t, frames, hop, pad, num_mels;
-  const float* window;
-  const float2* tw512;
-  const float2* tw1024;
-  const int* mel_start;
-  const int* mel_off;
-  const float* mel_w;
-  int stage_len;  // samples staged per block = (kFramesPerBlock-1)*hop + n_fft
-  int nnz;        // entries of mel_w
-};
-
-// shared-memory layout of mel_kernel (bytes, every region 16-byte aligned)
-struct MelSmem {
-  uint32_t win, tw512, tw1024, melw, melidx, meloff, buf0, buf1, outs, total;
-};
-__host__ __device__ inline MelSmem mel_smem_layout(int stage_len, int num_mels, int nnz) {
-  auto up = [](uint32_t v) { return (v + 15u) & ~15u; };
-  MelSmem l;
-  uint32_t o = up(static_cast<uint32_t>(stage_len) * 4u);
-  l.win = o;    o += kNfft * 4u;
-  l.tw512 = o;  o += kHalf * 8u;
-  l.tw1024 = o; o += up((kHalf + 1) * 8u);
-  l.melw = o;   o += up(static_cast<uint32_t>(nnz > 0 ? nnz : 1) * 4u);
-  l.melidx = o; o += up(static_cast<uint32_t>(num_mels) * 4u);            // mel_start
-  l.meloff = o; o += up(static_cast<uint32_t>(num_mels + 1) * 4u);        // mel_off
-  l.buf0 = o;   o += kGroups * kPadLen * 8u;
-  l.buf1 = o;   o += kGroups * kPadLen * 8u;
-  l.outs = o;   o += static_cast<uint32_t>(num_mels) * kFramesPerBlock * 4u;
-  l.total = o;
-  return l;
-}
 // asynchronous global -> shared copies (LDGSTS): every copy of the block prologue is in flight at once, so the
-// prologue costs one memory round trip instead of one per dependent load / store pair (ncu source view: the
-// staging stores waiting on their loads, and the barrier behind them, were ~25 % of this kernel's stall samples)
+// prologue costs one memory round trip instead of one per dependent load / store pair (ncu source view of the
+// round-1 forward kernel: the staging stores waiting on their loads, and the barrier behind them, were ~25 % of its
+// stall samples)
 __device__ __forceinline__ void cp_async16(void* dst_smem, const void* src) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(hg::smem_u32(dst_smem)), "l"(src) : "memory");
 }
@@ -219,93 +148,6 @@ __device__ __forceinline__ void group_sync(int g) {
   asm volatile("bar.sync %0, %1;" ::"r"(g + 1), "n"(kGroupThreads) : "memory");
 }
 
-__global__ void __launch_bounds__(kMelThreads) mel_kernel(const MelArgs a) {
-  extern __shared__ __align__(16) uint8_t sm[];
-  const MelSmem L = mel_smem_layout(a.stage_len, a.num_mels, a.nnz);
-  float* stage = reinterpret_cast<float*>(sm);                                 // [stage_len]
-  float* s_win = reinterpret_cast<float*>(sm + L.win);                         // tables: read ~18 KB per frame
-  float2* s_tw512 = reinterpret_cast<float2*>(sm + L.tw512);                   //   from L1 / L2 otherwise
-  float2* s_tw1024 = reinterpret_cast<float2*>(sm + L.tw1024);
-  float* s_melw = reinterpret_cast<float*>(sm + L.melw);
-  int* s_start = reinterpret_cast<int*>(sm + L.melidx);
-  int* s_off = reinterpret_cast<int*>(sm + L.meloff);
-  cpx* buf0 = reinterpret_cast<cpx*>(sm + L.buf0);                             // [groups][kPadLen]
-  cpx* buf1 = reinterpret_cast<cpx*>(sm + L.buf1);                             // [groups][kPadLen]
-  float* outs = reinterpret_cast<float*>(sm + L.outs);                         // [num_mels][frames per block]
-
-  const int b = blockIdx.y;
-  const int f0 = blockIdx.x * kFramesPerBlock;
-  const int tid = threadIdx.x;
-  const float* yb = a.y + static_cast<size_t>(b) * a.t;
-  const int base = f0 * a.hop - a.pad;
-  // samples actually used by this block's frames (the last block of an item may hold fewer than 16 frames)
-  const int nfr = min(kFramesPerBlock, a.frames - f0);
-  const int used = (nfr - 1) * a.hop + kNfft;
-  const bool interior = base >= 0 && base + used <= a.t && ((a.t | base) & 3) == 0 &&
-                        (reinterpret_cast<uintptr_t>(a.y) & 15) == 0;
-  if (interior) {
-    // no reflection, 16-byte aligned: straight vector copies
-    const int n16 = used >> 2;
-    for (int i = tid; i < n16; i += kMelThreads) cp_async16(stage + 4 * i, yb + base + 4 * i);
-    for (int i = n16 * 4 + tid; i < used; i += kMelThreads) cp_async4(stage + i, yb + base + i);
-  } else {
-    for (int i = tid; i < used; i += kMelThreads) cp_async4(stage + i, yb + reflect_index(base + i, a.t));
-  }
-  cp_async_table(s_win, a.window, kNfft * 4, tid, kMelThreads);
-  cp_async_table(s_tw512, a.tw512, kHalf * 8, tid, kMelThreads);
-  cp_async_table(s_tw1024, a.tw1024, (kHalf + 1) * 8, tid, kMelThreads);
-  cp_async_table(s_melw, a.mel_w, a.nnz * 4, tid, kMelThreads);
-  cp_async_table(s_start, a.mel_start, a.num_mels * 4, tid, kMelThreads);
-  cp_async_table(s_off, a.mel_off, (a.num_mels + 1) * 4, tid, kMelThreads);
-  cp_async_wait_all();
-  __syncthreads();
-  if (a.minmax) {
-    float vmin = INFINITY, vmax = -INFINITY;
-    for (int i = tid; i < used; i += kMelThreads) {
-      const float v = stage[i];
-      vmin = fminf(vmin, v);
-      vmax = fmaxf(vmax, v);
-    }
-    for (int o = 16; o > 0; o >>= 1) {
-      vmin = fminf(vmin, __shfl_xor_sync(0xffffffffu, vmin, o));
-      vmax = fmaxf(vmax, __shfl_xor_sync(0xffffffffu, vmax, o));
-    }
-    // almost every warp loses against the running extrema: peek first (a stale read only costs one
-    // redundant atomic), otherwise 2 x 16 same-address atomics per block serialise in L2
-    if ((tid & 31) == 0) {
-      if (vmin < *reinterpret_cast<volatile float*>(a.minmax)) atomic_min_f32(a.minmax, vmin);
-      if (vmax > *reinterpret_cast<volatile float*>(a.minmax + 1)) atomic_max_f32(a.minmax + 1, vmax);
-    }
-  }
-
-  const int g = tid / kGroupThreads, j = tid % kGroupThreads;
-  cpx* z0 = buf0 + g * kPadLen;
-  cpx* z1 = buf1 + g * kPadLen;
-  for (int it = 0; it < kFramesPerBlock / kGroups; ++it) {
-    const int fl = it * kGroups + g;  // frame within the block
-    if (fl >= nfr) break;             // group-uniform: the whole group leaves together
-    const float* smp = stage + fl * a.hop;
-    fft_pass<true>(j, 1, nullptr, z0, smp, s_win, s_tw512);
-    group_sync(g);
-    fft_pass<false>(j, 8, z0, z1, nullptr, nullptr, s_tw512);
-    group_sync(g);
-    fft_pass<false>(j, 64, z1, z0, nullptr, nullptr, s_tw512);
-    group_sync(g);
-    float* power = reinterpret_cast<float*>(z1);  // 513 floats fit in the 544-cpx scratch
-    unpack_power(j, z0, power, s_tw1024);
-    group_sync(g);
-    mel_project(j, a.num_mels, power, s_start, s_off, s_melw, outs + fl, kFramesPerBlock);
-    group_sync(g);
-  }
-  __syncthreads();
-  // outs[m][fl] -> out[b][m][f0 + fl]
-  float* ob = a.out + static_cast<size_t>(b) * a.num_mels * a.frames;
-  for (int i = tid; i < a.num_mels * kFramesPerBlock; i += kMelThreads) {
-    const int m = i / kFramesPerBlock, fl = i % kFramesPerBlock;
-    if (f0 + fl < a.frames) ob[static_cast<size_t>(m) * a.frames + f0 + fl] = outs[i];
-  }
-}
-
 // ---------------------------------------------------------------------------------------------
 // mel_kernel2 — the forward kernel of round 2: ONE WARP PER TWO FRAMES, the FFT held in registers.
 //
@@ -321,8 +163,8 @@ __global__ void __launch_bounds__(kMelThreads) mel_kernel(const MelArgs a) {
 //   phase 4  lane = mel bin mod 32: the CSR triangle sums + log(clamp), staged for 64-byte output runs
 // Warps never meet (__syncwarp between phases); a block is 8 warps = 16 consecutive frames and loops over frame
 // groups, so the constant tables are loaded once per block.  ~2.4x fewer warp-instructions per frame than the
-// radix-8 x 8 x 8 shared-memory kernel above (which stays: the backward kernel is built from its passes), and no
-// block-wide or named barriers on the frame path.
+// round-1 radix-8 x 8 x 8 shared-memory kernel (whose FFT passes, fft_pass above, the backward kernel still runs),
+// and no block-wide or named barriers on the frame path.
 // The lane phases are __host__ __device__ (hg_mel_emulate_host runs them lane by lane on the CPU).
 constexpr int kExPitch = 33;                              // complex per (frame, n2) row of the exchange buffer
 constexpr int kWarpScratch = 2 * 16 * kExPitch;           // complex per warp (8448 B) >= 2 x 512 (the Z / power view)
@@ -802,50 +644,29 @@ extern "C" int hg_mel_fwd(const hg_mel_plan* plan, const float* y, int batch, in
     return HG_OK;
   }
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  static const bool use_v1 = getenv("HG_MEL_V1") != nullptr;       // the round-1 kernel, kept for A/B measurements
-  if (!use_v1) {
-    Mel2Args a{};
-    a.y = y; a.out = out; a.minmax = minmax;
-    a.batch = batch; a.t = t; a.frames = frames; a.hop = plan->hop; a.pad = plan->pad;
-    a.num_mels = plan->num_mels;
-    a.window = plan->window; a.tw512 = plan->tw512; a.tw1024 = plan->tw1024;
-    a.mel_start = plan->mel_start; a.mel_off = plan->mel_off; a.mel_w = plan->mel_w;
-    a.nnz = plan->nnz;
-    a.max_bin = 0;
-    for (int m = 0; m < plan->num_mels; ++m) {
-      const int last = plan->h_mel_start[m] + (plan->h_mel_off[m + 1] - plan->h_mel_off[m]) - 1;
-      if (last > a.max_bin) a.max_bin = last;
-    }
-    a.groups_per_item = (frames + kFramesPerBlock - 1) / kFramesPerBlock;
-    a.total_groups = batch * a.groups_per_item;
-    const size_t smem = mel2_smem_layout(plan->num_mels, plan->nnz).total;
-    HG_REQUIRE(smem <= 113 * 1024, "hg_mel_fwd: %zu bytes of shared memory per block", smem);
-    static hg::PerDeviceOnce once2;
-    if (once2.need(smem))
-      HG_CHECK_CUDA(cudaFuncSetAttribute(mel_kernel2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int dev = 0, sms = 148;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int grid = a.total_groups < 2 * sms ? a.total_groups : 2 * sms;   // two resident blocks per SM, looping
-    mel_kernel2<<<grid, kMel2Threads, smem, st>>>(a);
-    HG_CHECK_CUDA(cudaGetLastError());
-    g_hg_launches.fetch_add(1, std::memory_order_relaxed);
-    return HG_OK;
-  }
-  MelArgs a{};
+  Mel2Args a{};
   a.y = y; a.out = out; a.minmax = minmax;
   a.batch = batch; a.t = t; a.frames = frames; a.hop = plan->hop; a.pad = plan->pad;
   a.num_mels = plan->num_mels;
   a.window = plan->window; a.tw512 = plan->tw512; a.tw1024 = plan->tw1024;
   a.mel_start = plan->mel_start; a.mel_off = plan->mel_off; a.mel_w = plan->mel_w;
-  a.stage_len = (kFramesPerBlock - 1) * plan->hop + plan->n_fft;
   a.nnz = plan->nnz;
-  const size_t smem = mel_smem_layout(a.stage_len, plan->num_mels, plan->nnz).total;
-  HG_REQUIRE(smem <= 227 * 1024, "hg_mel_fwd: hop_size %d needs %zu bytes of shared memory", plan->hop, smem);
-  static hg::PerDeviceOnce once;
-  if (once.need(smem))
-    HG_CHECK_CUDA(cudaFuncSetAttribute(mel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  dim3 grid((frames + kFramesPerBlock - 1) / kFramesPerBlock, batch);
-  mel_kernel<<<grid, kMelThreads, smem, st>>>(a);
+  a.max_bin = 0;
+  for (int m = 0; m < plan->num_mels; ++m) {
+    const int last = plan->h_mel_start[m] + (plan->h_mel_off[m + 1] - plan->h_mel_off[m]) - 1;
+    if (last > a.max_bin) a.max_bin = last;
+  }
+  a.groups_per_item = (frames + kFramesPerBlock - 1) / kFramesPerBlock;
+  a.total_groups = batch * a.groups_per_item;
+  const size_t smem = mel2_smem_layout(plan->num_mels, plan->nnz).total;
+  HG_REQUIRE(smem <= 113 * 1024, "hg_mel_fwd: %zu bytes of shared memory per block", smem);
+  static hg::PerDeviceOnce once2;
+  if (once2.need(smem))
+    HG_CHECK_CUDA(cudaFuncSetAttribute(mel_kernel2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int dev = 0, sms = 148;
+  if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int grid = a.total_groups < 2 * sms ? a.total_groups : 2 * sms;   // two resident blocks per SM, looping
+  mel_kernel2<<<grid, kMel2Threads, smem, st>>>(a);
   HG_CHECK_CUDA(cudaGetLastError());
   g_hg_launches.fetch_add(1, std::memory_order_relaxed);
   return HG_OK;
@@ -853,7 +674,7 @@ extern "C" int hg_mel_fwd(const hg_mel_plan* plan, const float* y, int batch, in
 
 // ---------------------------------------------------------------------------------------------
 // mel_spectrogram backward (the generated-mel L1 term of the generator loss, UPSTREAM train.py: F.l1_loss(y_mel,
-// y_g_hat_mel) * 45 through src/meldataset.py:78-83).  One 64-thread group per frame, the forward kernel's own FFT:
+// y_g_hat_mel) * 45 through src/meldataset.py:78-83).  One 64-thread group per frame, the radix-8 FFT of fft_pass:
 //   recompute Z = FFT512(packed windowed frame), un-pack X[0..512] (kept complex) and |X|^2, the CSR mel sums;
 //   dmel = g / mel above the 1e-5 clamp (0 below), dP[k] = sum_m fb[m][k] dmel[m], G[k] = 2 dP[k] X[k];
 //   the gradient at the windowed samples is S[n] = Re sum_{k=0..512} G[k] e^{+2 pi i k n / 1024}: the real inverse

@@ -389,7 +389,7 @@ extern "C" int hg_conv_post_tanh_fwd(const void* x, const float* w, const float*
   HG_REQUIRE(batch > 0 && t > 0 && c > 0 && c % 8 == 0 && k > 0 && (k & 1) && k <= 15,
              "hg_conv_post_tanh_fwd: bad shape (c %% 8 == 0, odd k <= 15 required)");
   HG_REQUIRE(batch <= 65535, "hg_conv_post_tanh_fwd: batch too large");
-  if (c == 32 && k == 7 && !getenv("HG_POST_V1")) {       // every shipped config (conv_post: 32 -> 1, k = 7)
+  if (c == 32 && k == 7) {  // every shipped config (conv_post: 32 -> 1, k = 7)
     // 64 threads x 9 outputs per block (42 KB of staged rows, 5 blocks per SM): 0.486 ms per 16.8 M samples against
     // 0.609 ms with 128 threads and 0.781 ms for the kernel above (profiles/r02_summary.md section 4)
     const int rc = launch_post2<64>(static_cast<const __nv_bfloat16*>(x), w, bias, batch, t, y,

@@ -553,8 +553,7 @@ extern "C" int hg_resblock_pair_fwd(const void* x, const void* w1_packed, const 
   rc = hg_encode_tmap_bf16_3d(&tw2, single ? w1_packed : w2_packed, c, c, ktaps, static_cast<uint64_t>(c) * 2,
                               static_cast<uint64_t>(c) * c * 2, c, c, ktaps, swz);
   if (rc) return rc;
-  const int sms = hg::cap_ctas(g_sms);
-  const int grid = p.num_tiles < sms ? p.num_tiles : sms;
+  const int grid = p.num_tiles < g_sms ? p.num_tiles : g_sms;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (single)
     rc = (c == 64) ? launch_pair<64, true>(tx, tw1, tw2, p, smem_bytes, grid, st)

@@ -463,25 +463,6 @@ __global__ void loss_grad_kernel(const float* __restrict__ a, const float* __res
   }
 }
 
-// sum |a - b| over bf16 arrays (feature maps in their internal layout; zero padding rows contribute nothing)
-__global__ void __launch_bounds__(256)
-l1_sum_bf16_kernel(const __nv_bfloat16* __restrict__ a, const __nv_bfloat16* __restrict__ b, long long n8,
-                   float* __restrict__ out) {
-  __shared__ float red[32];
-  float acc = 0.f;
-  for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n8; i += 256LL * gridDim.x) {
-    const uint4 av = reinterpret_cast<const uint4*>(a)[i], bv = reinterpret_cast<const uint4*>(b)[i];
-    const uint32_t aw[4] = {av.x, av.y, av.z, av.w}, bw[4] = {bv.x, bv.y, bv.z, bv.w};
-#pragma unroll
-    for (int h = 0; h < 4; ++h) {
-      const float2 x = hg::unpack_bf16x2(aw[h]), y = hg::unpack_bf16x2(bw[h]);
-      acc += fabsf(x.x - y.x) + fabsf(x.y - y.y);
-    }
-  }
-  acc = block_sum(acc, red);
-  if (threadIdx.x == 0) atomicAdd(out, acc);
-}
-
 struct UnpackArgs {
   int mode;          // 0: Conv1d, 1: ConvTranspose1d (polyphase)
   int d0, d1, k;     // parameter shape [d0][d1][k]  (conv: cout, cin/groups; convtr: cin, cout)
@@ -931,15 +912,6 @@ extern "C" int hg_loss_grad(const float* a, const float* b, long long n, int mod
   return HG_OK;
 }
 
-extern "C" int hg_l1_sum_bf16(const void* a, const void* b, long long n, float* out_acc, void* stream) {
-  HG_REQUIRE(a && b && out_acc && n > 0 && n % 8 == 0, "hg_l1_sum_bf16: n must be a positive multiple of 8");
-  l1_sum_bf16_kernel<<<blocks_for(n / 8), 256, 0, S(stream)>>>(static_cast<const __nv_bfloat16*>(a),
-                                                              static_cast<const __nv_bfloat16*>(b), n / 8, out_acc);
-  HG_CHECK_CUDA(cudaGetLastError());
-  count();
-  return HG_OK;
-}
-
 extern "C" int hg_unpack_wgrad_conv(const float* dw_packed, int cout, int cin_g, int k, int rows_p, int cin_tile,
                                     int cout_g, int merge, const int* host_tap_order, float* dw, void* stream) {
   HG_REQUIRE(dw_packed && dw && k > 0 && k <= 64 && cout > 0 && cin_g > 0 && merge >= 1 && cout_g >= 1,
@@ -949,21 +921,6 @@ extern "C" int hg_unpack_wgrad_conv(const float* dw_packed, int cout, int cin_g,
   a.cout_g = cout_g; a.merge = merge;
   for (int q = 0; q < k; ++q) a.pos[host_tap_order ? host_tap_order[q] : q] = q;
   unpack_wgrad_kernel<<<blocks_for(static_cast<long long>(cout) * cin_g * k), 256, 0, S(stream)>>>(dw_packed, a, dw);
-  HG_CHECK_CUDA(cudaGetLastError());
-  count();
-  return HG_OK;
-}
-
-extern "C" int hg_unpack_wgrad_convtr(const float* dw_packed, int cin, int cout, int k, int stride, int padding,
-                                      int cin_p, int cout_p, float* dw, void* stream) {
-  HG_REQUIRE(dw_packed && dw && k > 0 && cin > 0 && cout > 0 && stride > 0, "hg_unpack_wgrad_convtr: bad arguments");
-  int nshift = 0, smin = 0;
-  int rc = hg_convtr1d_geometry(k, stride, padding, &nshift, &smin);
-  if (rc) return rc;
-  UnpackArgs a{};
-  a.mode = 1; a.d0 = cin; a.d1 = cout; a.k = k; a.rows_p = stride * cout_p; a.cin_tile = cin_p;
-  a.stride = stride; a.padding = padding; a.shift_min = smin; a.cout_p = cout_p;
-  unpack_wgrad_kernel<<<blocks_for(static_cast<long long>(cin) * cout * k), 256, 0, S(stream)>>>(dw_packed, a, dw);
   HG_CHECK_CUDA(cudaGetLastError());
   count();
   return HG_OK;
@@ -1079,7 +1036,7 @@ extern "C" int hg_spectral_norm_bwd(const float* dw_eff, const float* w_eff, con
   return HG_OK;
 }
 
-// hg_wgrad_finish_*: hg_unpack_wgrad_* + hg_weight_norm_bwd fused (one launch per layer).  v, g: the module's
+// hg_wgrad_finish_*: the packed-gradient unpack + hg_weight_norm_bwd fused (one launch per layer).  v, g: the module's
 // weight_v / weight_g (g == NULL: plain `weight`, dv receives the unpacked gradient).
 extern "C" int hg_wgrad_finish_conv(const float* dw_packed, int cout, int cin_g, int k, int rows_p, int cin_tile,
                                     int cout_g, int merge, const int* host_tap_order, const float* v, const float* g,

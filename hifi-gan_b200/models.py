@@ -439,7 +439,6 @@ class _GeneratorEngine:
         for n in names:
             ws[n] = bf(biggest)
         ws["y"] = torch.empty(batch, 1, t, dtype=torch.float32, device=dev)
-        ws["_biggest"] = biggest
         if len(self.ws) >= 8:  # bound the cache: workspaces for config 2 are ~10 GB
             old = next(iter(self.ws))
             self.ws.pop(old)
@@ -466,7 +465,7 @@ class _GeneratorEngine:
         use_graph = (not time_convs and lengths is None and b * t_out <= self.GRAPH_MAX_SAMPLES
                      and not os.environ.get("HG_DISABLE_GRAPHS") and not torch.cuda.is_current_stream_capturing())
         if not use_graph:
-            return self._launch(xin, time_convs, lengths, lanes=b * t_out > self.GRAPH_MAX_SAMPLES)
+            return self._launch(xin, time_convs, lengths)
         key = (b, frames, _FUSE_PAIRS)
         entry = self.graphs.get(key)
         if entry is None:
@@ -498,59 +497,12 @@ class _GeneratorEngine:
         graph.replay()
         return out
 
-    # ---- MRF lanes: the nk branches of a stage side by side on disjoint SM subsets --------------------------------
-    # The branches of one stage (src/models.py:106-111) read the same x and are independent until their mean.  At
-    # large batch every launch is a persistent grid over all SMs, so run back to back the HBM-bound k = 3 chain
-    # leaves the tensor pipes idle and the tensor-bound k = 11 chain leaves HBM idle.  Each branch gets its own
-    # stream, its own ping-pong buffers and a share of the SMs (hg_set_cta_limit) proportional to its measured
-    # run time; the last branch's final launch (which adds the other branches' results) runs after the join on
-    # the whole GPU.  The first call of a shape runs the branches one after the other and times them.
-    # MEASURED (tests/lanes_ab.py, profiles/r02_summary.md section 4): bit-identical output, 56.9 ms against 56.2 ms one
-    # after the other at 64 x 1024 frames — the step is bound by SM-time under the power cap, not by idle HBM or
-    # tensor pipes — so the schedule is opt-in (HG_MRF_LANES=1, or "a,b,c" for a fixed CTA split).
-    LANE_MIN_CTAS = 8
-    LANE_CALIB_CALLS = 3      # call 1: branches alone; calls 2-3: side by side, split re-balanced from their run times
-
-    def _lane_state(self, ws, nk: int):
-        st = ws.get("_lanes")
-        if st is None:
-            dev = self.device
-            bf = lambda: torch.empty(ws["_biggest"], dtype=torch.bfloat16, device=dev)
-            bufs = [ws] + [dict(ws, **{n: bf() for n in ("t1", "a_raw", "a_act", "b_raw", "b_act")})
-                           for _ in range(nk - 1)]
-            forced = os.environ.get("HG_MRF_LANES", "")
-            st = dict(streams=[torch.cuda.Stream(device=dev) for _ in range(nk)], bufs=bufs, split=None, phase=0,
-                      forced=[int(v) for v in forced.split(",")] if "," in forced else None)
-            ws["_lanes"] = st
-        return st
-
-    @staticmethod
-    def _split_ctas(weights: List[float], total: int, floor: int) -> List[int]:
-        """even CTA counts proportional to `weights`, each >= floor, summing to `total` (CTA pairs stay whole)"""
-        tot = sum(weights) or 1.0
-        half = total // 2
-        s = [max(floor // 2, int(round(half * w / tot))) for w in weights]
-        while sum(s) > half:
-            s[s.index(max(s))] -= 1
-        while sum(s) < half:
-            s[weights.index(max(weights))] += 1
-        return [2 * v for v in s]
-
-    def _launch(self, xin: torch.Tensor, time_convs: bool, lengths: Optional[torch.Tensor] = None,
-                lanes: bool = False) -> torch.Tensor:
+    def _launch(self, xin: torch.Tensor, time_convs: bool, lengths: Optional[torch.Tensor] = None) -> torch.Tensor:
         L = _lib.lib()
         gen = self.gen
         b, c, frames = xin.shape
         ws = self.workspace(b, frames)
         nk = gen.num_kernels
-        lanes = bool(lanes and 2 <= nk <= 3 and os.environ.get("HG_MRF_LANES", "0") != "0")
-        lane = self._lane_state(ws, nk) if lanes else None
-        sms = torch.cuda.get_device_properties(self.device).multi_processor_count
-        if lane is not None and lane["forced"] is not None:
-            lane["split"], lane["phase"] = [lane["forced"]] * len(self.ups), self.LANE_CALIB_CALLS
-        measure = lane is not None and lane["phase"] < self.LANE_CALIB_CALLS      # time every branch
-        marks: List[list] = []
-        main = torch.cuda.current_stream()
         lp = 0 if lengths is None else lengths.data_ptr()     # ragged batch: per-item frame counts (device int32)
         mul = 1                                                # rows per frame at the current stage
         _lib.check(L.hg_ncl_to_nlc(xin.data_ptr(), b, c, frames, self.pre.cin_p, ws["mel"].data_ptr(), 0, 0.0,
@@ -572,12 +524,6 @@ class _GeneratorEngine:
             c_p = up.cout_p
             last_stage = i == len(self.ups) - 1
             out_slope = 0.01 if last_stage else LRELU_SLOPE  # models.py:112 uses the default slope
-            side = lane is not None and lane["split"] is not None      # this call runs the branches side by side
-            deferred: List[dict] = []
-            stage_marks = []
-            if side:
-                fork = torch.cuda.Event()
-                fork.record(main)
             for j in range(nk):
                 blk = gen.resblocks[i * nk + j]
                 packs = self.blocks[i * nk + j]
@@ -598,29 +544,7 @@ class _GeneratorEngine:
                     else:
                         _conv(L, kw["x"], kw["pc"], b, t, res=(kw["res0"],) + others, item=(lp, mul), **outs)
 
-                if lane is None:
-                    _resblock_chain(L, blk, packs, b, t, c_p, ws["x_raw"], ws["x_act"], ws, final, item=(lp, mul))
-                    continue
-                # the last branch's final launch needs the other branches' results: it runs after the join
-                fin = final if j < nk - 1 else deferred.append
-                stream = lane["streams"][j] if side else main
-                e0, e1 = torch.cuda.Event(enable_timing=measure), torch.cuda.Event(enable_timing=measure)
-                with torch.cuda.stream(stream):
-                    if side:
-                        stream.wait_event(fork)
-                        L.hg_set_cta_limit(lane["split"][i][j])
-                    e0.record()
-                    _resblock_chain(L, blk, packs, b, t, c_p, ws["x_raw"], ws["x_act"], lane["bufs"][j], fin,
-                                    item=(lp, mul))
-                    e1.record()
-                stage_marks.append((e0, e1))
-            if lane is not None:
-                L.hg_set_cta_limit(0)
-                if side:
-                    for _, e1 in stage_marks:
-                        main.wait_event(e1)
-                final(deferred[0], nk - 1)
-                marks.append(stage_marks)
+                _resblock_chain(L, blk, packs, b, t, c_p, ws["x_raw"], ws["x_act"], ws, final, item=(lp, mul))
             cur = ws["stage_out"]
         if time_convs:
             ev1.record()
@@ -629,14 +553,6 @@ class _GeneratorEngine:
         _lib.check(L.hg_conv_post_tanh_fwd(cur.data_ptr(), self.post_w.data_ptr(), self.post_b.data_ptr(), b, t,
                                            self.post_cin_p, post.kernel_size[0], ws["y"].data_ptr(), _stream()),
                    "hg_conv_post_tanh_fwd")
-        if measure:
-            # the first call timed the branches alone on all SMs, the next ones side by side on the previous split:
-            # SM-time of a branch = its run time x the CTAs it had; the next split is proportional to that
-            torch.cuda.synchronize(self.device)
-            had = lane["split"] or [[sms] * nk] * len(self.ups)
-            work = [[e0.elapsed_time(e1) * had[i][j] for j, (e0, e1) in enumerate(sm)] for i, sm in enumerate(marks)]
-            lane["split"] = [self._split_ctas(w, sms - (sms & 1), self.LANE_MIN_CTAS) for w in work]
-            lane["phase"] += 1
         return ws["y"]
 
 

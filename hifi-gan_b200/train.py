@@ -720,13 +720,13 @@ class _SubDiscTrainer:
         # is independent of the other layers': spread over W_CHAINS lanes instead of one.  (One lane made this the
         # longest dependent chain of the whole step: 3.9 ms for 2 x 8 layers, profiles/r02_summary.md section 2.)
         # weight_norm sub-discriminators: one lane (measured with 1 / 2 / 4 / 8: 12.01 / 12.01 / 12.06-12.12 / 12.10 ms —
-        # their chains are short and the phase is bound by SM-time; HG_W_CHAINS overrides)
-        self.n_chains = self.W_CHAINS if self.spectral else max(1, int(os.environ.get("HG_W_CHAINS", 1)))
+        # their chains are short and the phase is bound by SM-time)
+        self.n_chains = self.W_CHAINS if self.spectral else 1
         self.wl = _Lanes(self.n_chains, device, [0 + boost] * self.n_chains)
         self._scr = {}
         self.ws = {}
-        # packed fp32 weight gradients, one region per wide layer (zeroed once per backward; the wgrad launches and
-        # the batched finish accumulate)
+        # packed fp32 weight gradients, one region per wide layer (zeroed once per backward; the wgrad launches
+        # accumulate)
         sizes = [l.k * l.cout * l.cin_tile for l in self.mids]
         self.dwp_flat = torch.zeros(sum(sizes), dtype=torch.float32, device=device)
         self.dwps, off = [], 0
@@ -734,9 +734,6 @@ class _SubDiscTrainer:
             self.dwps.append(self.dwp_flat[off:off + n])
             off += n
         self._tables = {}
-        # A/B switches for profiles/r02_summary.md: per-layer launches (the round-1 scheme) instead of the batched ones
-        self.batch_prep = os.environ.get("HG_BATCH_D_PREP", "1") != "0"
-        self.batch_finish = os.environ.get("HG_BATCH_D_FINISH", "0") != "0"   # measured: +0.3 ms when batched (waits for the last wgrad)
         self.db = torch.zeros(1024, dtype=torch.float32, device=device)
         self.db_unused = torch.zeros(1024, dtype=torch.float32, device=device)    # the first conv's discarded bias column
         self.wbufs = {}
@@ -759,10 +756,9 @@ class _SubDiscTrainer:
             buf = self._scr[chain] = torch.empty(w.numel(), dtype=torch.float32, device=self.device)
         return buf
 
-    def _weights(self, part: int, only_buffers: bool = False):
-        """effective fp32 weights + forward GEMM packs of every layer, into per-part persistent buffers.
-        weight_norm layers: hg_fold_weight_norm + hg_pack_disc_weight.  spectral_norm layers: one power iteration
-        per call in train mode (torch ops on the u / v buffers, exactly like one reference forward)."""
+    def _weights(self, part: int):
+        """per-part persistent buffers of every layer's effective fp32 weight and forward GEMM pack; _weights_layer
+        and the table's "fwd" launch fill them"""
         bufs = self.wbufs.get(part)
         if bufs is None:
             bufs = {"eff": [], "fwd": []}
@@ -777,18 +773,12 @@ class _SubDiscTrainer:
                 else:
                     bufs["fwd"].append(None)
             self.wbufs[part] = bufs
-        ws = {"eff": bufs["eff"], "fwd": bufs["fwd"], "sn": [None] * len(self.mods)}
-        if only_buffers:
-            return ws
-        for li in range(len(self.mods)):
-            self._weights_layer(ws, bufs, li)
-        return ws
+        return {"eff": bufs["eff"], "fwd": bufs["fwd"], "sn": [None] * len(self.mods)}
 
     def _table(self, part: int):
         """Job table of part / call slot `part` (batched.py): phase "fwd" = weight_norm fold -> effective fp32 weight +
         forward bank of every layer (spectral-norm layers: forward bank from the effective weight their power
-        iteration produced), "dgrad" = the polyphase data-gradient banks, "finish" = packed dW -> (weight_g.grad,
-        weight_v.grad) of every wide weight_norm layer.  One launch each instead of one per layer."""
+        iteration produced), "dgrad" = the polyphase data-gradient banks.  One launch each instead of one per layer."""
         t = self._tables.get(part)
         if t is not None:
             return t
@@ -825,13 +815,6 @@ class _SubDiscTrainer:
                                        layer.stride, layer.pad, bl.nshift, bl.smin, cout_tile, tci, layer.cin // tci))
             else:
                 self.untiled.append(li - 1)
-            if not sn:
-                pos = [0] * layer.k
-                for q, j in enumerate(layer.order):
-                    pos[j] = q
-                t.add("finish", batched.FINISH_ROW, layer.cout, cin_g * layer.k * 4, self.dwps[li - 1], g, v,
-                      self.flat.grad(v), self.flat.grad(g), ints=(0, layer.cout, cin_g, layer.k, layer.cout, layer.cin_tile,
-                                    layer.cout // layer.groups, layer.merge, 0, 0, 0, 0, 1), tab=pos)
         self._tables[part] = t.finalize()
         return t
 
@@ -839,10 +822,10 @@ class _SubDiscTrainer:
         """effective weights + forward banks of part `part` on the current stream: spectral-norm layers run their
         power iteration (one per call in train mode, like the reference's hook), then ONE batched launch folds /
         packs every layer"""
-        W = self._weights(part, only_buffers=True)
+        W = self._weights(part)
         if self.spectral:
             for li in range(len(self.mods)):
-                self._weights_layer(W, self.wbufs[part], li, pack=False)
+                self._weights_layer(W, self.wbufs[part], li)
         self._table(part).launch("fwd")
         return W
 
@@ -854,12 +837,12 @@ class _SubDiscTrainer:
         lanes' persistent tensor-core kernels (measured: 0.98 -> 3.0 ms for chains that take 0.2 ms on a quiet GPU)."""
         if not self.spectral:
             return
-        Ws = [self._weights(pi, only_buffers=True) for pi in range(2)]
+        Ws = [self._weights(pi) for pi in range(2)]
         self.prep.fork()
         for li in range(len(self.mods)):
             with self.prep.lane(li):
                 for pi, W in enumerate(Ws):
-                    self._weights_layer(W, self.wbufs[pi], li, pack=False)
+                    self._weights_layer(W, self.wbufs[pi], li)
         p0 = self.prep.streams[0]
         for s_ in self.prep.streams[1:]:
             p0.wait_stream(s_)
@@ -868,8 +851,8 @@ class _SubDiscTrainer:
                 self._table(pi).launch("fwd")
         self._prefetched = Ws
 
-    def _weights_layer(self, ws, bufs, li: int, pack: bool = True) -> None:
-        """fold (weight norm) or power-iterate (spectral norm) layer li and pack its forward filter bank"""
+    def _weights_layer(self, ws, bufs, li: int) -> None:
+        """fold (weight norm) or power-iterate (spectral norm) layer li into its effective fp32 weight"""
         L = _lib.lib()
         st = _stream()
         m = self.mods[li]
@@ -893,11 +876,6 @@ class _SubDiscTrainer:
             g, v = _g_v(m)
             _lib.check(L.hg_fold_weight_norm(v.data_ptr(), 0 if g is None else g.data_ptr(), v.shape[0],
                                              v.numel() // v.shape[0], eff.data_ptr(), st), "hg_fold_weight_norm")
-        if pack and 1 <= li <= len(self.mids):
-            layer = self.mids[li - 1]
-            _lib.check(L.hg_pack_disc_weight(eff.data_ptr(), layer.cout, layer.cin, layer.groups, layer.merge,
-                                             layer.k, layer.stride, layer.pad, bufs["fwd"][li].data_ptr(), 0, st),
-                       "hg_pack_disc_weight")
 
     def _geometry(self, nb: int, t: int, slot: int = 0):
         key = (nb, t, slot)
@@ -984,24 +962,17 @@ class _SubDiscTrainer:
                 # per layer: the second call continues from the first's u, v): side by side on the prep lanes.  (Batched
                 # per stage over all layers, or as one cluster launch, they were slower: a many-block launch on this
                 # lane waits for whole tensor-core kernels of the other lanes to drain — profiles/r02_summary.md.)
-                Ws = [self._weights(pi, only_buffers=True) for pi in range(len(parts))]
+                Ws = [self._weights(pi) for pi in range(len(parts))]
                 self.prep.fork()
                 for li in range(len(self.mods)):
                     with self.prep.lane(li):
                         for pi, W in enumerate(Ws):
-                            self._weights_layer(W, self.wbufs[pi], li, pack=False)
+                            self._weights_layer(W, self.wbufs[pi], li)
                 self.prep.join()
                 for pi in range(len(parts)):
                     self._table(pi).launch("fwd")
-            elif self.batch_prep:
-                Ws = [self._prepare_weights(0)]
             else:
-                Ws = [self._weights(0, only_buffers=True)]
-                self.prep.fork()
-                for li in range(len(self.mods)):
-                    with self.prep.lane(li):
-                        self._weights_layer(Ws[0], self.wbufs[0], li)
-                self.prep.join()
+                Ws = [self._prepare_weights(0)]
             self.W_cached = Ws[-1]
             self.fwd_valid = True
         else:
@@ -1137,15 +1108,11 @@ class _SubDiscTrainer:
 
     def _pack_dgrad(self, W, part: int = 0) -> None:
         if self.spectral or not self.dgrad_valid:
-            if self.batch_prep:
-                t = self._table(part)
-                if t.has("dgrad"):
-                    t.launch("dgrad")
-                for i in self.untiled:
-                    self._bwd_bank(part)[i].pack(W["eff"][1 + i])
-            else:
-                for bl, w_eff in zip(self._bwd_bank(part), W["eff"][1:-1]):
-                    bl.pack(w_eff)
+            t = self._table(part)
+            if t.has("dgrad"):
+                t.launch("dgrad")
+            for i in self.untiled:
+                self._bwd_bank(part)[i].pack(W["eff"][1 + i])
             self.dgrad_valid = True
 
     # ---- one module call under torch autograd (autograd.py): forward with its own activation / weight slot ---------
@@ -1260,7 +1227,7 @@ class _SubDiscTrainer:
                     st = _stream()
                     sn = hasattr(m, "weight_orig")
                     # weight_norm layers: dwps[li] was zeroed with the whole region (zero_wgrads) and is finished by
-                    # the batched launch below; the spectral-norm scale's two halves each need their own sigma, so
+                    # hg_wgrad_finish_conv below; the spectral-norm scale's two halves each need their own sigma, so
                     # they start from zero and are routed layer by layer
                     _lib.check(L.hg_conv1d_wgrad(a_in[seq0:].data_ptr(), d_out.data_ptr(), 1, nseq * rows_in, layer.cin,
                                                  nseq * rows_out, nseq * rows_out, layer.groups_eff, layer.cout,
@@ -1274,7 +1241,7 @@ class _SubDiscTrainer:
                                                           layer.merge, order, scratch.data_ptr(), st),
                                    "hg_unpack_wgrad_conv")
                         self._route(L, m, scratch, layer.cout, cin_g * layer.k, W, 1 + li, True)
-                    elif not self.batch_finish:
+                    else:
                         g, v = _g_v(m)          # unpack + weight_norm backward in one launch, accumulating
                         _lib.check(L.hg_wgrad_finish_conv(self.dwps[li].data_ptr(), layer.cout, cin_g, layer.k,
                                                           layer.cout, layer.cin_tile, layer.cout // layer.groups,
@@ -1285,10 +1252,6 @@ class _SubDiscTrainer:
             bwd[li].dgrad(L, d_out, nseq, h_out, rows_out, rows_in, a_in[seq0:],
                           a_in[seq0 - nr:] if fm else None, nfm[li] if fm else 0.0, G["grad"][li][seq0:], _stream(),
                           flat_h_in=h_in, bias_dst=bias_of(li), pre_add=pre[li])
-        if want_wgrad and not self.spectral and self.batch_finish:
-            for s_ in self.wl.streams[1:]:                       # the batched finish reads every layer's wgrad
-                self.wl.streams[0].wait_stream(s_)
-            side(lambda scratch: self._table(part).launch("finish"), 0)   # every wide layer's unpack + weight_norm backward
         # first conv (Cin = 1)
         k0, s0, p0, c0 = self.first
         m0 = self.mods[0]

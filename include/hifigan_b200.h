@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define HG_ABI_VERSION 2
+#define HG_ABI_VERSION 3
 
 /* Library identity / diagnostics. */
 const char* hg_version(void);
@@ -34,12 +34,6 @@ const char* hg_last_error(void);
 int hg_abi_version(void);
 /* Number of kernel launches issued by this library since load (bench.py's gpu_launches). */
 int64_t hg_launch_count(void);
-/* Cap the persistent grids of hg_conv1d_fwd / hg_resblock_pair_fwd launched afterwards by the CALLING host thread
- * to `max_ctas` CTAs (0 restores one CTA per SM); returns the previous value.  The kernels stride their tile lists
- * by the grid size, so any cap is correct; it exists so that independent launch chains on different streams (the
- * three MRF branches of one Generator stage, src/models.py:106-111) can share the GPU side by side on disjoint SM
- * subsets — an HBM-bound k=3 branch next to a tensor-bound k=11 branch — instead of one after the other. */
-int hg_set_cta_limit(int max_ctas);
 /* Diagnostics: a one-thread kernel on `stream` stores the GPU's %globaltimer (ns) to *dst (device memory).  Unlike a
  * CUDA event it can be read after a graph replay: the training step marks where each discriminator lane finishes its
  * backward, its gradient all-reduce and its generator-step pass (HG_LANE_STAMPS=1, tests/lane_stamps.py). */
@@ -283,18 +277,16 @@ int hg_conv1d_wgrad(const void* x, const void* dy, int batch, int t_in_rows, int
                     int groups, int cout, int ktaps, int stride, int dilation, int pad_left, float* dw_packed,
                     int accumulate, void* stream);
 
-/* Packed weight gradient -> parameter layout.  conv: dw fp32 [cout][cin_g][k] from [k][rows_p][cin_tile]
+/* Packed weight gradient -> parameter layout: dw fp32 [cout][cin_g][k] from [k][rows_p][cin_tile]
  * (host_tap_order = hg_conv1d_tap_order or NULL for identity; merge = groups merged per block-diagonal tile,
- * cout_g = output channels per original group).  convtr: dw fp32 [cin][cout][k] from the polyphase
- * [nshift][stride*cout_p][cin_p]. */
+ * cout_g = output channels per original group). */
 int hg_unpack_wgrad_conv(const float* dw_packed, int cout, int cin_g, int k, int rows_p, int cin_tile, int cout_g,
                          int merge, const int* host_tap_order, float* dw, void* stream);
-int hg_unpack_wgrad_convtr(const float* dw_packed, int cin, int cout, int k, int stride, int padding, int cin_p,
-                           int cout_p, float* dw, void* stream);
 
-/* hg_wgrad_finish_conv / _convtr — hg_unpack_wgrad_* and hg_weight_norm_bwd in ONE launch per layer: packed
- * weight gradient -> (weight_v.grad, weight_g.grad), or -> weight.grad when g == NULL.  Added to the existing
- * values when accumulate != 0. */
+/* hg_wgrad_finish_conv / _convtr — the unpack to parameter layout and hg_weight_norm_bwd in ONE launch per layer:
+ * packed weight gradient -> (weight_v.grad, weight_g.grad), or -> weight.grad when g == NULL.  conv: the layout of
+ * hg_unpack_wgrad_conv; convtr: dw [cin][cout][k] from the polyphase [nshift][stride*cout_p][cin_p].  Added to the
+ * existing values when accumulate != 0. */
 int hg_wgrad_finish_conv(const float* dw_packed, int cout, int cin_g, int k, int rows_p, int cin_tile, int cout_g,
                          int merge, const int* host_tap_order, const float* v, const float* g, int accumulate,
                          float* dv, float* dg, void* stream);
@@ -362,10 +354,10 @@ int hg_spectral_norm_bwd(const float* dw_eff, const float* w_eff, const float* u
  *                          (NULL: plain weight), src2 v -> dst0 dv, dst1 dg (hg_wgrad_finish_conv / _convtr).
  *                          i = {mode (0 conv, 1 convtr), d0, d1, k, rows_p, cin_tile, cout_g, merge, stride, padding,
  *                          shift_min, cout_p, accumulate}, tab = packed position of tap j (conv)
- *   HG_JOB_LOSS_SUM        one block per `chunk` elements: *dst0 += partial sum (the reductions of hg_loss_sum /
- *                          hg_l1_sum_bf16 for many tensors at once).  src0 a, src1 b.  i = {mode (0: fp32 |a - b|,
- *                          1: fp32 (c - a)^2, 2: bf16 |a - b| counted in 16-byte groups), n low 32 bits, n high 32
- *                          bits, chunk, c as float bits}
+ *   HG_JOB_LOSS_SUM        one block per `chunk` elements: *dst0 += partial sum (the reductions of hg_loss_sum and
+ *                          of the bf16 feature maps, for many tensors at once).  src0 a, src1 b.  i = {mode (0: fp32
+ *                          |a - b|, 1: fp32 (c - a)^2, 2: bf16 |a - b| counted in 16-byte groups), n low 32 bits,
+ *                          n high 32 bits, chunk, c as float bits}
  */
 enum {
   HG_JOB_GEN_CONV = 0, HG_JOB_GEN_CONVTR = 1, HG_JOB_GEN_POST = 2, HG_JOB_DISC_ROW = 3, HG_JOB_TRANSPOSE_TILE = 4,
@@ -414,11 +406,9 @@ int hg_avgpool_4_2_2_bwd(const float* dout, int batch, int t, float* din, void* 
 
 /* Loss gradients (src/models.py:251-282 and the mel L1): mode 0 out = coef * sgn(a - b); mode 1 out = coef * (a - c);
  * mode 2 out = coef * (a - c) + coef2 * sgn(a - b).  scale_dev (optional): device scalar multiplied into coef and
- * coef2 (the gradient arriving at the mean, under torch autograd).  hg_l1_sum_bf16: *out_acc += sum |a - b| over
- * bf16 arrays. */
+ * coef2 (the gradient arriving at the mean, under torch autograd). */
 int hg_loss_grad(const float* a, const float* b, long long n, int mode, float c, float coef, float coef2,
                  const float* scale_dev, float* out, void* stream);
-int hg_l1_sum_bf16(const void* a, const void* b, long long n, float* out_acc, void* stream);
 
 /* hg_adamw_step — torch.optim.AdamW on one flat fp32 tensor (decoupled weight decay, bias correction by `step`,
  * or by the device-resident counter *dev_step when non-NULL so that a captured CUDA graph advances it; *dev_lr,

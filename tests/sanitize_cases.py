@@ -7,7 +7,7 @@ missing item 5).  Tool, not a pytest module.
 
 Families: conv (conv1d_tc_kernel, resident + ring weights, strided / grouped), conv2 (conv1d_tc2_kernel, CTA pairs),
 pair (resblock_pair_kernel, C = 32 / 64, one- and two-conv steps), wgrad (wgrad_tc_kernel wide / narrow / grouped),
-mel (mel_kernel, mel_dft_kernel, mel_bwd_kernel), ends (the Cin = 1 / Cout = 1 discriminator kernels, pooling, packs),
+mel (mel_kernel2, mel_dft_kernel, mel_bwd_kernel), ends (the Cin = 1 / Cout = 1 discriminator kernels, pooling, packs),
 step (one whole TrainStep at batch 1: every kernel of the training path, lanes included).
 Each case also checks its result against torch so a sanitizer-clean but wrong kernel cannot pass.  Shapes are the
 smallest that still exercise every code path (ring wrap-around, several tiles per CTA, partial last tile).

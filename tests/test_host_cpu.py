@@ -126,7 +126,7 @@ def test_losses_have_no_cpu_path():
 
 
 # ------------------------------------------------------------------------------------------- C-ABI surface
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_at_abi_3():
     header = open(os.path.join(ROOT, "include", "hifigan_b200.h")).read()
     declared = set(re.findall(r"\b(hg_[a-z0-9_]+)\s*\(", header))
     declared -= {"hg_mel_plan"}
@@ -134,7 +134,10 @@ def test_library_exports_every_declared_symbol():
     for name in sorted(declared):
         assert hasattr(lib, name), f"{name} declared in include/hifigan_b200.h but not exported"
     assert declared == set(_lib.EXPORTED_SYMBOLS)
-    assert _lib.lib().hg_abi_version() == 2
+    # ABI 3 dropped these entry points (ABI 2 had them)
+    for name in ("hg_set_cta_limit", "hg_unpack_wgrad_convtr", "hg_l1_sum_bf16"):
+        assert not hasattr(lib, name), f"{name} is still exported"
+    assert _lib.lib().hg_abi_version() == 3
 
 
 def test_convtr_geometry():
@@ -419,29 +422,6 @@ def test_epoch_learning_rate_matches_torch_exponential_lr():
         assert opt2.param_groups[0]["lr"] == pytest.approx(epoch_learning_rate(h, epoch), rel=1e-12)
         opt2.step()
         sch2.step()
-
-
-def test_cta_limit_is_a_per_thread_setting_that_returns_the_previous_value():
-    """hg_set_cta_limit (include/hifigan_b200.h): host-only state, no CUDA call."""
-    import threading
-    L = _lib.lib()
-    assert L.hg_set_cta_limit(0) == 0
-    assert L.hg_set_cta_limit(48) == 0 and L.hg_set_cta_limit(-5) == 48 and L.hg_set_cta_limit(0) == 0   # negative -> off
-    L.hg_set_cta_limit(40)
-    seen = []
-    t = threading.Thread(target=lambda: seen.append(L.hg_set_cta_limit(0)))
-    t.start(); t.join()
-    assert seen == [0]                      # another thread starts unlimited
-    assert L.hg_set_cta_limit(0) == 40      # and did not touch this thread's value
-
-
-def test_mrf_lane_split_gives_even_cta_counts_that_fill_the_gpu():
-    from hifigan_b200.models import _GeneratorEngine
-    for weights in ([1.0, 1.0, 1.0], [5.2, 6.1, 7.2], [0.01, 1.0, 1.0], [2.1, 3.0, 5.2], [1.0, 3.0]):
-        s = _GeneratorEngine._split_ctas(weights, 148, _GeneratorEngine.LANE_MIN_CTAS)
-        assert sum(s) == 148 and all(v % 2 == 0 and v >= _GeneratorEngine.LANE_MIN_CTAS for v in s), (weights, s)
-        if len(set(weights)) == len(weights):
-            assert s.index(max(s)) == weights.index(max(weights))
 
 
 def test_lane_stamps_are_off_unless_asked_for(monkeypatch):
