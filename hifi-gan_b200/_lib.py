@@ -114,6 +114,9 @@ _SIGNATURES = {
     "hg_conv1d_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                               c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_float, c_void_p, c_int,
                               c_void_p]),
+    "hg_conv1d_fwd_actres": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                                     c_void_p, c_float, c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_float,
+                                     c_void_p, c_int, c_void_p]),
     "hg_conv1d_tap_order": (c_int, [c_int, c_int, c_int, POINTER(c_int)]),
     "hg_conv1d_general_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                                       c_int, c_int, c_int, c_void_p, c_float, c_void_p, c_int, c_int, c_void_p]),
@@ -131,6 +134,9 @@ _SIGNATURES = {
     "hg_resblock_pair_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                                      c_int, c_float, c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_float,
                                      c_void_p, c_int, c_void_p]),
+    "hg_resblock_pair_fwd_actin": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
+                                           c_int, c_int, c_float, c_void_p, c_void_p, c_float, c_void_p, c_void_p,
+                                           c_float, c_void_p, c_int, c_void_p]),
     "hg_float_to_int16": (c_int, [c_void_p, ctypes.c_longlong, c_float, c_void_p, c_void_p]),
     "hg_loss_sum": (c_int, [c_void_p, c_void_p, ctypes.c_longlong, c_int, c_float, c_void_p, c_void_p]),
     "hg_segment_gather": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),

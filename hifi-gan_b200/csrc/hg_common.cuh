@@ -305,6 +305,19 @@ __device__ __forceinline__ void add_bf16x16(float (&v)[16], const U8& r) {
     v[2 * i + 1] += f.y;
   }
 }
+// v += leaky_relu^-1(r): r holds bf16(leaky_relu(x, slope)) with 0 < slope <= 1 and inv_slope = 1 / slope computed
+// on the host (inv_slope = 1: r is raw and the add is exact, as add_bf16x16).  min(a, a / slope) undoes the
+// activation for either sign.  Multiplying by the fp32 reciprocal instead of dividing by slope differs from the
+// division by at most one fp32 ulp, far below the 2^-9 relative rounding the bf16 copy already carries, which is
+// the same error as storing x raw.
+__device__ __forceinline__ void add_bf16x16_unlrelu(float (&v)[16], const U8& r, float inv_slope) {
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    const float2 f = unpack_bf16x2(r.v[i]);
+    v[2 * i] += fminf(f.x, f.x * inv_slope);
+    v[2 * i + 1] += fminf(f.y, f.y * inv_slope);
+  }
+}
 
 
 

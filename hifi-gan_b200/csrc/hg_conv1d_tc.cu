@@ -91,6 +91,10 @@ struct ConvArgs {
   // the item were run alone (results stay bit-identical to the per-item call).  NULL: every item is t rows long.
   const int* item_len;
   int item_mul;
+  // res0 holds bf16(leaky_relu(x, slope)) and res0_inv = 1 / slope: the residual x is rebuilt in the epilogue, so a
+  // tensor that feeds both a conv and a residual add is stored once, activated.  1: res0 is raw.  Forward flavours
+  // (kEpi 0 and 5) only.
+  float res0_inv;
 };
 
 // One 16-column group of one accumulator row: everything the epilogue does between the TMEM load and the
@@ -102,6 +106,7 @@ struct ConvArgs {
 //   3  data gradient of the generator step through a discriminator: + mask, feature-matching sign term
 //   4  everything (+ the pre-add of an incoming feature-map gradient: the autograd path)
 //   5  forward with the two extra addends of an MRF-final launch (flavours 0 and 1 take one residual only)
+// Flavours 0 and 5 also rebuild an activated res0 (res0_inv); the others take a raw res0.
 // Carrying the warp-uniform branches of the full epilogue in every kernel cost 9 % of the inference forward
 // (55.4 -> 50.4 ms at 64 x 1024 frames) and 0.4 ms of the 11.9 ms training step (profiles/r02_summary.md).
 __host__ __device__ constexpr bool epi_mask(int k) { return k >= 2; }
@@ -109,6 +114,7 @@ __host__ __device__ constexpr bool epi_sums(int k) { return k == 2 || k == 4; }
 __host__ __device__ constexpr bool epi_fm(int k) { return k == 3 || k == 4; }
 __host__ __device__ constexpr bool epi_pre(int k) { return k == 4; }
 __host__ __device__ constexpr bool epi_mrf(int k) { return k >= 2; }   // second / third addend (res1, res2)
+__host__ __device__ constexpr bool epi_actres(int k) { return k == 0 || k == 5; }
 template <int kEpi>
 __device__ __forceinline__ void epi_group(const ConvArgs& p, bool valid, bool keep, size_t off, int ch,
                                           const uint32_t (&raw)[16], const hg::U8* r0, const hg::U8* r1,
@@ -146,7 +152,10 @@ __device__ __forceinline__ void epi_group(const ConvArgs& p, bool valid, bool ke
       if (!(a.y > 0.f)) v[2 * i + 1] *= p.mask_slope;
     }
   }
-  if (p.res0) hg::add_bf16x16(v, *r0);
+  if (p.res0) {
+    if (epi_actres(kEpi)) hg::add_bf16x16_unlrelu(v, *r0, p.res0_inv);
+    else hg::add_bf16x16(v, *r0);
+  }
   if (epi_mrf(kEpi) && p.res1) hg::add_bf16x16(v, r1 ? *r1 : hg::ldg256(p.res1 + off));
   if (epi_mrf(kEpi) && p.res2) hg::add_bf16x16(v, r2 ? *r2 : hg::ldg256(p.res2 + off));
   const float sc = keep ? p.scale : 0.f;                               // rows past a ragged item's end: zeros
@@ -866,6 +875,7 @@ struct ConvExtra {
   int colsum_mod = 0;     // 0: the launch's output channel count
   const int* item_len = nullptr;
   int item_mul = 1;
+  float res0_inv = 1.f;   // 1 / slope of an activated res0 (forward launches only); 1: raw
 };
 
 int conv_forward(const void* x, const void* w_packed, const float* bias, int batch, int t_in_rows,
@@ -975,6 +985,7 @@ int conv_forward(const void* x, const void* w_packed, const float* bias, int bat
   for (int i = 0; i < 3; ++i) p.colsum[i] = ex.colsum[i];
   p.colsum_mod = ex.colsum_mod > 0 ? ex.colsum_mod : cout;
   p.item_len = ex.item_len; p.item_mul = ex.item_mul;
+  p.res0_inv = ex.res0_inv;
   HG_REQUIRE(!ex.colsum[1] || ex.colsum[0], "conv: bias-gradient destinations must be filled from slot 0");
   p.seq_div = ex.seq_div > 0 ? ex.seq_div : (1 << 30);
   HG_REQUIRE(ex.seq_pitch >= 0 && (ex.seq_pitch == 0 || batch == 1), "conv: flat sequences need batch == 1");
@@ -1028,11 +1039,12 @@ int conv_forward(const void* x, const void* w_packed, const float* bias, int bat
 
 }  // namespace
 
-extern "C" int hg_conv1d_fwd(const void* x, const void* w_packed, const float* bias, int batch, int t,
-                             int cin, int cout, int ktaps, int dilation, int pad_left,
-                             const void* res0, const void* res1, const void* res2, float scale,
-                             void* out_raw, void* out_act, float act_slope, const int* item_len, int item_mul,
-                             void* stream) {
+namespace {
+
+int conv1d_fwd(const void* x, const void* w_packed, const float* bias, int batch, int t, int cin, int cout, int ktaps,
+               int dilation, int pad_left, const void* res0, float res0_inv, const void* res1, const void* res2,
+               float scale, void* out_raw, void* out_act, float act_slope, const int* item_len, int item_mul,
+               void* stream) {
   HG_REQUIRE(cout > 0 && cout % 32 == 0, "hg_conv1d_fwd: cout=%d must be a multiple of 32", cout);
   HG_REQUIRE(cin > 0 && cin % 32 == 0, "hg_conv1d_fwd: cin=%d must be a multiple of 32", cin);
   HG_REQUIRE(ktaps > 0 && dilation > 0 && 128 + (ktaps - 1) * dilation <= 256,
@@ -1040,8 +1052,31 @@ extern "C" int hg_conv1d_fwd(const void* x, const void* w_packed, const float* b
   const int n_tile = (cout % 256 == 0) ? 256 : (cout % 128 == 0) ? 128 : (cout % 64 == 0) ? 64 : 32;
   ConvExtra ex;
   ex.item_len = item_len; ex.item_mul = item_mul > 0 ? item_mul : 1;
+  ex.res0_inv = res0_inv;
   return conv_forward(x, w_packed, bias, batch, t, cin, t, t, cin, cout, n_tile, 0, ktaps, 1, dilation, pad_left,
                       res0, res1, res2, scale, out_raw, out_act, act_slope, stream, ex);
+}
+
+}  // namespace
+
+extern "C" int hg_conv1d_fwd(const void* x, const void* w_packed, const float* bias, int batch, int t,
+                             int cin, int cout, int ktaps, int dilation, int pad_left,
+                             const void* res0, const void* res1, const void* res2, float scale,
+                             void* out_raw, void* out_act, float act_slope, const int* item_len, int item_mul,
+                             void* stream) {
+  return conv1d_fwd(x, w_packed, bias, batch, t, cin, cout, ktaps, dilation, pad_left, res0, 1.f, res1, res2, scale,
+                    out_raw, out_act, act_slope, item_len, item_mul, stream);
+}
+
+extern "C" int hg_conv1d_fwd_actres(const void* x, const void* w_packed, const float* bias, int batch, int t,
+                                    int cin, int cout, int ktaps, int dilation, int pad_left,
+                                    const void* res0, float res0_slope, const void* res1, const void* res2,
+                                    float scale, void* out_raw, void* out_act, float act_slope, const int* item_len,
+                                    int item_mul, void* stream) {
+  HG_REQUIRE(res0 && res0_slope > 0.f && res0_slope <= 1.f,
+             "hg_conv1d_fwd_actres: needs res0 and a slope in (0, 1] (got %g)", res0_slope);
+  return conv1d_fwd(x, w_packed, bias, batch, t, cin, cout, ktaps, dilation, pad_left, res0, 1.f / res0_slope, res1,
+                    res2, scale, out_raw, out_act, act_slope, item_len, item_mul, stream);
 }
 
 extern "C" int hg_conv1d_tap_order(int ktaps, int stride, int pad_left, int* host_order) {

@@ -11,11 +11,13 @@
 // so conv1 produces exactly 128 rows):
 //   producer warp   TMA box of 128 + (k-1)*d1 raw rows of x           -> X[slot]          (x_full)
 //   transform warps in-place leaky_relu on the box (generic proxy), fence.proxy.async      (x_ready)
+//                   (kActIn: x arrives already leaky_relu'd, the box is left as it is)
 //   MMA thread      acc1 = sum_j X[slot][r + j*d1] * W1_j   (row-shifted descriptors)      (acc1_full)
 //   E1 warps (8)    t1 = leaky_relu(acc1 + b1), zero outside [0,T), bf16 -> T1[i&1] in the swizzled
 //                   K-major layout UMMA expects, fence.proxy.async                         (t1_full)
 //   MMA thread      acc2 = sum_j T1[i&1][r + j] * W2_j                                     (acc2_full)
 //   E2 warps (8)    y = (acc2 + b2 + x + res1 + res2) * scale -> raw / leaky_relu'd bf16 outputs
+//                   (kActIn: x is rebuilt from its activated copy, hg::add_bf16x16_unlrelu)
 // The MMA thread issues conv1 of tile i+1 before conv2 of tile i, and the two epilogue groups work on
 // different tiles concurrently, so the tensor pipe stays busy while an intermediate is being written.  Both filter banks stay
 // resident in shared memory for the whole kernel.  The residual x is re-read from global memory
@@ -62,6 +64,7 @@ struct PairArgs {
   // zero padding when the item runs alone) and the output rows up to t are stored as zeros.  NULL: all items t rows.
   const int* item_len;
   int item_mul;
+  float x_inv;          // kActIn: 1 / in_slope, undoes the activation of the re-read residual
 };
 
 struct PairBarriers {
@@ -85,7 +88,9 @@ __device__ __forceinline__ uint32_t lrelu_bf16x2(uint32_t w, __nv_bfloat162 slop
 // batches).  kMrf = false: the plain step "one residual in, raw out, every item t rows long, scale 1" — 15 of the 18
 // pair launches of a V1 forward.  The output role is the kernel's bottleneck at C = 32: compiled without the other
 // paths it takes 0.86 -> 0.76 ms (k = 3) and 0.89 -> 0.75 ms (k = 7) per launch at 64 x 1024 frames.
-template <int C, bool kSingle, bool kMrf>
+// kActIn = true: x holds leaky_relu(x, in_slope), the only copy a stage input that also feeds unfused convs is
+// stored as; false: x is raw.
+template <int C, bool kSingle, bool kMrf, bool kActIn>
 __global__ void __launch_bounds__(pair_threads(C), 1)
 resblock_pair_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_w1,
                      const __grid_constant__ CUtensorMap tm_w2, const PairArgs p) {
@@ -248,14 +253,16 @@ resblock_pair_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_cons
     uint32_t slot = 0, phase = 0;
     for (int i = 0; i < n_local; ++i) {
       hg::mbar_wait(&bars->x_full[slot], phase);
-      uint4* xs = reinterpret_cast<uint4*>(x_buf + slot * p.x_slot_bytes);
-      for (int q = tid; q < n_chunks; q += kXformWarps * 32) {
-        uint4 v = xs[q];
-        v.x = lrelu_bf16x2(v.x, slope2); v.y = lrelu_bf16x2(v.y, slope2);
-        v.z = lrelu_bf16x2(v.z, slope2); v.w = lrelu_bf16x2(v.w, slope2);
-        xs[q] = v;
+      if (!kActIn) {
+        uint4* xs = reinterpret_cast<uint4*>(x_buf + slot * p.x_slot_bytes);
+        for (int q = tid; q < n_chunks; q += kXformWarps * 32) {
+          uint4 v = xs[q];
+          v.x = lrelu_bf16x2(v.x, slope2); v.y = lrelu_bf16x2(v.y, slope2);
+          v.z = lrelu_bf16x2(v.z, slope2); v.w = lrelu_bf16x2(v.w, slope2);
+          xs[q] = v;
+        }
+        hg::fence_proxy_async_smem();
       }
-      hg::fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) hg::mbar_arrive(&bars->x_ready[slot]);
       if (++slot == static_cast<uint32_t>(p.x_slots)) { slot = 0; phase ^= 1u; }
@@ -409,7 +416,8 @@ resblock_pair_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_cons
               v[4 * q + 2] = __uint_as_float(raw[4 * q + 2]) + bq.z;
               v[4 * q + 3] = __uint_as_float(raw[4 * q + 3]) + bq.w;
             }
-            hg::add_bf16x16(v, rcur[g]);
+            if (kActIn) hg::add_bf16x16_unlrelu(v, rcur[g], p.x_inv);
+            else hg::add_bf16x16(v, rcur[g]);
             if (kMrf && p.res1) hg::add_bf16x16(v, kPreRes ? r1[kPreRes ? g : 0] : hg::ldg256(p.res1 + off + g * 16));
             if (kMrf && p.res2) hg::add_bf16x16(v, kPreRes ? r2[kPreRes ? g : 0] : hg::ldg256(p.res2 + off + g * 16));
             if (kMrf) {
@@ -445,24 +453,27 @@ resblock_pair_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_cons
 
 int g_sms = 0, g_smem = 0;
 
-template <int C, bool kSingle, bool kMrf>
+template <int C, bool kSingle, bool kMrf, bool kActIn>
 int launch_pair_as(const CUtensorMap& tx, const CUtensorMap& tw1, const CUtensorMap& tw2, const PairArgs& p,
                 size_t smem_bytes, int grid, cudaStream_t st) {
   static hg::PerDeviceOnce once;
   if (once.need())
-    HG_CHECK_CUDA(cudaFuncSetAttribute(resblock_pair_kernel<C, kSingle, kMrf>,
+    HG_CHECK_CUDA(cudaFuncSetAttribute(resblock_pair_kernel<C, kSingle, kMrf, kActIn>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, g_smem));
-  resblock_pair_kernel<C, kSingle, kMrf><<<grid, pair_threads(C), smem_bytes, st>>>(tx, tw1, tw2, p);
+  resblock_pair_kernel<C, kSingle, kMrf, kActIn><<<grid, pair_threads(C), smem_bytes, st>>>(tx, tw1, tw2, p);
   HG_CHECK_CUDA(cudaGetLastError());
   return HG_OK;
 }
 
 template <int C, bool kSingle>
 int launch_pair(const CUtensorMap& tx, const CUtensorMap& tw1, const CUtensorMap& tw2, const PairArgs& p,
-                size_t smem_bytes, int grid, cudaStream_t st) {
+                bool act_in, size_t smem_bytes, int grid, cudaStream_t st) {
   const bool mrf = p.res1 || p.res2 || p.out_act || p.item_len || p.scale != 1.f;   // anything beyond the plain step
-  return mrf ? launch_pair_as<C, kSingle, true>(tx, tw1, tw2, p, smem_bytes, grid, st)
-             : launch_pair_as<C, kSingle, false>(tx, tw1, tw2, p, smem_bytes, grid, st);
+  if (act_in)
+    return mrf ? launch_pair_as<C, kSingle, true, true>(tx, tw1, tw2, p, smem_bytes, grid, st)
+               : launch_pair_as<C, kSingle, false, true>(tx, tw1, tw2, p, smem_bytes, grid, st);
+  return mrf ? launch_pair_as<C, kSingle, true, false>(tx, tw1, tw2, p, smem_bytes, grid, st)
+             : launch_pair_as<C, kSingle, false, false>(tx, tw1, tw2, p, smem_bytes, grid, st);
 }
 
 size_t pair_smem_bytes(int c, int ktaps, int dil1, int subs, int x_slots, int single, PairArgs* out) {
@@ -509,11 +520,12 @@ extern "C" int hg_resblock_single_supported(int c, int ktaps, int dil1) {
   return pick_subs(c, ktaps, dil1, 1) > 0 ? 1 : 0;
 }
 
-extern "C" int hg_resblock_pair_fwd(const void* x, const void* w1_packed, const float* b1,
-                                    const void* w2_packed, const float* b2, int batch, int t, int c,
-                                    int ktaps, int dil1, float in_slope, const void* res1,
-                                    const void* res2, float scale, void* out_raw, void* out_act,
-                                    float out_slope, const int* item_len, int item_mul, void* stream) {
+namespace {
+
+int resblock_pair_fwd(const void* x, bool act_in, const void* w1_packed, const float* b1, const void* w2_packed,
+                      const float* b2, int batch, int t, int c, int ktaps, int dil1, float in_slope, const void* res1,
+                      const void* res2, float scale, void* out_raw, void* out_act, float out_slope,
+                      const int* item_len, int item_mul, void* stream) {
   const int single = w2_packed == nullptr;   // ResBlock2 step: one conv + residual
   HG_REQUIRE(x && w1_packed && b1 && (single || b2), "hg_resblock_pair_fwd: null input");
   HG_REQUIRE(out_raw || out_act, "hg_resblock_pair_fwd: no output requested");
@@ -541,6 +553,7 @@ extern "C" int hg_resblock_pair_fwd(const void* x, const void* w1_packed, const 
   p.out_raw = static_cast<__nv_bfloat16*>(out_raw);
   p.out_act = static_cast<__nv_bfloat16*>(out_act);
   p.item_len = item_len; p.item_mul = item_mul > 0 ? item_mul : 1;
+  p.x_inv = act_in ? 1.f / in_slope : 1.f;
 
   CUtensorMap tx, tw1, tw2;
   const int swz = c * 2;
@@ -556,12 +569,33 @@ extern "C" int hg_resblock_pair_fwd(const void* x, const void* w1_packed, const 
   const int grid = p.num_tiles < g_sms ? p.num_tiles : g_sms;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (single)
-    rc = (c == 64) ? launch_pair<64, true>(tx, tw1, tw2, p, smem_bytes, grid, st)
-                   : launch_pair<32, true>(tx, tw1, tw2, p, smem_bytes, grid, st);
+    rc = (c == 64) ? launch_pair<64, true>(tx, tw1, tw2, p, act_in, smem_bytes, grid, st)
+                   : launch_pair<32, true>(tx, tw1, tw2, p, act_in, smem_bytes, grid, st);
   else
-    rc = (c == 64) ? launch_pair<64, false>(tx, tw1, tw2, p, smem_bytes, grid, st)
-                   : launch_pair<32, false>(tx, tw1, tw2, p, smem_bytes, grid, st);
+    rc = (c == 64) ? launch_pair<64, false>(tx, tw1, tw2, p, act_in, smem_bytes, grid, st)
+                   : launch_pair<32, false>(tx, tw1, tw2, p, act_in, smem_bytes, grid, st);
   if (rc) return rc;
   g_hg_launches.fetch_add(1, std::memory_order_relaxed);
   return HG_OK;
+}
+
+}  // namespace
+
+extern "C" int hg_resblock_pair_fwd(const void* x, const void* w1_packed, const float* b1,
+                                    const void* w2_packed, const float* b2, int batch, int t, int c,
+                                    int ktaps, int dil1, float in_slope, const void* res1,
+                                    const void* res2, float scale, void* out_raw, void* out_act,
+                                    float out_slope, const int* item_len, int item_mul, void* stream) {
+  return resblock_pair_fwd(x, false, w1_packed, b1, w2_packed, b2, batch, t, c, ktaps, dil1, in_slope, res1, res2,
+                           scale, out_raw, out_act, out_slope, item_len, item_mul, stream);
+}
+
+extern "C" int hg_resblock_pair_fwd_actin(const void* x_act, const void* w1_packed, const float* b1,
+                                          const void* w2_packed, const float* b2, int batch, int t, int c,
+                                          int ktaps, int dil1, float in_slope, const void* res1,
+                                          const void* res2, float scale, void* out_raw, void* out_act,
+                                          float out_slope, const int* item_len, int item_mul, void* stream) {
+  HG_REQUIRE(in_slope > 0.f && in_slope <= 1.f, "hg_resblock_pair_fwd_actin: slope %g not in (0, 1]", in_slope);
+  return resblock_pair_fwd(x_act, true, w1_packed, b1, w2_packed, b2, batch, t, c, ktaps, dil1, in_slope, res1, res2,
+                           scale, out_raw, out_act, out_slope, item_len, item_mul, stream);
 }

@@ -177,27 +177,32 @@ class _PackedConv:
         self.key = key
 
 
-def _conv(L, x, pc: _PackedConv, batch: int, t: int, *, res=(None, None, None), scale=1.0,
+def _conv(L, x, pc: _PackedConv, batch: int, t: int, *, res=(None, None, None), res0_slope=0.0, scale=1.0,
           out_raw=None, out_act=None, slope=LRELU_SLOPE, item=(0, 1)) -> None:
-    """item = (device pointer of int32 item lengths or 0, rows per length unit): ragged batches, see hg_conv1d_fwd"""
+    """item = (device pointer of int32 item lengths or 0, rows per length unit): ragged batches, see hg_conv1d_fwd.
+    res0_slope > 0: res[0] holds leaky_relu(residual, res0_slope), undone in the epilogue (hg_conv1d_fwd_actres)."""
     p = [0 if r is None else r.data_ptr() for r in res]
-    _lib.check(L.hg_conv1d_fwd(x.data_ptr(), pc.w.data_ptr(), pc.bias.data_ptr(), batch, t, pc.cin_p,
-                               pc.w.shape[1], pc.taps, pc.dil, pc.pad_left, p[0], p[1], p[2], scale,
-                               0 if out_raw is None else out_raw.data_ptr(),
-                               0 if out_act is None else out_act.data_ptr(), slope, item[0], item[1], _stream()),
-               "hg_conv1d_fwd")
+    outs = (0 if out_raw is None else out_raw.data_ptr(), 0 if out_act is None else out_act.data_ptr(), slope,
+            item[0], item[1], _stream())
+    head = (x.data_ptr(), pc.w.data_ptr(), pc.bias.data_ptr(), batch, t, pc.cin_p, pc.w.shape[1], pc.taps, pc.dil,
+            pc.pad_left)
+    if res0_slope:
+        _lib.check(L.hg_conv1d_fwd_actres(*head, p[0], res0_slope, p[1], p[2], scale, *outs), "hg_conv1d_fwd_actres")
+    else:
+        _lib.check(L.hg_conv1d_fwd(*head, p[0], p[1], p[2], scale, *outs), "hg_conv1d_fwd")
 
 
-def _pair(L, x, pc1: _PackedConv, pc2: _PackedConv, batch: int, t: int, *, res=(None, None), scale=1.0,
-          out_raw=None, out_act=None, slope=LRELU_SLOPE, item=(0, 1)) -> None:
-    """One fused ResBlock1 step: conv2(lrelu(conv1(lrelu(x)) + b1)) + b2 + x (+ res) — hg_resblock_pair_fwd."""
+def _pair(L, x, pc1: _PackedConv, pc2: _PackedConv, batch: int, t: int, *, x_act=False, res=(None, None),
+          scale=1.0, out_raw=None, out_act=None, slope=LRELU_SLOPE, item=(0, 1)) -> None:
+    """One fused ResBlock1 step: conv2(lrelu(conv1(lrelu(x)) + b1)) + b2 + x (+ res) — hg_resblock_pair_fwd.
+    x_act: x holds leaky_relu(x, LRELU_SLOPE) (hg_resblock_pair_fwd_actin)."""
     p = [0 if r is None else r.data_ptr() for r in res]
     w2, b2 = (0, 0) if pc2 is None else (pc2.w.data_ptr(), pc2.bias.data_ptr())   # None: one ResBlock2 step
-    _lib.check(L.hg_resblock_pair_fwd(x.data_ptr(), pc1.w.data_ptr(), pc1.bias.data_ptr(), w2,
-                                      b2, batch, t, pc1.cin_p, pc1.taps, pc1.dil, LRELU_SLOPE,
-                                      p[0], p[1], scale, 0 if out_raw is None else out_raw.data_ptr(),
-                                      0 if out_act is None else out_act.data_ptr(), slope, item[0], item[1], _stream()),
-               "hg_resblock_pair_fwd")
+    fn, name = ((L.hg_resblock_pair_fwd_actin, "hg_resblock_pair_fwd_actin") if x_act
+                else (L.hg_resblock_pair_fwd, "hg_resblock_pair_fwd"))
+    _lib.check(fn(x.data_ptr(), pc1.w.data_ptr(), pc1.bias.data_ptr(), w2, b2, batch, t, pc1.cin_p, pc1.taps,
+                  pc1.dil, LRELU_SLOPE, p[0], p[1], scale, 0 if out_raw is None else out_raw.data_ptr(),
+                  0 if out_act is None else out_act.data_ptr(), slope, item[0], item[1], _stream()), name)
 
 
 _FUSE_PAIRS = True  # tests flip this to compare the fused and the two-launch paths
@@ -224,8 +229,10 @@ def _resblock_chain(L, block: "nn.Module", packs: List[_PackedConv], batch: int,
                     x_raw, x_act, bufs: Dict[str, torch.Tensor], final, item=(0, 1)) -> None:
     """Run one ResBlock (type 1: packs = [c1_0, c2_0, c1_1, ...]; type 2: packs = [c_0, c_1, ...]).
     `final(kw)` issues the LAST launch of the block (so the caller can fuse the MRF average): kw is either
-    dict(pair=(pc1, pc2), x=raw_input) or dict(pc=conv, x=activated_input, res0=raw_residual).
-    x_act may be None when the first step is fused (fused steps read the raw tensor)."""
+    dict(pair=(pc1, pc2), x=input, x_act=bool) or dict(pc=conv, x=activated_input, res0=residual, res0_slope=s).
+    A step's input is stored once: raw when the step is fused (the pair kernel applies the leaky_relu itself),
+    leaky_relu'd when it is not (its convs read that copy and the residual add undoes the activation, res0_slope).
+    x_raw or x_act may be None; a fused step reads x_raw when it exists."""
     two_conv = isinstance(block, ResBlock1)
     fused = _block_plan(L, block, packs)
     steps = len(fused)
@@ -234,24 +241,27 @@ def _resblock_chain(L, block: "nn.Module", packs: List[_PackedConv], batch: int,
     for i in range(steps):
         last = i == steps - 1
         nr, na = ping[i & 1]
-        want_act = (not last) and (not fused[i + 1])  # only an unfused consumer needs the activated copy
+        if not last:   # the one copy the next step reads
+            nr, na = (nr, None) if fused[i + 1] else (None, na)
         if fused[i]:
             pc1, pc2 = (packs[2 * i], packs[2 * i + 1]) if two_conv else (packs[i], None)
+            x, x_is_act = (cur_raw, False) if cur_raw is not None else (cur_act, True)
             if last:
-                final(dict(pair=(pc1, pc2), x=cur_raw))
+                final(dict(pair=(pc1, pc2), x=x, x_act=x_is_act))
             else:
-                _pair(L, cur_raw, pc1, pc2, batch, t, out_raw=nr, out_act=na if want_act else None, item=item)
+                _pair(L, x, pc1, pc2, batch, t, x_act=x_is_act, out_raw=nr, out_act=na, item=item)
         else:
             if two_conv:
                 _conv(L, cur_act, packs[2 * i], batch, t, out_act=bufs["t1"], item=item)
                 src, pc = bufs["t1"], packs[2 * i + 1]
             else:
                 src, pc = cur_act, packs[i]
+            res0, res0_slope = (cur_raw, 0.0) if cur_raw is not None else (cur_act, LRELU_SLOPE)
             if last:
-                final(dict(pc=pc, x=src, res0=cur_raw))
+                final(dict(pc=pc, x=src, res0=res0, res0_slope=res0_slope))
             else:
-                _conv(L, src, pc, batch, t, res=(cur_raw, None, None), out_raw=nr,
-                      out_act=na if (want_act or not two_conv) else None, item=item)
+                _conv(L, src, pc, batch, t, res=(res0, None, None), res0_slope=res0_slope, out_raw=nr, out_act=na,
+                      item=item)
         cur_raw, cur_act = nr, na
 
 
@@ -285,9 +295,10 @@ class _StandaloneBlockMixin:
 
         def final(kw):
             if "pair" in kw:
-                _pair(L, kw["x"], *kw["pair"], b, t, out_raw=bufs["out"])
+                _pair(L, kw["x"], *kw["pair"], b, t, x_act=kw["x_act"], out_raw=bufs["out"])
             else:
-                _conv(L, kw["x"], kw["pc"], b, t, res=(kw["res0"], None, None), out_raw=bufs["out"])
+                _conv(L, kw["x"], kw["pc"], b, t, res=(kw["res0"], None, None), res0_slope=kw["res0_slope"],
+                      out_raw=bufs["out"])
 
         _resblock_chain(L, self, packs, b, t, c_p, bufs["x_raw"], bufs["x_act"], bufs, final)
         y = torch.empty(b, c_p, t, dtype=torch.float32, device=x.device)
@@ -514,11 +525,14 @@ class _GeneratorEngine:
         _conv(L, ws["mel"], self.pre, b, frames, out_act=ws["pre"], item=(lp, mul))
         cur, t = ws["pre"], frames
         for i, up in enumerate(self.ups):
-            # the leaky_relu'd copy of the stage input is only needed by branches whose first step is unfused
+            # The stage input is stored once: leaky_relu'd when a branch's first step is unfused (its convs read that
+            # copy; the fused first steps of the other branches read it through hg_resblock_pair_fwd_actin), raw
+            # when every first step is fused.
             need_act = any(not _block_plan(L, gen.resblocks[i * nk + j], self.blocks[i * nk + j])[0]
                            for j in range(nk))
+            x_raw, x_act = (None, ws["x_act"]) if need_act else (ws["x_raw"], None)
             # polyphase: one output row of this launch is `stride` samples, so its valid rows are the INPUT's
-            _conv(L, cur, up, b, t, out_raw=ws["x_raw"], out_act=ws["x_act"] if need_act else None, item=(lp, mul))
+            _conv(L, cur, up, b, t, out_raw=x_raw, out_act=x_act, item=(lp, mul))
             t *= up.stride
             mul *= up.stride
             c_p = up.cout_p
@@ -540,11 +554,12 @@ class _GeneratorEngine:
                             others = tuple(ws[f"r{q}"] for q in range(nk - 1)) + (None,) * (3 - nk)
                         outs = dict(scale=1.0 / nk, out_act=ws["stage_out"], slope=out_slope)
                     if "pair" in kw:
-                        _pair(L, kw["x"], *kw["pair"], b, t, res=others, item=(lp, mul), **outs)
+                        _pair(L, kw["x"], *kw["pair"], b, t, x_act=kw["x_act"], res=others, item=(lp, mul), **outs)
                     else:
-                        _conv(L, kw["x"], kw["pc"], b, t, res=(kw["res0"],) + others, item=(lp, mul), **outs)
+                        _conv(L, kw["x"], kw["pc"], b, t, res=(kw["res0"],) + others, res0_slope=kw["res0_slope"],
+                              item=(lp, mul), **outs)
 
-                _resblock_chain(L, blk, packs, b, t, c_p, ws["x_raw"], ws["x_act"], ws, final, item=(lp, mul))
+                _resblock_chain(L, blk, packs, b, t, c_p, x_raw, x_act, ws, final, item=(lp, mul))
             cur = ws["stage_out"]
         if time_convs:
             ev1.record()

@@ -88,6 +88,14 @@ int hg_conv1d_fwd(const void* x, const void* w_packed, const float* bias, int ba
                   int cout, int ktaps, int dilation, int pad_left, const void* res0,
                   const void* res1, const void* res2, float scale, void* out_raw, void* out_act,
                   float act_slope, const int* item_len, int item_mul, void* stream);
+/* hg_conv1d_fwd_actres — hg_conv1d_fwd whose first residual is stored activated: res0 holds
+ * bf16(leaky_relu(r, res0_slope)), 0 < res0_slope <= 1, and the epilogue adds r = min(res0, res0 / res0_slope)
+ * (same 2^-9 relative rounding as a raw copy of r).  A tensor that feeds both a conv and a residual add is
+ * then stored once, as the conv's input. */
+int hg_conv1d_fwd_actres(const void* x, const void* w_packed, const float* bias, int batch, int t, int cin,
+                         int cout, int ktaps, int dilation, int pad_left, const void* res0, float res0_slope,
+                         const void* res1, const void* res2, float scale, void* out_raw, void* out_act,
+                         float act_slope, const int* item_len, int item_mul, void* stream);
 
 /* hg_conv1d_general_fwd — strided and/or grouped Conv1d on the same tcgen05 kernel (the discriminator stacks:
  * DiscriminatorS src/models.py:195-204 — k=41, stride 1/2/4, groups 4/16; DiscriminatorP :133-140 — (5,1)
@@ -133,6 +141,13 @@ int hg_resblock_pair_fwd(const void* x, const void* w1_packed, const float* b1, 
                          const float* b2, int batch, int t, int c, int ktaps, int dil1, float in_slope,
                          const void* res1, const void* res2, float scale, void* out_raw, void* out_act,
                          float out_slope, const int* item_len, int item_mul, void* stream);   /* item_*: hg_conv1d_fwd */
+/* hg_resblock_pair_fwd_actin — hg_resblock_pair_fwd on x_act = bf16(leaky_relu(x, in_slope)), 0 < in_slope <= 1,
+ * instead of x: the first leaky_relu is already applied, and the residual x is rebuilt as
+ * min(x_act, x_act / in_slope) (see hg_conv1d_fwd_actres). */
+int hg_resblock_pair_fwd_actin(const void* x_act, const void* w1_packed, const float* b1, const void* w2_packed,
+                               const float* b2, int batch, int t, int c, int ktaps, int dil1, float in_slope,
+                               const void* res1, const void* res2, float scale, void* out_raw, void* out_act,
+                               float out_slope, const int* item_len, int item_mul, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Discriminator ends (bandwidth-bound CUDA-core kernels).
