@@ -1,9 +1,10 @@
 // hg_mel.cu — mel_spectrogram (src/meldataset.py:56-85) as ONE fused kernel:
-//   reflect-pad -> frame x periodic Hann -> rFFT(1024) -> |X|^2 -> HTK mel (sparse) -> log(clamp(.,1e-5))
+//   reflect-pad -> frame x periodic Hann -> rFFT(n_fft) -> |X|^2 -> HTK mel (sparse) -> log(clamp(.,1e-5))
 // The reference goes through torchaudio.transforms.MelSpectrogram (meldataset.py:59-71): >= 6 library
-// launches and three HBM round trips of the [B,513,F] spectrum.  n_fft == 1024 runs mel_kernel2 (one warp per two
-// frames, the FFT in registers), any other n_fft the direct-DFT mel_dft_kernel, and the backward mel_bwd_kernel
-// (64-thread groups running a 512-point complex Stockham FFT, radix 8 x 8 x 8, on the even/odd packed samples).
+// launches and three HBM round trips of the [B,513,F] spectrum.  n_fft in {256, 512, 1024, 2048} runs mel_kernel2<N2>
+// (one warp per 32 / N2 frames, the FFT in registers), any other n_fft the direct-DFT mel_dft_kernel.  The backward
+// mel_bwd_kernel<N> (one thread group per frame running an N = n_fft / 2 point complex Stockham FFT, radix 8 x 8 then
+// 2, 4, 8 or 8 x 2, on the even/odd packed samples) takes the same four sizes.
 //
 // The per-thread phases are __host__ __device__ so tests can run the exact same arithmetic on the CPU
 // (hg_mel_emulate_host, hg_mel_bwd_emulate_host below) — there is no GPU in the development container.
@@ -23,28 +24,29 @@ struct hg_mel_plan {
   int nnz;
   // device tables
   float* window;     // [n_fft]
-  float2* tw512;     // [512]  exp(-2*pi*i*m/512)
-  float2* tw1024;    // [513]  exp(-2*pi*i*k/1024)
+  float2* tw_half;   // [n_fft/2]    exp(-2*pi*i*m/(n_fft/2)): the FFT sizes only (null otherwise)
+  float2* tw_full;   // [n_fft/2+1]  exp(-2*pi*i*k/n_fft): the FFT sizes only (null otherwise)
   float2* tw_n;      // [n_fft] (cos, sin)(2*pi*n/n_fft): the direct-DFT path of every other n_fft
   int* mel_start;    // [num_mels] first rFFT bin with a non-zero weight
   int* mel_off;      // [num_mels+1] CSR offsets into mel_w
   float* mel_w;      // [nnz]
   // host copies (CPU emulation for tests, and geometry queries)
   std::vector<float> h_window;
-  std::vector<float2> h_tw512, h_tw1024, h_tw_n;
+  std::vector<float2> h_tw_half, h_tw_full, h_tw_n;
   std::vector<int> h_mel_start, h_mel_off;
   std::vector<float> h_mel_w;
 };
 
 namespace {
 
-constexpr int kNfft = 1024;
-constexpr int kHalf = 512;
-constexpr int kFramesPerBlock = 16;
-constexpr int kGroupThreads = 64;
-constexpr int kPadLen = kHalf + kHalf / 16;  // PADI(511) + 1 = 543 -> 544
+// the transform sizes with an FFT path, forward and backward: n_fft = 256, 512, 1024, 2048
+__host__ __device__ constexpr bool is_fft_size(int n_fft) {
+  return n_fft == 256 || n_fft == 512 || n_fft == 1024 || n_fft == 2048;
+}
 
 __host__ __device__ __forceinline__ int padi(int i) { return i + (i >> 4); }
+// complex entries of an N-point buffer addressed through padi: padi(N - 1) + 1, rounded up
+__host__ __device__ constexpr int pad_len(int n) { return n + n / 16; }
 
 struct cpx {
   float x, y;
@@ -80,34 +82,61 @@ __host__ __device__ __forceinline__ void fft8(cpx (&v)[8]) {
   v[1] = a4; v[3] = a5; v[5] = a6; v[7] = a7;
 }
 
-// One Stockham radix-8 pass of a 512-point FFT for butterfly j in [0,64).
+__host__ __device__ __forceinline__ void fft_radix(cpx (&v)[2]) {
+  const cpx a = cadd(v[0], v[1]);
+  v[1] = csub(v[0], v[1]);
+  v[0] = a;
+}
+__host__ __device__ __forceinline__ void fft_radix(cpx (&v)[4]) { fft4(v[0], v[1], v[2], v[3]); }
+__host__ __device__ __forceinline__ void fft_radix(cpx (&v)[8]) { fft8(v); }
+
+// One Stockham radix-R pass of an N-point FFT for butterfly j in [0, N / R); tw holds W_N^m, m in [0, N).
 //   FIRST: inputs come from the staged real samples (even/odd packing + window), Ns = 1.
-template <bool FIRST>
+template <int R, int N, bool FIRST>
 __host__ __device__ __forceinline__ void fft_pass(int j, int ns, const cpx* __restrict__ in,
                                                   cpx* __restrict__ out,
                                                   const float* __restrict__ samples,
                                                   const float* __restrict__ window,
-                                                  const float2* __restrict__ tw512) {
-  cpx v[8];
+                                                  const float2* __restrict__ tw) {
+  constexpr int kStride = N / R;
+  cpx v[R];
   const int k = j & (ns - 1);
 #pragma unroll
-  for (int r = 0; r < 8; ++r) {
-    const int n = j + r * 64;
+  for (int r = 0; r < R; ++r) {
+    const int n = j + r * kStride;
     if (FIRST) {
       v[r] = cpx{samples[2 * n] * window[2 * n], samples[2 * n + 1] * window[2 * n + 1]};
     } else {
       v[r] = in[padi(n)];
       if (r) {
-        const float2 w = tw512[r * k * (64 / ns)];
+        const float2 w = tw[r * k * (kStride / ns)];
         v[r] = cmul(v[r], cpx{w.x, w.y});
       }
     }
   }
-  fft8(v);
-  const int j0 = (j / ns) * ns * 8 + k;
+  fft_radix(v);
+  const int j0 = (j / ns) * ns * R + k;
 #pragma unroll
-  for (int r = 0; r < 8; ++r) out[padi(j0 + r * ns)] = v[r];
+  for (int r = 0; r < R; ++r) out[padi(j0 + r * ns)] = v[r];
 }
+// the pass for thread j of a G-thread group: N / R butterflies, a whole number of them per thread, or (N = 128, radix
+// 8: 16 butterflies over 32 threads) one each for the first N / R threads
+template <int R, int N, int G, bool FIRST>
+__host__ __device__ __forceinline__ void fft_pass_group(int j, int ns, const cpx* __restrict__ in,
+                                                        cpx* __restrict__ out, const float* __restrict__ samples,
+                                                        const float* __restrict__ window,
+                                                        const float2* __restrict__ tw) {
+  constexpr int kBfly = N / R;
+  if constexpr (kBfly < G) {
+    if (j < kBfly) fft_pass<R, N, FIRST>(j, ns, in, out, samples, window, tw);
+  } else {
+    static_assert(kBfly % G == 0, "butterflies must split evenly over the group");
+#pragma unroll
+    for (int i = 0; i < kBfly / G; ++i) fft_pass<R, N, FIRST>(j + i * G, ns, in, out, samples, window, tw);
+  }
+}
+// N = 8 x 8 x R3 (x 2 at N = 1024): the radix of the third pass
+__host__ __device__ constexpr int third_radix(int n) { return n >= 512 ? 8 : n / 64; }
 
 __host__ __device__ __forceinline__ int reflect_index(int i, int t) {
   if (i < 0) i = -i;
@@ -143,34 +172,46 @@ __device__ __forceinline__ void cp_async_table(void* dst_smem, const void* src, 
   for (int i = n16 * 4 + tid; i < (nbytes >> 2); i += nthreads)
     cp_async4(static_cast<uint8_t*>(dst_smem) + 4 * i, static_cast<const uint8_t*>(src) + 4 * i);
 }
-// the two warps of a frame group meet on their own named barrier: groups drift apart freely
+// the G threads (whole warps) of a frame group meet on their own named barrier: groups drift apart freely
+template <int G>
 __device__ __forceinline__ void group_sync(int g) {
-  asm volatile("bar.sync %0, %1;" ::"r"(g + 1), "n"(kGroupThreads) : "memory");
+  asm volatile("bar.sync %0, %1;" ::"r"(g + 1), "n"(G) : "memory");
 }
 
 // ---------------------------------------------------------------------------------------------
 // mel_kernel2 — the forward kernel of round 2: ONE WARP PER TWO FRAMES, the FFT held in registers.
 //
-// The 512-point complex FFT of a frame's even/odd packed samples is split 512 = 32 x 16 (n = 16 n1 + n2,
-// k = k1 + 32 k2):   Z[k1 + 32 k2] = sum_n2 W16^(n2 k2) [ W512^(n2 k1) sum_n1 z[16 n1 + n2] W32^(n1 k1) ]
+// The N-point complex FFT (N = n_fft / 2 = 32 N2, N2 in {4, 8, 16, 32}) of a frame's even/odd packed samples is split
+// N = 32 x N2 (n = N2 n1 + n2, k = k1 + 32 k2):
+//   Z[k1 + 32 k2] = sum_n2 W_N2^(n2 k2) [ W_N^(n2 k1) sum_n1 z[N2 n1 + n2] W32^(n1 k1) ]
+// A warp serves 32 / N2 frames (n_fft 256 / 512 / 1024 / 2048: 8 / 4 / 2 / 1).
 //   phase 1  lane = (frame, n2): 32 windowed complex samples straight from global memory (64-bit coalesced loads,
 //            reflect padding by index arithmetic), a 32-point DFT in registers (4 x 8, compile-time twiddles), the
-//            W512 twiddles from a padded shared table, results to the warp's exchange buffer (conflict-free pitch 33)
-//   phase 2  lane = k1: the 16 values of each frame from the exchange buffer, a 16-point DFT in registers (4 x 4),
+//            W_N twiddles from a padded shared table, results to the warp's exchange buffer (conflict-free pitch 33)
+//   phase 2  lane = k1: the N2 values of each frame from the exchange buffer, an N2-point DFT in registers,
 //            Z to shared memory in natural order
-//   phase 3  lane = k mod 32: real-FFT un-pack of its 16 (+1) bins from Z[k], Z[512 - k], |X|^2 (only up to the last
+//   phase 3  lane = k mod 32: real-FFT un-pack of its N2 (+1) bins from Z[k], Z[N - k], |X|^2 (only up to the last
 //            bin any mel filter reads), written over the frame's own Z region
 //   phase 4  lane = mel bin mod 32: the CSR triangle sums + log(clamp), staged for 64-byte output runs
-// Warps never meet (__syncwarp between phases); a block is 8 warps = 16 consecutive frames and loops over frame
-// groups, so the constant tables are loaded once per block.  ~2.4x fewer warp-instructions per frame than the
-// round-1 radix-8 x 8 x 8 shared-memory kernel (whose FFT passes, fft_pass above, the backward kernel still runs),
-// and no block-wide or named barriers on the frame path.
+// Warps never meet (__syncwarp between phases); a block is 8 warps = 8 x 32 / N2 consecutive frames and loops over
+// frame groups, so the constant tables are loaded once per block.  At n_fft 1024 ~2.4x fewer warp-instructions per
+// frame than the round-1 radix-8 x 8 x 8 shared-memory kernel (whose FFT passes, fft_pass above, the backward kernel
+// still runs), and no block-wide or named barriers on the frame path.  Every size holds 32 complex values per lane in
+// phases 1 and 2, and uses the same exchange buffer.
 // The lane phases are __host__ __device__ (hg_mel_emulate_host runs them lane by lane on the CPU).
 constexpr int kExPitch = 33;                              // complex per (frame, n2) row of the exchange buffer
-constexpr int kWarpScratch = 2 * 16 * kExPitch;           // complex per warp (8448 B) >= 2 x 512 (the Z / power view)
-constexpr int kTwPad = kHalf + kHalf / 16;                // padi(511) + 1
-constexpr int kMel2Warps = 8;                             // 8 warps x 2 frames = kFramesPerBlock
+constexpr int kWarpScratch = 32 * kExPitch;               // complex per warp (8448 B) >= (32 / N2) x N (the Z / power view)
+constexpr int kMel2Warps = 8;
 constexpr int kMel2Threads = kMel2Warps * 32;
+template <int N2>
+struct Mel2Size {
+  static constexpr int kN = 32 * N2;                      // complex FFT points; n_fft = 2 kN
+  static constexpr int kNfft = 2 * kN;
+  static constexpr int kFramesPerWarp = 32 / N2;
+  static constexpr int kFramesPerBlock = kMel2Warps * kFramesPerWarp;
+  static constexpr int kTwPad = pad_len(kN);              // padi(kN - 1) + 1, rounded up
+  static_assert(kFramesPerWarp * kN <= kWarpScratch, "the Z view must fit the exchange buffer");
+};
 
 // e^{-2 pi i j / 32}, j a compile-time constant after unrolling
 __host__ __device__ __forceinline__ cpx w32(int j) {
@@ -230,33 +271,40 @@ __host__ __device__ __forceinline__ void fft16(cpx (&v)[16]) {
   for (int i = 0; i < 16; ++i) v[i] = o[i];
 }
 
+// the N2-point DFT of the second factor (phase 2 of mel_kernel2<N2>)
+__host__ __device__ __forceinline__ void fft_n2(cpx (&v)[4]) { fft4(v[0], v[1], v[2], v[3]); }
+__host__ __device__ __forceinline__ void fft_n2(cpx (&v)[8]) { fft8(v); }
+__host__ __device__ __forceinline__ void fft_n2(cpx (&v)[16]) { fft16(v); }
+__host__ __device__ __forceinline__ void fft_n2(cpx (&v)[32]) { fft32(v); }
+
 struct Mel2Args {
   const float* y;
   float* out;
   float* minmax;
   int batch, t, frames, hop, pad, num_mels;
   const float* window;
-  const float2* tw512;
-  const float2* tw1024;
+  const float2* tw_half;  // W_N^m, m < N
+  const float2* tw_full;  // W_2N^k, k <= N
   const int* mel_start;
   const int* mel_off;
   const float* mel_w;
   int nnz, max_bin;       // max_bin: the last rFFT bin any mel filter reads
-  int groups_per_item;    // ceil(frames / 16)
+  int groups_per_item;    // ceil(frames / kFramesPerBlock)
   int total_groups;       // batch * groups_per_item
 };
 
-// phase 1 (lane = 16 * frame + n2): frame samples -> window -> DFT-32 -> W512 twiddle -> exchange buffer.
+// phase 1 (lane = N2 * frame + n2): frame samples -> window -> DFT-32 -> W_N twiddle -> exchange buffer.
 // `yb` is the batch item, `start` the (possibly negative) first sample of this lane's frame, `vec` whether the
 // frame is interior and 8-byte aligned (plain 64-bit loads).  Returns the lane's sample extrema through lo / hi.
+template <int N2>
 __host__ __device__ __forceinline__ void mel2_phase1(int lane, const float* __restrict__ yb, int start, int t, bool vec,
-                                                     const float* __restrict__ window, const float2* __restrict__ tw512p,
+                                                     const float* __restrict__ window, const float2* __restrict__ twp,
                                                      cpx* __restrict__ ex, float& lo, float& hi) {
-  const int n2 = lane & 15;
+  const int n2 = lane & (N2 - 1);
   cpx v[32];
 #pragma unroll
   for (int n1 = 0; n1 < 32; ++n1) {
-    const int s = 32 * n1 + 2 * n2;
+    const int s = 2 * N2 * n1 + 2 * n2;
     float x0, x1;
     if (vec) {
       const float2 xv = *reinterpret_cast<const float2*>(yb + start + s);
@@ -271,62 +319,67 @@ __host__ __device__ __forceinline__ void mel2_phase1(int lane, const float* __re
     v[n1] = cpx{x0 * w.x, x1 * w.y};
   }
   fft32(v);
-  cpx* row = ex + lane * kExPitch;          // (frame * 16 + n2) * pitch
+  cpx* row = ex + lane * kExPitch;          // (frame * N2 + n2) * pitch
   row[0] = v[0];
 #pragma unroll
   for (int k1 = 1; k1 < 32; ++k1) {
-    const float2 w = tw512p[padi(n2 * k1)];
+    const float2 w = twp[padi(n2 * k1)];
     row[k1] = cmul(v[k1], cpx{w.x, w.y});
   }
 }
-// phase 2a (lane = k1): gather the 16 n2 values of both frames; 2b: DFT-16, Z in natural order over the same buffer
-__host__ __device__ __forceinline__ void mel2_phase2_read(int lane, const cpx* __restrict__ ex, cpx (&a)[16], cpx (&b)[16]) {
+// phase 2a (lane = k1): gather the N2 n2 values of each of the warp's frames; 2b: DFT-N2, Z in natural order over the
+// same buffer (frame h's Z at z + h N)
+template <int N2>
+__host__ __device__ __forceinline__ void mel2_phase2_read(int lane, const cpx* __restrict__ ex,
+                                                          cpx (&a)[32 / N2][N2]) {
 #pragma unroll
-  for (int n2 = 0; n2 < 16; ++n2) {
-    a[n2] = ex[n2 * kExPitch + lane];
-    b[n2] = ex[(16 + n2) * kExPitch + lane];
-  }
+  for (int n2 = 0; n2 < N2; ++n2)
+#pragma unroll
+    for (int h = 0; h < 32 / N2; ++h) a[h][n2] = ex[(h * N2 + n2) * kExPitch + lane];
 }
-__host__ __device__ __forceinline__ void mel2_phase2_write(int lane, cpx (&a)[16], cpx (&b)[16], cpx* __restrict__ z) {
-  fft16(a);
-  fft16(b);
+template <int N2>
+__host__ __device__ __forceinline__ void mel2_phase2_write(int lane, cpx (&a)[32 / N2][N2], cpx* __restrict__ z) {
 #pragma unroll
-  for (int k2 = 0; k2 < 16; ++k2) {
-    z[lane + 32 * k2] = a[k2];
-    z[kHalf + lane + 32 * k2] = b[k2];
-  }
+  for (int h = 0; h < 32 / N2; ++h) fft_n2(a[h]);
+#pragma unroll
+  for (int k2 = 0; k2 < N2; ++k2)
+#pragma unroll
+    for (int h = 0; h < 32 / N2; ++h) z[h * Mel2Size<N2>::kN + lane + 32 * k2] = a[h][k2];
 }
 // phase 3a (lane = k mod 32): |X[k]|^2 of the lane's bins k = lane + 32 k2 (k <= max_bin) of one frame's Z;
-// pw[16] is bin 512 (lane 0).  3b: the powers go over the frame's own Z region (as floats).
+// pw[N2] is bin N (lane 0).  3b: the powers go over the frame's own Z region (as floats).
+template <int N2>
 __host__ __device__ __forceinline__ void mel2_phase3_compute(int lane, const cpx* __restrict__ z, int max_bin,
-                                                             const float2* __restrict__ tw1024, float (&pw)[17]) {
+                                                             const float2* __restrict__ tw_full, float (&pw)[N2 + 1]) {
+  constexpr int kN = Mel2Size<N2>::kN;
 #pragma unroll
-  for (int k2 = 0; k2 < 16; ++k2) {
+  for (int k2 = 0; k2 < N2; ++k2) {
     const int k = lane + 32 * k2;
     float p = 0.f;
     if (k <= max_bin) {
       const cpx zk = z[k];
-      cpx zc = z[(kHalf - k) & (kHalf - 1)];
+      cpx zc = z[(kN - k) & (kN - 1)];
       zc.y = -zc.y;
       const cpx e = cpx{0.5f * (zk.x + zc.x), 0.5f * (zk.y + zc.y)};
       const cpx d = csub(zk, zc);
       const cpx o = cpx{0.5f * d.y, -0.5f * d.x};  // (zk - zc) / (2i)
-      const float2 w = tw1024[k];
+      const float2 w = tw_full[k];
       const cpx x = cadd(e, cmul(o, cpx{w.x, w.y}));
       p = x.x * x.x + x.y * x.y;
     }
     pw[k2] = p;
   }
-  pw[16] = 0.f;
-  if (lane == 0 && kHalf <= max_bin) {
-    const cpx z0 = z[0];                           // X[512] = Re Z[0] - Im Z[0]
-    pw[16] = (z0.x - z0.y) * (z0.x - z0.y);
+  pw[N2] = 0.f;
+  if (lane == 0 && kN <= max_bin) {
+    const cpx z0 = z[0];                           // X[N] = Re Z[0] - Im Z[0]
+    pw[N2] = (z0.x - z0.y) * (z0.x - z0.y);
   }
 }
-__host__ __device__ __forceinline__ void mel2_phase3_write(int lane, const float (&pw)[17], float* __restrict__ power) {
+template <int N2>
+__host__ __device__ __forceinline__ void mel2_phase3_write(int lane, const float (&pw)[N2 + 1], float* __restrict__ power) {
 #pragma unroll
-  for (int k2 = 0; k2 < 16; ++k2) power[lane + 32 * k2] = pw[k2];
-  if (lane == 0) power[kHalf] = pw[16];
+  for (int k2 = 0; k2 < N2; ++k2) power[lane + 32 * k2] = pw[k2];
+  if (lane == 0) power[Mel2Size<N2>::kN] = pw[N2];
 }
 // phase 4 (lane = m mod 32): CSR triangle sums + log(clamp(., 1e-5)) of one frame -> out_col[m * out_stride]
 __host__ __device__ __forceinline__ void mel2_phase4(int lane, int num_mels, const float* __restrict__ power,
@@ -342,85 +395,90 @@ __host__ __device__ __forceinline__ void mel2_phase4(int lane, int num_mels, con
 }
 
 struct Mel2Smem {
-  uint32_t win, tw512, tw1024, melw, melidx, meloff, scratch, outs, total;
+  uint32_t win, tw_half, tw_full, melw, melidx, meloff, scratch, outs, total;
 };
+template <int N2>
 __host__ __device__ inline Mel2Smem mel2_smem_layout(int num_mels, int nnz) {
+  using S = Mel2Size<N2>;
   auto up = [](uint32_t v) { return (v + 15u) & ~15u; };
   Mel2Smem l;
   uint32_t o = 0;
-  l.win = o;     o += kNfft * 4u;
-  l.tw512 = o;   o += up(kTwPad * 8u);
-  l.tw1024 = o;  o += up((kHalf + 1) * 8u);
-  l.melw = o;    o += up(static_cast<uint32_t>(nnz > 0 ? nnz : 1) * 4u);
-  l.melidx = o;  o += up(static_cast<uint32_t>(num_mels) * 4u);
-  l.meloff = o;  o += up(static_cast<uint32_t>(num_mels + 1) * 4u);
-  l.scratch = o; o += kMel2Warps * kWarpScratch * 8u;
-  l.outs = o;    o += static_cast<uint32_t>(num_mels) * kFramesPerBlock * 4u;
+  l.win = o;      o += S::kNfft * 4u;
+  l.tw_half = o;  o += up(S::kTwPad * 8u);
+  l.tw_full = o;  o += up((S::kN + 1) * 8u);
+  l.melw = o;     o += up(static_cast<uint32_t>(nnz > 0 ? nnz : 1) * 4u);
+  l.melidx = o;   o += up(static_cast<uint32_t>(num_mels) * 4u);
+  l.meloff = o;   o += up(static_cast<uint32_t>(num_mels + 1) * 4u);
+  l.scratch = o;  o += kMel2Warps * kWarpScratch * 8u;
+  l.outs = o;     o += static_cast<uint32_t>(num_mels) * S::kFramesPerBlock * 4u;
   l.total = o;
   return l;
 }
 
+template <int N2>
 __global__ void __launch_bounds__(kMel2Threads, 2) mel_kernel2(const Mel2Args a) {
+  using S = Mel2Size<N2>;
+  constexpr int kN = S::kN, kFPW = S::kFramesPerWarp, kFPB = S::kFramesPerBlock;
   extern __shared__ __align__(16) uint8_t sm[];
   constexpr int kThreads2 = kMel2Threads;
-  const Mel2Smem L = mel2_smem_layout(a.num_mels, a.nnz);
+  const Mel2Smem L = mel2_smem_layout<N2>(a.num_mels, a.nnz);
   float* s_win = reinterpret_cast<float*>(sm + L.win);
-  float2* s_tw512p = reinterpret_cast<float2*>(sm + L.tw512);                  // padded: entry i at padi(i)
-  float2* s_tw1024 = reinterpret_cast<float2*>(sm + L.tw1024);
+  float2* s_twp = reinterpret_cast<float2*>(sm + L.tw_half);                   // padded: entry i at padi(i)
+  float2* s_twf = reinterpret_cast<float2*>(sm + L.tw_full);
   float* s_melw = reinterpret_cast<float*>(sm + L.melw);
   int* s_start = reinterpret_cast<int*>(sm + L.melidx);
   int* s_off = reinterpret_cast<int*>(sm + L.meloff);
-  float* outs = reinterpret_cast<float*>(sm + L.outs);                         // [num_mels][16]
+  float* outs = reinterpret_cast<float*>(sm + L.outs);                         // [num_mels][kFPB]
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   cpx* scratch = reinterpret_cast<cpx*>(sm + L.scratch) + warp * kWarpScratch;
 
-  cp_async_table(s_win, a.window, kNfft * 4, tid, kThreads2);
-  cp_async_table(s_tw1024, a.tw1024, (kHalf + 1) * 8, tid, kThreads2);
+  cp_async_table(s_win, a.window, S::kNfft * 4, tid, kThreads2);
+  cp_async_table(s_twf, a.tw_full, (kN + 1) * 8, tid, kThreads2);
   cp_async_table(s_melw, a.mel_w, a.nnz * 4, tid, kThreads2);
   cp_async_table(s_start, a.mel_start, a.num_mels * 4, tid, kThreads2);
   cp_async_table(s_off, a.mel_off, (a.num_mels + 1) * 4, tid, kThreads2);
-  for (int i = tid; i < kHalf; i += kThreads2) s_tw512p[padi(i)] = a.tw512[i];
+  for (int i = tid; i < kN; i += kThreads2) s_twp[padi(i)] = a.tw_half[i];
   cp_async_wait_all();
   __syncthreads();
 
   float vmin = INFINITY, vmax = -INFINITY;
   for (int grp = blockIdx.x; grp < a.total_groups; grp += gridDim.x) {
     const int b = grp / a.groups_per_item;
-    const int f0 = (grp - b * a.groups_per_item) * kFramesPerBlock;
+    const int f0 = (grp - b * a.groups_per_item) * kFPB;
     const float* yb = a.y + static_cast<size_t>(b) * a.t;
-    const int fl0 = 2 * warp;                           // this warp's two frames within the group
-    const int f = f0 + fl0 + (lane >> 4);
-    const bool live = f < a.frames;                     // half-warp uniform
+    const int fl0 = kFPW * warp;                        // this warp's frames within the group
+    const int f = f0 + fl0 + lane / N2;
+    const bool live = f < a.frames;                     // uniform over the lane's N2-lane frame
     if (f0 + fl0 < a.frames) {                          // warp-uniform: at least the first frame exists
       const int start = (live ? f : a.frames - 1) * a.hop - a.pad;
-      const bool vec = start >= 0 && start + kNfft <= a.t &&
+      const bool vec = start >= 0 && start + S::kNfft <= a.t &&
                        ((reinterpret_cast<uintptr_t>(yb + start) & 7) == 0);
       float lo = INFINITY, hi = -INFINITY;
-      mel2_phase1(lane, yb, start, a.t, vec, s_win, s_tw512p, scratch, lo, hi);
+      mel2_phase1<N2>(lane, yb, start, a.t, vec, s_win, s_twp, scratch, lo, hi);
       if (live) { vmin = fminf(vmin, lo); vmax = fmaxf(vmax, hi); }
       __syncwarp();
-      cpx za[16], zb[16];
-      mel2_phase2_read(lane, scratch, za, zb);
+      cpx za[kFPW][N2];
+      mel2_phase2_read<N2>(lane, scratch, za);
       __syncwarp();
-      mel2_phase2_write(lane, za, zb, scratch);
+      mel2_phase2_write<N2>(lane, za, scratch);
       __syncwarp();
 #pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        float pw[17];
-        mel2_phase3_compute(lane, scratch + h * kHalf, a.max_bin, s_tw1024, pw);
+      for (int h = 0; h < kFPW; ++h) {
+        float pw[N2 + 1];
+        mel2_phase3_compute<N2>(lane, scratch + h * kN, a.max_bin, s_twf, pw);
         __syncwarp();
-        float* power = reinterpret_cast<float*>(scratch + h * kHalf);
-        mel2_phase3_write(lane, pw, power);
+        float* power = reinterpret_cast<float*>(scratch + h * kN);
+        mel2_phase3_write<N2>(lane, pw, power);
         __syncwarp();
         if (f0 + fl0 + h < a.frames)
-          mel2_phase4(lane, a.num_mels, power, s_start, s_off, s_melw, outs + fl0 + h, kFramesPerBlock);
+          mel2_phase4(lane, a.num_mels, power, s_start, s_off, s_melw, outs + fl0 + h, kFPB);
       }
     }
     __syncthreads();
     // outs[m][fl] -> out[b][m][f0 + fl]
     float* ob = a.out + static_cast<size_t>(b) * a.num_mels * a.frames;
-    for (int i = tid; i < a.num_mels * kFramesPerBlock; i += kThreads2) {
-      const int m = i / kFramesPerBlock, fl = i % kFramesPerBlock;
+    for (int i = tid; i < a.num_mels * kFPB; i += kThreads2) {
+      const int m = i / kFPB, fl = i % kFPB;
       if (f0 + fl < a.frames) ob[static_cast<size_t>(m) * a.frames + f0 + fl] = outs[i];
     }
     __syncthreads();
@@ -438,8 +496,9 @@ __global__ void __launch_bounds__(kMel2Threads, 2) mel_kernel2(const Mel2Args a)
 }
 
 // ---------------------------------------------------------------------------------------------
-// Any other n_fft (the reference's other callers pass n_fft = a layer's kernel size at sr 16000,
-// src/speech_distillation/lightning_model.py:513-522, custom_layers.py:138-161): one block per frame, direct DFT
+// Every n_fft without an FFT path (not a power of two, or outside 256..2048: the reference's other callers pass n_fft =
+// a layer's kernel size at sr 16000, src/speech_distillation/lightning_model.py:513-522, custom_layers.py:138-161):
+// one block per frame, direct DFT
 // over a shared-memory twiddle table.  O(n_fft^2 / 2) per frame — a general-purpose path, not the tuned one.
 // Per-bin and per-mel phases are __host__ __device__ so hg_mel_emulate_host runs the same arithmetic.
 __host__ __device__ inline float dft_bin_power(int k, int n_fft, const float* xw, const float2* tw) {
@@ -532,16 +591,17 @@ extern "C" int hg_mel_plan_create(hg_mel_plan** out_plan, int n_fft, int num_mel
   const double two_pi = 6.283185307179586476925286766559;
   for (int i = 0; i < win_size; ++i)
     p->h_window[left + i] = static_cast<float>(0.5 - 0.5 * std::cos(two_pi * i / win_size));
-  p->h_tw512.resize(kHalf);
-  for (int m = 0; m < kHalf; ++m)
-    p->h_tw512[m] = make_float2(static_cast<float>(std::cos(two_pi * m / kHalf)),
-                                static_cast<float>(-std::sin(two_pi * m / kHalf)));
-  p->h_tw1024.resize(kHalf + 1);
-  for (int k = 0; k <= kHalf; ++k)
-    p->h_tw1024[k] = make_float2(static_cast<float>(std::cos(two_pi * k / kNfft)),
-                                 static_cast<float>(-std::sin(two_pi * k / kNfft)));
-
-  if (n_fft != kNfft) {
+  if (is_fft_size(n_fft)) {
+    const int half = n_fft / 2;
+    p->h_tw_half.resize(half);
+    for (int m = 0; m < half; ++m)
+      p->h_tw_half[m] = make_float2(static_cast<float>(std::cos(two_pi * m / half)),
+                                    static_cast<float>(-std::sin(two_pi * m / half)));
+    p->h_tw_full.resize(half + 1);
+    for (int k = 0; k <= half; ++k)
+      p->h_tw_full[k] = make_float2(static_cast<float>(std::cos(two_pi * k / n_fft)),
+                                    static_cast<float>(-std::sin(two_pi * k / n_fft)));
+  } else {
     p->h_tw_n.resize(n_fft);
     for (int n = 0; n < n_fft; ++n)
       p->h_tw_n[n] = make_float2(static_cast<float>(std::cos(two_pi * n / n_fft)),
@@ -585,7 +645,7 @@ extern "C" int hg_mel_plan_create(hg_mel_plan** out_plan, int n_fft, int num_mel
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
     // host-only plan (CPU emulation in tests); device tables stay null
     (void)cudaGetLastError();
-    p->window = nullptr; p->tw512 = nullptr; p->tw1024 = nullptr; p->tw_n = nullptr;
+    p->window = nullptr; p->tw_half = nullptr; p->tw_full = nullptr; p->tw_n = nullptr;
     p->mel_start = nullptr; p->mel_off = nullptr; p->mel_w = nullptr;
     *out_plan = p;
     return HG_OK;
@@ -595,9 +655,8 @@ extern "C" int hg_mel_plan_create(hg_mel_plan** out_plan, int n_fft, int num_mel
   HG_CHECK_CUDA(cudaMemcpyAsync(p->dst, p->src.data(), p->src.size() * sizeof(type),        \
                                 cudaMemcpyHostToDevice, st));
   HG_UP(window, h_window, float)
-  HG_UP(tw512, h_tw512, float2)
-  HG_UP(tw1024, h_tw1024, float2)
-  p->tw_n = nullptr;
+  p->tw_half = nullptr; p->tw_full = nullptr; p->tw_n = nullptr;
+  if (!p->h_tw_half.empty()) { HG_UP(tw_half, h_tw_half, float2) HG_UP(tw_full, h_tw_full, float2) }
   if (!p->h_tw_n.empty()) { HG_UP(tw_n, h_tw_n, float2) }
   HG_UP(mel_start, h_mel_start, int)
   HG_UP(mel_off, h_mel_off, int)
@@ -611,8 +670,8 @@ extern "C" int hg_mel_plan_create(hg_mel_plan** out_plan, int n_fft, int num_mel
 extern "C" int hg_mel_plan_destroy(hg_mel_plan* p) {
   if (!p) return HG_OK;
   if (p->window) cudaFree(p->window);
-  if (p->tw512) cudaFree(p->tw512);
-  if (p->tw1024) cudaFree(p->tw1024);
+  if (p->tw_half) cudaFree(p->tw_half);
+  if (p->tw_full) cudaFree(p->tw_full);
   if (p->tw_n) cudaFree(p->tw_n);
   if (p->mel_start) cudaFree(p->mel_start);
   if (p->mel_off) cudaFree(p->mel_off);
@@ -620,6 +679,49 @@ extern "C" int hg_mel_plan_destroy(hg_mel_plan* p) {
   delete p;
   return HG_OK;
 }
+
+namespace {
+
+// the last rFFT bin any mel filter reads: the forward un-packs and squares bins up to here only
+int mel_max_bin(const hg_mel_plan* plan) {
+  int max_bin = 0;
+  for (int m = 0; m < plan->num_mels; ++m) {
+    const int last = plan->h_mel_start[m] + (plan->h_mel_off[m + 1] - plan->h_mel_off[m]) - 1;
+    if (last > max_bin) max_bin = last;
+  }
+  return max_bin;
+}
+
+template <int N2>
+int launch_mel_kernel2(const hg_mel_plan* plan, const float* y, int batch, int t, int frames, float* out,
+                       float* minmax, cudaStream_t st) {
+  constexpr int kFPB = Mel2Size<N2>::kFramesPerBlock;
+  Mel2Args a{};
+  a.y = y; a.out = out; a.minmax = minmax;
+  a.batch = batch; a.t = t; a.frames = frames; a.hop = plan->hop; a.pad = plan->pad;
+  a.num_mels = plan->num_mels;
+  a.window = plan->window; a.tw_half = plan->tw_half; a.tw_full = plan->tw_full;
+  a.mel_start = plan->mel_start; a.mel_off = plan->mel_off; a.mel_w = plan->mel_w;
+  a.nnz = plan->nnz;
+  a.max_bin = mel_max_bin(plan);
+  a.groups_per_item = (frames + kFPB - 1) / kFPB;
+  a.total_groups = batch * a.groups_per_item;
+  const size_t smem = mel2_smem_layout<N2>(plan->num_mels, plan->nnz).total;
+  // two resident blocks per SM (the launch bounds and the grid below assume it)
+  HG_REQUIRE(smem <= 113 * 1024, "hg_mel_fwd: %zu bytes of shared memory per block", smem);
+  static hg::PerDeviceOnce once;                          // per instantiation
+  if (once.need(smem))
+    HG_CHECK_CUDA(cudaFuncSetAttribute(mel_kernel2<N2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int dev = 0, sms = 148;
+  if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int grid = a.total_groups < 2 * sms ? a.total_groups : 2 * sms;   // two resident blocks per SM, looping
+  mel_kernel2<N2><<<grid, kMel2Threads, smem, st>>>(a);
+  HG_CHECK_CUDA(cudaGetLastError());
+  g_hg_launches.fetch_add(1, std::memory_order_relaxed);
+  return HG_OK;
+}
+
+}  // namespace
 
 extern "C" int hg_mel_fwd(const hg_mel_plan* plan, const float* y, int batch, int t, float* out,
                           float* minmax, void* stream) {
@@ -629,44 +731,23 @@ extern "C" int hg_mel_fwd(const hg_mel_plan* plan, const float* y, int batch, in
   HG_REQUIRE(t > plan->pad, "hg_mel_fwd: reflect padding %d needs more than %d samples", plan->pad, t);
   const int frames = hg_mel_num_frames(plan, t);
   HG_REQUIRE(frames > 0, "hg_mel_fwd: input too short for one frame");
-  if (plan->n_fft != kNfft) {
-    const size_t smem = static_cast<size_t>(plan->n_fft) * (sizeof(float2) + sizeof(float)) +
-                        (plan->n_fft / 2 + 1) * sizeof(float);
-    static hg::PerDeviceOnce once;
-    if (once.need())
-      HG_CHECK_CUDA(cudaFuncSetAttribute(mel_dft_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-    dim3 grid(frames, batch);
-    mel_dft_kernel<<<grid, 256, smem, static_cast<cudaStream_t>(stream)>>>(
-        y, t, frames, plan->n_fft, plan->hop, plan->pad, plan->num_mels, plan->window, plan->tw_n, plan->mel_start,
-        plan->mel_off, plan->mel_w, out, minmax);
-    HG_CHECK_CUDA(cudaGetLastError());
-    g_hg_launches.fetch_add(1, std::memory_order_relaxed);
-    return HG_OK;
-  }
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  Mel2Args a{};
-  a.y = y; a.out = out; a.minmax = minmax;
-  a.batch = batch; a.t = t; a.frames = frames; a.hop = plan->hop; a.pad = plan->pad;
-  a.num_mels = plan->num_mels;
-  a.window = plan->window; a.tw512 = plan->tw512; a.tw1024 = plan->tw1024;
-  a.mel_start = plan->mel_start; a.mel_off = plan->mel_off; a.mel_w = plan->mel_w;
-  a.nnz = plan->nnz;
-  a.max_bin = 0;
-  for (int m = 0; m < plan->num_mels; ++m) {
-    const int last = plan->h_mel_start[m] + (plan->h_mel_off[m + 1] - plan->h_mel_off[m]) - 1;
-    if (last > a.max_bin) a.max_bin = last;
+  switch (plan->n_fft) {
+    case 256: return launch_mel_kernel2<4>(plan, y, batch, t, frames, out, minmax, st);
+    case 512: return launch_mel_kernel2<8>(plan, y, batch, t, frames, out, minmax, st);
+    case 1024: return launch_mel_kernel2<16>(plan, y, batch, t, frames, out, minmax, st);
+    case 2048: return launch_mel_kernel2<32>(plan, y, batch, t, frames, out, minmax, st);
+    default: break;
   }
-  a.groups_per_item = (frames + kFramesPerBlock - 1) / kFramesPerBlock;
-  a.total_groups = batch * a.groups_per_item;
-  const size_t smem = mel2_smem_layout(plan->num_mels, plan->nnz).total;
-  HG_REQUIRE(smem <= 113 * 1024, "hg_mel_fwd: %zu bytes of shared memory per block", smem);
-  static hg::PerDeviceOnce once2;
-  if (once2.need(smem))
-    HG_CHECK_CUDA(cudaFuncSetAttribute(mel_kernel2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int dev = 0, sms = 148;
-  if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  const int grid = a.total_groups < 2 * sms ? a.total_groups : 2 * sms;   // two resident blocks per SM, looping
-  mel_kernel2<<<grid, kMel2Threads, smem, st>>>(a);
+  const size_t smem = static_cast<size_t>(plan->n_fft) * (sizeof(float2) + sizeof(float)) +
+                      (plan->n_fft / 2 + 1) * sizeof(float);
+  static hg::PerDeviceOnce once;
+  if (once.need())
+    HG_CHECK_CUDA(cudaFuncSetAttribute(mel_dft_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+  dim3 grid(frames, batch);
+  mel_dft_kernel<<<grid, 256, smem, st>>>(
+      y, t, frames, plan->n_fft, plan->hop, plan->pad, plan->num_mels, plan->window, plan->tw_n, plan->mel_start,
+      plan->mel_off, plan->mel_w, out, minmax);
   HG_CHECK_CUDA(cudaGetLastError());
   g_hg_launches.fetch_add(1, std::memory_order_relaxed);
   return HG_OK;
@@ -674,41 +755,44 @@ extern "C" int hg_mel_fwd(const hg_mel_plan* plan, const float* y, int batch, in
 
 // ---------------------------------------------------------------------------------------------
 // mel_spectrogram backward (the generated-mel L1 term of the generator loss, UPSTREAM train.py: F.l1_loss(y_mel,
-// y_g_hat_mel) * 45 through src/meldataset.py:78-83).  One 64-thread group per frame, the radix-8 FFT of fft_pass:
-//   recompute Z = FFT512(packed windowed frame), un-pack X[0..512] (kept complex) and |X|^2, the CSR mel sums;
+// y_g_hat_mel) * 45 through src/meldataset.py:78-83).  One G-thread group per frame (G = max(32, N / 8), N = n_fft / 2),
+// the Stockham FFT of fft_pass (N = 8 x 8 x R3, and x 2 at N = 1024):
+//   recompute Z = FFT_N(packed windowed frame), un-pack X[0..N] (kept complex) and |X|^2, the CSR mel sums;
 //   dmel = g / mel above the 1e-5 clamp (0 below), dP[k] = sum_m fb[m][k] dmel[m], G[k] = 2 dP[k] X[k];
-//   the gradient at the windowed samples is S[n] = Re sum_{k=0..512} G[k] e^{+2 pi i k n / 1024}: the real inverse
-//   transform of the Hermitian spectrum H (H[k] = G[k] / 2, H[0] = Re G[0], H[512] = Re G[512]), taken as ONE
-//   512-point complex transform of Zc[k] = (H[k] + conj H[512-k]) + i e^{+2 pi i k / 1024} (H[k] - conj H[512-k])
-//   (S[2m] + i S[2m+1] = sum_k Zc[k] e^{+2 pi i m k / 512}), run through the same forward passes on conj(Zc);
+//   the gradient at the windowed samples is S[n] = Re sum_{k=0..N} G[k] e^{+2 pi i k n / 2N}: the real inverse
+//   transform of the Hermitian spectrum H (H[k] = G[k] / 2, H[0] = Re G[0], H[N] = Re G[N]), taken as ONE
+//   N-point complex transform of Zc[k] = (H[k] + conj H[N-k]) + i e^{+2 pi i k / 2N} (H[k] - conj H[N-k])
+//   (S[2m] + i S[2m+1] = sum_k Zc[k] e^{+2 pi i m k / N}), run through the same forward passes on conj(Zc);
 //   then the window, and a scatter-add into dy with the reflect padding folded back.
 // The phases are __host__ __device__ (hg_mel_bwd_emulate_host runs them with the threads serialised).
 namespace {
 
-// un-pack the real spectrum, keeping X complex: bins k = tid, tid + 64, ... (0..512)
+// un-pack the real spectrum, keeping X complex: bins k = tid, tid + G, ... (0..N)
+template <int N, int G>
 __host__ __device__ __forceinline__ void unpack_spectrum(int tid, const cpx* __restrict__ z, cpx* __restrict__ X,
                                                          float* __restrict__ power,
-                                                         const float2* __restrict__ tw1024) {
-  for (int k = tid; k <= kHalf; k += kGroupThreads) {
-    const cpx zk = z[padi(k & (kHalf - 1))];
-    cpx zc = z[padi((kHalf - k) & (kHalf - 1))];
+                                                         const float2* __restrict__ tw_full) {
+  for (int k = tid; k <= N; k += G) {
+    const cpx zk = z[padi(k & (N - 1))];
+    cpx zc = z[padi((N - k) & (N - 1))];
     zc.y = -zc.y;
     const cpx e = cpx{0.5f * (zk.x + zc.x), 0.5f * (zk.y + zc.y)};
     const cpx d = csub(zk, zc);
     const cpx o = cpx{0.5f * d.y, -0.5f * d.x};  // (zk - zc) / (2i)
-    const float2 w = tw1024[k];
+    const float2 w = tw_full[k];
     const cpx x = cadd(e, cmul(o, cpx{w.x, w.y}));
     X[k] = x;
     power[k] = x.x * x.x + x.y * x.y;
   }
 }
-// dm[m] = g[m] / mel[m] above the clamp, else 0 (m = tid, tid + 64, ...); also clears dP for the scatter
+// dm[m] = g[m] / mel[m] above the clamp, else 0 (m = tid, tid + G, ...); also clears dP for the scatter
+template <int N, int G>
 __host__ __device__ __forceinline__ void mel_grad(int tid, int num_mels, const float* __restrict__ power,
                                                   const int* __restrict__ mel_start, const int* __restrict__ mel_off,
                                                   const float* __restrict__ mel_w, const float* __restrict__ g_col,
                                                   int g_stride, float* __restrict__ dm, float* __restrict__ dp) {
-  for (int k = tid; k <= kHalf; k += kGroupThreads) dp[k] = 0.f;
-  for (int m = tid; m < num_mels; m += kGroupThreads) {
+  for (int k = tid; k <= N; k += G) dp[k] = 0.f;
+  for (int m = tid; m < num_mels; m += G) {
     const int s = mel_start[m], o = mel_off[m], n = mel_off[m + 1] - o;
     float acc = 0.f;
     for (int i = 0; i < n; ++i) acc += mel_w[o + i] * power[s + i];
@@ -716,11 +800,11 @@ __host__ __device__ __forceinline__ void mel_grad(int tid, int num_mels, const f
   }
 }
 // dP[k] += fb[m][k] * dm[m]
-template <bool DEVICE>
+template <int G>
 __host__ __device__ __forceinline__ void mel_scatter(int tid, int num_mels, const int* __restrict__ mel_start,
                                                      const int* __restrict__ mel_off, const float* __restrict__ mel_w,
                                                      const float* __restrict__ dm, float* __restrict__ dp) {
-  for (int m = tid; m < num_mels; m += kGroupThreads) {
+  for (int m = tid; m < num_mels; m += G) {
     const int s = mel_start[m], o = mel_off[m], n = mel_off[m + 1] - o;
     const float d = dm[m];
     for (int i = 0; i < n; ++i) {
@@ -732,31 +816,32 @@ __host__ __device__ __forceinline__ void mel_scatter(int tid, int num_mels, cons
     }
   }
 }
-// conj(Zc)[k] for k = tid, tid + 64, ... (0..511) into the padded FFT buffer
+// conj(Zc)[k] for k = tid, tid + G, ... (0..N-1) into the padded FFT buffer
+template <int N, int G>
 __host__ __device__ __forceinline__ void build_adjoint_input(int tid, const cpx* __restrict__ X,
                                                              const float* __restrict__ dp, cpx* __restrict__ out,
-                                                             const float2* __restrict__ tw1024) {
+                                                             const float2* __restrict__ tw_full) {
   auto hk = [&](int k) -> cpx {
     const float d = dp[k];
-    if (k == 0 || k == kHalf) return cpx{2.f * d * X[k].x, 0.f};
+    if (k == 0 || k == N) return cpx{2.f * d * X[k].x, 0.f};
     return cpx{d * X[k].x, d * X[k].y};
   };
-  for (int k = tid; k < kHalf; k += kGroupThreads) {
+  for (int k = tid; k < N; k += G) {
     const cpx a = hk(k);
-    cpx b = hk(kHalf - k);
+    cpx b = hk(N - k);
     b.y = -b.y;
     const cpx sum = cadd(a, b), dif = csub(a, b);
-    const float2 w = tw1024[k];                       // e^{-2 pi i k / 1024}; its conjugate is needed
-    const cpx rot = cmul(dif, cpx{w.x, -w.y});        // e^{+2 pi i k / 1024} (a - b)
+    const float2 w = tw_full[k];                      // e^{-2 pi i k / 2N}; its conjugate is needed
+    const cpx rot = cmul(dif, cpx{w.x, -w.y});        // e^{+2 pi i k / 2N} (a - b)
     const cpx zc = cpx{sum.x - rot.y, sum.y + rot.x};  // sum + i * rot
     out[padi(k)] = cpx{zc.x, -zc.y};
   }
 }
-// samples 2m, 2m+1 of the frame's gradient from R = FFT512(conj Zc): S[2m] = R[m].x, S[2m+1] = -R[m].y
-template <bool DEVICE>
+// samples 2m, 2m+1 of the frame's gradient from R = FFT_N(conj Zc): S[2m] = R[m].x, S[2m+1] = -R[m].y
+template <int N, int G>
 __host__ __device__ __forceinline__ void scatter_frame(int tid, const cpx* __restrict__ r, const float* __restrict__ window,
                                                        int frame_start, int t, float* __restrict__ dy_row) {
-  for (int m = tid; m < kHalf; m += kGroupThreads) {
+  for (int m = tid; m < N; m += G) {
     const cpx v = r[padi(m)];
     const float s0 = v.x * window[2 * m], s1 = -v.y * window[2 * m + 1];
     const int i0 = reflect_index(frame_start + 2 * m, t), i1 = reflect_index(frame_start + 2 * m + 1, t);
@@ -770,50 +855,164 @@ __host__ __device__ __forceinline__ void scatter_frame(int tid, const cpx* __res
   }
 }
 
-constexpr int kBwdGroups = 2;                       // frames per block (39 KB of static shared memory)
+// geometry of mel_bwd_kernel<N>: G threads per frame group (whole warps for bar.sync, at least one butterfly per
+// thread in a radix-8 pass from N = 256 up), 128 threads a block; the static shared memory stays under 40 KB
+// (N = 128 / 256 / 512 / 1024: 4 / 4 / 2 / 1 frames a block, 21 / 40 / 39 / 38 KB)
+template <int N>
+struct BwdSize {
+  static constexpr int kG = N / 8 < 32 ? 32 : N / 8;
+  static constexpr int kGroups = 128 / kG;
+  static constexpr int kPasses = N == 1024 ? 4 : 3;
+};
 
-__global__ void __launch_bounds__(kBwdGroups* kGroupThreads)
+// the N-point transform of a frame group, ping-ponging from `in` (unused when FIRST: pass 0 reads the staged samples)
+// through `other`; returns the buffer that holds the result (`other` after an odd number of passes, else `in`)
+template <int N, int G, bool FIRST>
+__device__ __forceinline__ cpx* group_fft(int j, int g, cpx* in, cpx* other, const float* __restrict__ samples,
+                                          const float* __restrict__ window, const float2* __restrict__ tw) {
+  fft_pass_group<8, N, G, FIRST>(j, 1, in, other, samples, window, tw);
+  group_sync<G>(g);
+  fft_pass_group<8, N, G, false>(j, 8, other, in, nullptr, nullptr, tw);
+  group_sync<G>(g);
+  fft_pass_group<third_radix(N), N, G, false>(j, 64, in, other, nullptr, nullptr, tw);
+  group_sync<G>(g);
+  if constexpr (BwdSize<N>::kPasses == 4) {
+    fft_pass_group<2, N, G, false>(j, 512, other, in, nullptr, nullptr, tw);
+    group_sync<G>(g);
+    return in;
+  }
+  return other;
+}
+// the same passes with the G threads serialised (hg_mel_bwd_emulate_host)
+template <int N, int G, bool FIRST>
+cpx* host_fft(cpx* in, cpx* other, const float* samples, const float* window, const float2* tw) {
+  for (int j = 0; j < G; ++j) fft_pass_group<8, N, G, FIRST>(j, 1, in, other, samples, window, tw);
+  for (int j = 0; j < G; ++j) fft_pass_group<8, N, G, false>(j, 8, other, in, nullptr, nullptr, tw);
+  for (int j = 0; j < G; ++j) fft_pass_group<third_radix(N), N, G, false>(j, 64, in, other, nullptr, nullptr, tw);
+  if constexpr (BwdSize<N>::kPasses == 4) {
+    for (int j = 0; j < G; ++j) fft_pass_group<2, N, G, false>(j, 512, other, in, nullptr, nullptr, tw);
+    return in;
+  }
+  return other;
+}
+
+template <int N>
+__global__ void __launch_bounds__(BwdSize<N>::kGroups * BwdSize<N>::kG)
 mel_bwd_kernel(const float* __restrict__ y, const float* __restrict__ dmel, int t, int frames, int hop, int pad,
-               int num_mels, const float* __restrict__ window, const float2* __restrict__ tw512,
-               const float2* __restrict__ tw1024, const int* __restrict__ mel_start, const int* __restrict__ mel_off,
+               int num_mels, const float* __restrict__ window, const float2* __restrict__ tw_half,
+               const float2* __restrict__ tw_full, const int* __restrict__ mel_start, const int* __restrict__ mel_off,
                const float* __restrict__ mel_w, float* __restrict__ dy) {
-  __shared__ float smp[kBwdGroups][kNfft];
-  __shared__ cpx zbuf[kBwdGroups][2][kPadLen];
-  __shared__ cpx xs[kBwdGroups][kHalf + 1];
-  __shared__ float dps[kBwdGroups][kHalf + 1];
-  __shared__ float dms[kBwdGroups][128];
-  const int g = threadIdx.x / kGroupThreads, j = threadIdx.x % kGroupThreads;
-  const int f = blockIdx.x * kBwdGroups + g, b = blockIdx.y;
+  constexpr int G = BwdSize<N>::kG, kGroups = BwdSize<N>::kGroups;
+  constexpr bool kOdd = BwdSize<N>::kPasses & 1;
+  __shared__ float smp[kGroups][2 * N];
+  __shared__ cpx zbuf[kGroups][2][pad_len(N)];
+  __shared__ cpx xs[kGroups][N + 1];
+  __shared__ float dps[kGroups][N + 1];
+  __shared__ float dms[kGroups][128];
+  const int g = threadIdx.x / G, j = threadIdx.x % G;
+  const int f = blockIdx.x * kGroups + g, b = blockIdx.y;
   if (f >= frames) return;                          // group-uniform; the groups only meet on their own barriers
   const float* yb = y + static_cast<size_t>(b) * t;
   const int start = f * hop - pad;
-  for (int n = j; n < kNfft; n += kGroupThreads) smp[g][n] = yb[reflect_index(start + n, t)];
-  group_sync(g);
+  for (int n = j; n < 2 * N; n += G) smp[g][n] = yb[reflect_index(start + n, t)];
+  group_sync<G>(g);
   cpx* z0 = zbuf[g][0];
   cpx* z1 = zbuf[g][1];
-  fft_pass<true>(j, 1, nullptr, z0, smp[g], window, tw512);
-  group_sync(g);
-  fft_pass<false>(j, 8, z0, z1, nullptr, nullptr, tw512);
-  group_sync(g);
-  fft_pass<false>(j, 64, z1, z0, nullptr, nullptr, tw512);
-  group_sync(g);
-  float* power = reinterpret_cast<float*>(z1);
-  unpack_spectrum(j, z0, xs[g], power, tw1024);
-  group_sync(g);
-  mel_grad(j, num_mels, power, mel_start, mel_off, mel_w, dmel + static_cast<size_t>(b) * num_mels * frames + f, frames,
-           dms[g], dps[g]);
-  group_sync(g);
-  mel_scatter<true>(j, num_mels, mel_start, mel_off, mel_w, dms[g], dps[g]);
-  group_sync(g);
-  build_adjoint_input(j, xs[g], dps[g], z1, tw1024);
-  group_sync(g);
-  fft_pass<false>(j, 1, z1, z0, nullptr, nullptr, tw512);
-  group_sync(g);
-  fft_pass<false>(j, 8, z0, z1, nullptr, nullptr, tw512);
-  group_sync(g);
-  fft_pass<false>(j, 64, z1, z0, nullptr, nullptr, tw512);
-  group_sync(g);
-  scatter_frame<true>(j, z0, window, start, t, dy + static_cast<size_t>(b) * t);
+  cpx* zr = kOdd ? z0 : z1;                         // where the recomputed spectrum lands
+  cpx* zo = kOdd ? z1 : z0;
+  group_fft<N, G, true>(j, g, z1, z0, smp[g], window, tw_half);
+  float* power = reinterpret_cast<float*>(zo);
+  unpack_spectrum<N, G>(j, zr, xs[g], power, tw_full);
+  group_sync<G>(g);
+  mel_grad<N, G>(j, num_mels, power, mel_start, mel_off, mel_w,
+                 dmel + static_cast<size_t>(b) * num_mels * frames + f, frames, dms[g], dps[g]);
+  group_sync<G>(g);
+  mel_scatter<G>(j, num_mels, mel_start, mel_off, mel_w, dms[g], dps[g]);
+  group_sync<G>(g);
+  build_adjoint_input<N, G>(j, xs[g], dps[g], zo, tw_full);
+  group_sync<G>(g);
+  const cpx* r = group_fft<N, G, false>(j, g, zo, zr, nullptr, nullptr, tw_half);
+  scatter_frame<N, G>(j, r, window, start, t, dy + static_cast<size_t>(b) * t);
+}
+
+template <int N>
+int launch_mel_bwd(const hg_mel_plan* plan, const float* y, const float* dmel, int batch, int t, int frames, float* dy,
+                   cudaStream_t st) {
+  constexpr int kGroups = BwdSize<N>::kGroups;
+  dim3 grid((frames + kGroups - 1) / kGroups, batch);
+  mel_bwd_kernel<N><<<grid, kGroups * BwdSize<N>::kG, 0, st>>>(
+      y, dmel, t, frames, plan->hop, plan->pad, plan->num_mels, plan->window, plan->tw_half, plan->tw_full,
+      plan->mel_start, plan->mel_off, plan->mel_w, dy);
+  HG_CHECK_CUDA(cudaGetLastError());
+  g_hg_launches.fetch_add(1, std::memory_order_relaxed);
+  return HG_OK;
+}
+
+template <int N>
+void mel_bwd_emulate(const hg_mel_plan* plan, const float* host_y, const float* host_dmel, int batch, int t,
+                     int frames, float* host_dy) {
+  constexpr int G = BwdSize<N>::kG;
+  std::vector<float> smp(2 * N), dp(N + 1), dm(128);
+  std::vector<cpx> z0(pad_len(N)), z1(pad_len(N)), X(N + 1);
+  const float* win = plan->h_window.data();
+  const float2 *twh = plan->h_tw_half.data(), *twf = plan->h_tw_full.data();
+  const int *ms = plan->h_mel_start.data(), *mo = plan->h_mel_off.data();
+  const float* mw = plan->h_mel_w.data();
+  for (int b = 0; b < batch; ++b)
+    for (int f = 0; f < frames; ++f) {
+      const int start = f * plan->hop - plan->pad;
+      for (int n = 0; n < 2 * N; ++n) smp[n] = host_y[static_cast<size_t>(b) * t + reflect_index(start + n, t)];
+      cpx* zr = host_fft<N, G, true>(z1.data(), z0.data(), smp.data(), win, twh);
+      cpx* zo = zr == z0.data() ? z1.data() : z0.data();
+      float* power = reinterpret_cast<float*>(zo);
+      for (int j = 0; j < G; ++j) unpack_spectrum<N, G>(j, zr, X.data(), power, twf);
+      for (int j = 0; j < G; ++j)
+        mel_grad<N, G>(j, plan->num_mels, power, ms, mo, mw,
+                       host_dmel + static_cast<size_t>(b) * plan->num_mels * frames + f, frames, dm.data(), dp.data());
+      for (int j = 0; j < G; ++j) mel_scatter<G>(j, plan->num_mels, ms, mo, mw, dm.data(), dp.data());
+      for (int j = 0; j < G; ++j) build_adjoint_input<N, G>(j, X.data(), dp.data(), zo, twf);
+      const cpx* r = host_fft<N, G, false>(zo, zr, nullptr, nullptr, twh);
+      for (int j = 0; j < G; ++j) scatter_frame<N, G>(j, r, win, start, t, host_dy + static_cast<size_t>(b) * t);
+    }
+}
+
+// mel_kernel2<N2>'s lane phases, the 32 lanes of a warp serialised, 32 / N2 frames at a time
+template <int N2>
+void mel_emulate(const hg_mel_plan* plan, const float* host_y, int batch, int t, int frames, float* host_out) {
+  using S = Mel2Size<N2>;
+  constexpr int kFPW = S::kFramesPerWarp;
+  std::vector<cpx> scratch(kWarpScratch);
+  std::vector<float2> twp(S::kTwPad);
+  for (int i = 0; i < S::kN; ++i) twp[padi(i)] = plan->h_tw_half[i];
+  const int max_bin = mel_max_bin(plan);
+  std::vector<cpx> regs(32 * 32);                  // each lane's 32 phase-2 registers
+  std::vector<float> pws(32 * (N2 + 1));
+  for (int b = 0; b < batch; ++b)
+    for (int f0 = 0; f0 < frames; f0 += kFPW) {
+      const float* yb = host_y + static_cast<size_t>(b) * t;
+      for (int lane = 0; lane < 32; ++lane) {
+        const int f = f0 + lane / N2;
+        const int start = (f < frames ? f : frames - 1) * plan->hop - plan->pad;
+        float lo = 0.f, hi = 0.f;
+        mel2_phase1<N2>(lane, yb, start, t, false, plan->h_window.data(), twp.data(), scratch.data(), lo, hi);
+      }
+      for (int lane = 0; lane < 32; ++lane)
+        mel2_phase2_read<N2>(lane, scratch.data(), *reinterpret_cast<cpx(*)[kFPW][N2]>(&regs[lane * 32]));
+      for (int lane = 0; lane < 32; ++lane)
+        mel2_phase2_write<N2>(lane, *reinterpret_cast<cpx(*)[kFPW][N2]>(&regs[lane * 32]), scratch.data());
+      for (int h = 0; h < kFPW && f0 + h < frames; ++h) {
+        for (int lane = 0; lane < 32; ++lane)
+          mel2_phase3_compute<N2>(lane, scratch.data() + h * S::kN, max_bin, plan->h_tw_full.data(),
+                                  *reinterpret_cast<float(*)[N2 + 1]>(&pws[lane * (N2 + 1)]));
+        float* power = reinterpret_cast<float*>(scratch.data() + h * S::kN);
+        for (int lane = 0; lane < 32; ++lane)
+          mel2_phase3_write<N2>(lane, *reinterpret_cast<float(*)[N2 + 1]>(&pws[lane * (N2 + 1)]), power);
+        float* col = host_out + static_cast<size_t>(b) * plan->num_mels * frames + f0 + h;
+        for (int lane = 0; lane < 32; ++lane)
+          mel2_phase4(lane, plan->num_mels, power, plan->h_mel_start.data(), plan->h_mel_off.data(),
+                      plan->h_mel_w.data(), col, frames);
+      }
+    }
 }
 
 }  // namespace
@@ -822,18 +1021,17 @@ extern "C" int hg_mel_bwd(const hg_mel_plan* plan, const float* y, const float* 
                           void* stream) {
   HG_REQUIRE(plan && y && dmel && dy, "hg_mel_bwd: null pointer");
   HG_REQUIRE(plan->window, "hg_mel_bwd: plan has no device tables");
-  HG_REQUIRE(plan->n_fft == kNfft, "hg_mel_bwd: only n_fft == 1024 (the training configs) is implemented (got %d)",
-             plan->n_fft);
+  HG_REQUIRE(is_fft_size(plan->n_fft), "hg_mel_bwd: n_fft must be 256, 512, 1024 or 2048 (got %d)", plan->n_fft);
   HG_REQUIRE(batch > 0 && batch <= 65535 && t > plan->pad && plan->num_mels <= 128, "hg_mel_bwd: bad arguments");
   const int frames = hg_mel_num_frames(plan, t);
   HG_REQUIRE(frames > 0, "hg_mel_bwd: input too short for one frame");
-  dim3 grid((frames + kBwdGroups - 1) / kBwdGroups, batch);
-  mel_bwd_kernel<<<grid, kBwdGroups * kGroupThreads, 0, static_cast<cudaStream_t>(stream)>>>(
-      y, dmel, t, frames, plan->hop, plan->pad, plan->num_mels, plan->window, plan->tw512, plan->tw1024,
-      plan->mel_start, plan->mel_off, plan->mel_w, dy);
-  HG_CHECK_CUDA(cudaGetLastError());
-  g_hg_launches.fetch_add(1, std::memory_order_relaxed);
-  return HG_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  switch (plan->n_fft) {
+    case 256: return launch_mel_bwd<128>(plan, y, dmel, batch, t, frames, dy, st);
+    case 512: return launch_mel_bwd<256>(plan, y, dmel, batch, t, frames, dy, st);
+    case 1024: return launch_mel_bwd<512>(plan, y, dmel, batch, t, frames, dy, st);
+    default: return launch_mel_bwd<1024>(plan, y, dmel, batch, t, frames, dy, st);
+  }
 }
 
 // Test hook: the backward kernel's phase functions on the HOST (threads serialised).  host_y fp32 [B][T],
@@ -841,34 +1039,16 @@ extern "C" int hg_mel_bwd(const hg_mel_plan* plan, const float* y, const float* 
 extern "C" int hg_mel_bwd_emulate_host(const hg_mel_plan* plan, const float* host_y, const float* host_dmel,
                                        int batch, int t, float* host_dy) {
   HG_REQUIRE(plan && host_y && host_dmel && host_dy, "hg_mel_bwd_emulate_host: null pointer");
-  HG_REQUIRE(plan->n_fft == kNfft, "hg_mel_bwd_emulate_host: only n_fft == 1024 is implemented");
+  HG_REQUIRE(is_fft_size(plan->n_fft), "hg_mel_bwd_emulate_host: n_fft must be 256, 512, 1024 or 2048 (got %d)",
+             plan->n_fft);
   const int frames = hg_mel_num_frames(plan, t);
   HG_REQUIRE(frames > 0 && t > plan->pad, "hg_mel_bwd_emulate_host: input too short");
-  std::vector<float> smp(plan->n_fft), dp(kHalf + 1), dm(128);
-  std::vector<cpx> z0(kPadLen), z1(kPadLen), X(kHalf + 1);
-  const float* win = plan->h_window.data();
-  const float2 *t512 = plan->h_tw512.data(), *t1024 = plan->h_tw1024.data();
-  const int *ms = plan->h_mel_start.data(), *mo = plan->h_mel_off.data();
-  const float* mw = plan->h_mel_w.data();
-  for (int b = 0; b < batch; ++b)
-    for (int f = 0; f < frames; ++f) {
-      const int start = f * plan->hop - plan->pad;
-      for (int n = 0; n < plan->n_fft; ++n) smp[n] = host_y[static_cast<size_t>(b) * t + reflect_index(start + n, t)];
-      for (int j = 0; j < 64; ++j) fft_pass<true>(j, 1, nullptr, z0.data(), smp.data(), win, t512);
-      for (int j = 0; j < 64; ++j) fft_pass<false>(j, 8, z0.data(), z1.data(), nullptr, nullptr, t512);
-      for (int j = 0; j < 64; ++j) fft_pass<false>(j, 64, z1.data(), z0.data(), nullptr, nullptr, t512);
-      float* power = reinterpret_cast<float*>(z1.data());
-      for (int j = 0; j < 64; ++j) unpack_spectrum(j, z0.data(), X.data(), power, t1024);
-      for (int j = 0; j < 64; ++j)
-        mel_grad(j, plan->num_mels, power, ms, mo, mw, host_dmel + static_cast<size_t>(b) * plan->num_mels * frames + f,
-                 frames, dm.data(), dp.data());
-      for (int j = 0; j < 64; ++j) mel_scatter<false>(j, plan->num_mels, ms, mo, mw, dm.data(), dp.data());
-      for (int j = 0; j < 64; ++j) build_adjoint_input(j, X.data(), dp.data(), z1.data(), t1024);
-      for (int j = 0; j < 64; ++j) fft_pass<false>(j, 1, z1.data(), z0.data(), nullptr, nullptr, t512);
-      for (int j = 0; j < 64; ++j) fft_pass<false>(j, 8, z0.data(), z1.data(), nullptr, nullptr, t512);
-      for (int j = 0; j < 64; ++j) fft_pass<false>(j, 64, z1.data(), z0.data(), nullptr, nullptr, t512);
-      for (int j = 0; j < 64; ++j) scatter_frame<false>(j, z0.data(), win, start, t, host_dy + static_cast<size_t>(b) * t);
-    }
+  switch (plan->n_fft) {
+    case 256: mel_bwd_emulate<128>(plan, host_y, host_dmel, batch, t, frames, host_dy); break;
+    case 512: mel_bwd_emulate<256>(plan, host_y, host_dmel, batch, t, frames, host_dy); break;
+    case 1024: mel_bwd_emulate<512>(plan, host_y, host_dmel, batch, t, frames, host_dy); break;
+    default: mel_bwd_emulate<1024>(plan, host_y, host_dmel, batch, t, frames, host_dy); break;
+  }
   return HG_OK;
 }
 
@@ -881,59 +1061,24 @@ extern "C" int hg_mel_emulate_host(const hg_mel_plan* plan, const float* host_y,
   HG_REQUIRE(plan && host_y && host_out, "hg_mel_emulate_host: null pointer");
   const int frames = hg_mel_num_frames(plan, t);
   HG_REQUIRE(frames > 0 && t > plan->pad, "hg_mel_emulate_host: input too short");
-  if (plan->n_fft != kNfft) {
-    const int n_fft = plan->n_fft, nbins = n_fft / 2 + 1;
-    std::vector<float> xw(n_fft), pw(nbins);
-    for (int b = 0; b < batch; ++b)
-      for (int f = 0; f < frames; ++f) {
-        for (int n = 0; n < n_fft; ++n)
-          xw[n] = host_y[static_cast<size_t>(b) * t + reflect_index(f * plan->hop - plan->pad + n, t)] *
-                  plan->h_window[n];
-        for (int k = 0; k < nbins; ++k) pw[k] = dft_bin_power(k, n_fft, xw.data(), plan->h_tw_n.data());
-        for (int m = 0; m < plan->num_mels; ++m)
-          host_out[(static_cast<size_t>(b) * plan->num_mels + m) * frames + f] =
-              mel_bin_log(m, pw.data(), plan->h_mel_start.data(), plan->h_mel_off.data(), plan->h_mel_w.data());
-      }
-    return HG_OK;
+  switch (plan->n_fft) {
+    case 256: mel_emulate<4>(plan, host_y, batch, t, frames, host_out); return HG_OK;
+    case 512: mel_emulate<8>(plan, host_y, batch, t, frames, host_out); return HG_OK;
+    case 1024: mel_emulate<16>(plan, host_y, batch, t, frames, host_out); return HG_OK;
+    case 2048: mel_emulate<32>(plan, host_y, batch, t, frames, host_out); return HG_OK;
+    default: break;
   }
-  // mel_kernel2's lane phases, the 32 lanes of a warp serialised, two frames at a time
-  std::vector<cpx> scratch(kWarpScratch);
-  std::vector<float2> tw512p(kTwPad);
-  for (int i = 0; i < kHalf; ++i) tw512p[padi(i)] = plan->h_tw512[i];
-  int max_bin = 0;
-  for (int m = 0; m < plan->num_mels; ++m) {
-    const int last = plan->h_mel_start[m] + (plan->h_mel_off[m + 1] - plan->h_mel_off[m]) - 1;
-    if (last > max_bin) max_bin = last;
-  }
-  std::vector<cpx> ra(32 * 16), rb(32 * 16);
-  std::vector<float> pws(32 * 17);
+  const int n_fft = plan->n_fft, nbins = n_fft / 2 + 1;
+  std::vector<float> xw(n_fft), pw(nbins);
   for (int b = 0; b < batch; ++b)
-    for (int f0 = 0; f0 < frames; f0 += 2) {
-      const float* yb = host_y + static_cast<size_t>(b) * t;
-      for (int lane = 0; lane < 32; ++lane) {
-        const int f = f0 + (lane >> 4);
-        const int start = (f < frames ? f : frames - 1) * plan->hop - plan->pad;
-        float lo = 0.f, hi = 0.f;
-        mel2_phase1(lane, yb, start, t, false, plan->h_window.data(), tw512p.data(), scratch.data(), lo, hi);
-      }
-      for (int lane = 0; lane < 32; ++lane)
-        mel2_phase2_read(lane, scratch.data(), *reinterpret_cast<cpx(*)[16]>(&ra[lane * 16]),
-                         *reinterpret_cast<cpx(*)[16]>(&rb[lane * 16]));
-      for (int lane = 0; lane < 32; ++lane)
-        mel2_phase2_write(lane, *reinterpret_cast<cpx(*)[16]>(&ra[lane * 16]),
-                          *reinterpret_cast<cpx(*)[16]>(&rb[lane * 16]), scratch.data());
-      for (int h = 0; h < 2 && f0 + h < frames; ++h) {
-        for (int lane = 0; lane < 32; ++lane)
-          mel2_phase3_compute(lane, scratch.data() + h * kHalf, max_bin, plan->h_tw1024.data(),
-                              *reinterpret_cast<float(*)[17]>(&pws[lane * 17]));
-        float* power = reinterpret_cast<float*>(scratch.data() + h * kHalf);
-        for (int lane = 0; lane < 32; ++lane)
-          mel2_phase3_write(lane, *reinterpret_cast<float(*)[17]>(&pws[lane * 17]), power);
-        float* col = host_out + static_cast<size_t>(b) * plan->num_mels * frames + f0 + h;
-        for (int lane = 0; lane < 32; ++lane)
-          mel2_phase4(lane, plan->num_mels, power, plan->h_mel_start.data(), plan->h_mel_off.data(),
-                      plan->h_mel_w.data(), col, frames);
-      }
+    for (int f = 0; f < frames; ++f) {
+      for (int n = 0; n < n_fft; ++n)
+        xw[n] = host_y[static_cast<size_t>(b) * t + reflect_index(f * plan->hop - plan->pad + n, t)] *
+                plan->h_window[n];
+      for (int k = 0; k < nbins; ++k) pw[k] = dft_bin_power(k, n_fft, xw.data(), plan->h_tw_n.data());
+      for (int m = 0; m < plan->num_mels; ++m)
+        host_out[(static_cast<size_t>(b) * plan->num_mels + m) * frames + f] =
+            mel_bin_log(m, pw.data(), plan->h_mel_start.data(), plan->h_mel_off.data(), plan->h_mel_w.data());
     }
   return HG_OK;
 }

@@ -210,9 +210,10 @@ int hg_conv_post_tanh_fwd(const void* x, const float* w, const float* bias, int 
  * periodic Hann window, rFFT(n_fft), |X|^2, HTK mel filterbank (un-normalised triangles), and
  * log(clamp(., 1e-5)) in ONE kernel.  The plan owns the immutable tables (window, twiddles, sparse
  * filterbank), keyed like the reference's cache key (meldataset.py:57).
- * n_fft == 1024 (every HiFi-GAN config) runs the fused radix-8 FFT kernel; any other even n_fft in [16, 4096]
- * (the reference's other callers: src/speech_distillation/lightning_model.py:513-522 pass 16 kHz / fmax None /
- * n_fft = a layer's kernel size) runs a general direct-DFT kernel, one block per frame.
+ * n_fft 256 / 512 / 1024 / 2048 (the 16 kHz, 22.05 kHz and 44.1 / 48 kHz HiFi-GAN recipes) run the fused kernel with
+ * the FFT held in registers; any other even n_fft in [16, 4096] (the reference's other callers:
+ * src/speech_distillation/lightning_model.py:513-522 pass 16 kHz / fmax None / n_fft = a layer's kernel size) runs a
+ * general direct-DFT kernel, one block per frame.
  * win_size <= n_fft, hop_size <= n_fft, num_mels <= 128.
  */
 typedef struct hg_mel_plan hg_mel_plan;
@@ -230,12 +231,12 @@ int hg_mel_fwd(const hg_mel_plan* plan, const float* y, int batch, int t, float*
 
 /* hg_mel_bwd — backward of hg_mel_fwd: dmel fp32 [B][num_mels][frames] (gradient at the log-mel output) ->
  * dy fp32 [B][T] ADDED to (zero it first).  y is the forward input; the spectrum is recomputed with the forward
- * kernel's FFT and the adjoint is one more 512-point transform per frame.  n_fft == 1024 only (the training configs). */
+ * kernel's FFT and the adjoint is one more n_fft / 2-point transform per frame.  n_fft 256, 512, 1024 or 2048. */
 int hg_mel_bwd(const hg_mel_plan* plan, const float* y, const float* dmel, int batch, int t, float* dy,
                void* stream);
 
 /* Test hook: the backward kernel's phase functions on the HOST (threads serialised).  host_y fp32 [B][T], host_dmel
- * fp32 [B][num_mels][frames]; host_dy fp32 [B][T] is ADDED to.  n_fft == 1024 only. */
+ * fp32 [B][num_mels][frames]; host_dy fp32 [B][T] is ADDED to.  n_fft 256, 512, 1024 or 2048. */
 int hg_mel_bwd_emulate_host(const hg_mel_plan* plan, const float* host_y, const float* host_dmel, int batch, int t,
                             float* host_dy);
 
