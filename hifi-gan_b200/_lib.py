@@ -179,6 +179,13 @@ _SIGNATURES = {
                              c_void_p, c_void_p]),
     "hg_adamw_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, ctypes.c_longlong, c_float, c_float, c_float,
                               c_float, c_float, c_int, c_void_p, c_void_p, c_float, c_void_p]),
+    "hg_grad_norm_slot_size": (c_int, []),
+    "hg_grad_sumsq": (c_int, [c_void_p, ctypes.c_longlong, c_void_p, c_void_p]),
+    "hg_grad_norm_finalize": (c_int, [c_void_p, c_int, c_float, c_float, c_void_p, c_void_p, c_void_p, c_void_p,
+                                      c_void_p, c_void_p]),
+    "hg_adamw_step_guarded": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, ctypes.c_longlong, c_float, c_float,
+                                      c_float, c_float, c_float, c_void_p, c_void_p, c_float, c_void_p, c_void_p,
+                                      c_void_p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

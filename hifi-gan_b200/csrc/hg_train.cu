@@ -6,7 +6,8 @@
 //   * loss gradients (src/models.py:251-282 + the mel L1), L1 sums over internal bf16 feature maps
 //   * unpacking of hg_conv1d_wgrad results to the parameter layout, weight_norm backward
 //     (torch._weight_norm_interface_backward; reparametrisation at src/models.py:16-31,81,86-88,96,132-140)
-//   * AdamW (torch.optim.AdamW semantics, decoupled weight decay)
+//   * AdamW (torch.optim.AdamW semantics, decoupled weight decay), and the gradient norm of
+//     torch.nn.utils.clip_grad_norm_ with the skip of a non-finite step that guards it
 #include "hg_common.cuh"
 
 #include <atomic>
@@ -570,11 +571,19 @@ weight_norm_bwd_kernel(const float* __restrict__ dw, const float* __restrict__ v
   if (threadIdx.x == 0) dg[r] = accumulate ? dg[r] + dot * inv : dot * inv;
 }
 
-// torch.optim.AdamW step on one flat fp32 tensor
+// torch.optim.AdamW step on one flat fp32 tensor.  kGuard: the clip_grad_norm_ / non-finite-skip flavour — nothing
+// is written when *skip is set, otherwise the gradient scale is multiplied by *clip_coef (hg_grad_norm_finalize).
+// The guard arguments come last so the unguarded instantiation keeps its parameter offsets.
+template <bool kGuard>
 __global__ void adamw_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                              float* __restrict__ v, long long n, float lr, float b1, float b2, float eps, float wd,
                              float bc1, float bc2_sqrt, float gscale, const int* __restrict__ dev_step,
-                             const float* __restrict__ dev_lr) {
+                             const float* __restrict__ dev_lr, const float* __restrict__ clip_coef,
+                             const int* __restrict__ skip) {
+  if constexpr (kGuard) {
+    if (*skip) return;
+    gscale = gscale * *clip_coef;
+  }
   if (dev_step) {   // step counter kept on the device so a captured CUDA graph advances it
     const float st = static_cast<float>(*dev_step);
     bc1 = 1.f - powf(b1, st);
@@ -780,6 +789,87 @@ sn_bwd_apply_kernel(const float* __restrict__ d, const float* __restrict__ u, co
   }
 }
 
+// ---- gradient norm (torch.nn.utils.clip_grad_norm_) -------------------------------------------------------------
+// Deterministic: the grid and every thread's share depend on n alone, the sums run in a fixed order, and no
+// floating-point atomics are used, so the same gradient bits give the same norm bits on any stream or lane order.
+constexpr int kNormSlot = 1024;         // per-block partials of one hg_grad_sumsq call = max blocks
+constexpr int kNormPerBlock = 4096;     // at least 16 elements (4 groups) per thread before another block is added
+
+__device__ __forceinline__ double warp_sum_d(double v) {
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
+
+// 256 threads: the fixed-order block sum of one double per thread (valid in thread 0)
+__device__ __forceinline__ double block_sum_d(double v, double* red) {
+  v = warp_sum_d(v);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  double s = 0.0;
+  if (threadIdx.x == 0)
+    for (int i = 0; i < 8; ++i) s += red[i];
+  return s;
+}
+
+inline int norm_blocks(long long n) {
+  const long long b = (n + kNormPerBlock - 1) / kNormPerBlock;
+  return static_cast<int>(b < 1 ? 1 : (b > kNormSlot ? kNormSlot : b));
+}
+
+// partial[b] = sum of x^2 over the 4-element groups j = b*256 + tid (+ k * grid * 256) of block b, the squares of
+// one group summed in fp32, the groups of a thread in fp64.  16-byte loads when x is 16-byte aligned; otherwise the
+// same groups are read element by element, so the result does not depend on the alignment.  Blocks past the grid
+// write zeros into the rest of the slot (the finalize sums the whole slot).
+__global__ void __launch_bounds__(256)
+grad_sumsq_kernel(const float* __restrict__ x, long long n, double* __restrict__ partial) {
+  __shared__ double red[8];
+  const long long groups = (n + 3) >> 2, full = n >> 2;
+  const long long stride = 256LL * gridDim.x;
+  const bool vec = (reinterpret_cast<uintptr_t>(x) & 15) == 0;
+  double acc = 0.0;
+  for (long long j = blockIdx.x * 256LL + threadIdx.x; j < groups; j += stride) {
+    float4 q;
+    if (vec && j < full) {
+      q = __ldg(reinterpret_cast<const float4*>(x) + j);
+    } else {
+      const long long e = 4 * j;
+      q.x = x[e];
+      q.y = e + 1 < n ? x[e + 1] : 0.f;
+      q.z = e + 2 < n ? x[e + 2] : 0.f;
+      q.w = e + 3 < n ? x[e + 3] : 0.f;
+    }
+    acc += static_cast<double>(fmaf(q.w, q.w, fmaf(q.z, q.z, fmaf(q.y, q.y, q.x * q.x))));
+  }
+  const double s = block_sum_d(acc, red);
+  if (threadIdx.x == 0) partial[blockIdx.x] = s;
+  if (blockIdx.x == 0)
+    for (int i = gridDim.x + threadIdx.x; i < kNormSlot; i += 256) partial[i] = 0.0;
+}
+
+// One block: norm = sqrt(sum of every partial of `nslots` slots) * grad_scale, then torch's coefficient and the
+// skip decision; the step counter advances only for a step that will be applied.
+__global__ void __launch_bounds__(256)
+grad_norm_finalize_kernel(const double* __restrict__ partial, int nslots, float max_norm, float grad_scale,
+                          float* __restrict__ norm_out, float* __restrict__ coef_out, int* __restrict__ skip_out,
+                          int* __restrict__ dev_step, int* __restrict__ skipped) {
+  __shared__ double red[8];
+  double acc = 0.0;
+  const int total = nslots * kNormSlot;
+  for (int i = threadIdx.x; i < total; i += 256) acc += partial[i];
+  const double s = block_sum_d(acc, red);
+  if (threadIdx.x != 0) return;
+  const float norm = static_cast<float>(sqrt(s) * static_cast<double>(grad_scale));
+  const bool finite = isfinite(norm);
+  *norm_out = norm;
+  *coef_out = fminf(max_norm / (norm + 1e-6f), 1.f);    // clip_grad_norm_: clamp(max_norm / (total + 1e-6), max=1)
+  *skip_out = finite ? 0 : 1;
+  if (finite) {
+    if (dev_step) *dev_step += 1;
+  } else if (skipped) {
+    *skipped += 1;
+  }
+}
+
 int blocks_for(long long n, int per = 256) {
   long long b = (n + per - 1) / per;
   if (b > 148 * 16) b = 148 * 16;
@@ -942,8 +1032,44 @@ extern "C" int hg_adamw_step(float* p, const float* g, float* m, float* v, long 
   if (step < 1) step = 1;
   const float bc1 = 1.f - powf(beta1, static_cast<float>(step));
   const float bc2 = 1.f - powf(beta2, static_cast<float>(step));
-  adamw_kernel<<<blocks_for(n, 1024), 256, 0, S(stream)>>>(p, g, m, v, n, lr, beta1, beta2, eps, weight_decay, bc1,
-                                                           sqrtf(bc2), grad_scale, dev_step, dev_lr);
+  adamw_kernel<false><<<blocks_for(n, 1024), 256, 0, S(stream)>>>(p, g, m, v, n, lr, beta1, beta2, eps, weight_decay,
+                                                                  bc1, sqrtf(bc2), grad_scale, dev_step, dev_lr,
+                                                                  nullptr, nullptr);
+  HG_CHECK_CUDA(cudaGetLastError());
+  count();
+  return HG_OK;
+}
+
+extern "C" int hg_adamw_step_guarded(float* p, const float* g, float* m, float* v, long long n, float lr, float beta1,
+                                     float beta2, float eps, float weight_decay, const int* dev_step,
+                                     const float* dev_lr, float grad_scale, const float* clip_coef, const int* skip,
+                                     void* stream) {
+  HG_REQUIRE(p && g && m && v && n > 0 && dev_step && clip_coef && skip, "hg_adamw_step_guarded: bad arguments");
+  adamw_kernel<true><<<blocks_for(n, 1024), 256, 0, S(stream)>>>(p, g, m, v, n, lr, beta1, beta2, eps, weight_decay,
+                                                                 1.f, 1.f, grad_scale, dev_step, dev_lr, clip_coef,
+                                                                 skip);
+  HG_CHECK_CUDA(cudaGetLastError());
+  count();
+  return HG_OK;
+}
+
+extern "C" int hg_grad_norm_slot_size(void) { return kNormSlot; }
+
+extern "C" int hg_grad_sumsq(const float* x, long long n, double* partials, void* stream) {
+  HG_REQUIRE(x && partials && n > 0 && (reinterpret_cast<uintptr_t>(x) & 3) == 0, "hg_grad_sumsq: bad arguments");
+  grad_sumsq_kernel<<<norm_blocks(n), 256, 0, S(stream)>>>(x, n, partials);
+  HG_CHECK_CUDA(cudaGetLastError());
+  count();
+  return HG_OK;
+}
+
+extern "C" int hg_grad_norm_finalize(const double* partials, int nslots, float max_norm, float grad_scale,
+                                     float* norm, float* clip_coef, int* skip, int* dev_step, int* skipped,
+                                     void* stream) {
+  HG_REQUIRE(partials && nslots > 0 && nslots <= 64 && norm && clip_coef && skip && max_norm > 0.f,
+             "hg_grad_norm_finalize: bad arguments");
+  grad_norm_finalize_kernel<<<1, 256, 0, S(stream)>>>(partials, nslots, max_norm, grad_scale, norm, clip_coef, skip,
+                                                      dev_step, skipped);
   HG_CHECK_CUDA(cudaGetLastError());
   count();
   return HG_OK;

@@ -93,6 +93,7 @@ class FlatParams:
         self.step_dev = torch.zeros(1, dtype=torch.int32, device=device)   # AdamW step counter (graph-capturable)
         self.lr_dev = torch.zeros(1, dtype=torch.float32, device=device)   # learning rate, read by the kernel
         self._lr_host = None
+        self.max_norm: Optional[float] = None          # clip_grad_norm (enable_guard); None: the unguarded update
         with torch.no_grad():
             for p, o, s in zip(ps, self.offsets, self.sizes):
                 view = self.p[o:o + s].view(p.shape)
@@ -107,12 +108,11 @@ class FlatParams:
 
     def adamw(self, lr: float, betas=(0.8, 0.99), eps: float = 1e-8, weight_decay: float = 0.01,
               grad_scale: float = 1.0) -> None:
-        """torch.optim.AdamW(lr, betas) semantics (UPSTREAM train.py: AdamW(h.learning_rate, [adam_b1, adam_b2]))."""
-        self.step_dev.add_(1)
-        _lib.check(_lib.lib().hg_adamw_step(self.p.data_ptr(), self.g.data_ptr(), self.m.data_ptr(), self.v.data_ptr(),
-                                            self.numel, lr, betas[0], betas[1], eps, weight_decay, 0,
-                                            self.step_dev.data_ptr(), self.lr_dev.data_ptr(), grad_scale, _stream()),
-                   "hg_adamw_step")
+        """torch.optim.AdamW(lr, betas) semantics (UPSTREAM train.py: AdamW(h.learning_rate, [adam_b1, adam_b2])).
+        Guarded (enable_guard): after grad_norm and finalize_norm, which advance the step counter themselves."""
+        if not self.guarded:
+            self.step_dev.add_(1)
+        self._adamw(0, self.numel, lr, betas, eps, weight_decay, grad_scale)
 
     def bump_step(self) -> None:
         """advance the device-side AdamW step counter once per optimizer step (before any adamw_slice of that step)"""
@@ -120,13 +120,59 @@ class FlatParams:
 
     def adamw_slice(self, lo: int, hi: int, lr: float, betas=(0.8, 0.99), eps: float = 1e-8,
                     weight_decay: float = 0.01, grad_scale: float = 1.0) -> None:
-        """the same update on elements [lo, hi) of the flat buffers only (after bump_step): lets independent parts of
-        a network update on their own stream lanes as soon as their gradients are complete"""
-        o = 4 * lo
-        _lib.check(_lib.lib().hg_adamw_step(self.p.data_ptr() + o, self.g.data_ptr() + o, self.m.data_ptr() + o,
-                                            self.v.data_ptr() + o, hi - lo, lr, betas[0], betas[1], eps, weight_decay,
-                                            0, self.step_dev.data_ptr(), self.lr_dev.data_ptr(), grad_scale, _stream()),
-                   "hg_adamw_step")
+        """the same update on elements [lo, hi) of the flat buffers only (after bump_step, or guarded after
+        finalize_norm): lets independent parts of a network update on their own stream lanes as soon as their
+        gradients are complete"""
+        self._adamw(lo, hi, lr, betas, eps, weight_decay, grad_scale)
+
+    def _adamw(self, lo: int, hi: int, lr: float, betas, eps: float, weight_decay: float, grad_scale: float) -> None:
+        L, o = _lib.lib(), 4 * lo
+        ptrs = (self.p.data_ptr() + o, self.g.data_ptr() + o, self.m.data_ptr() + o, self.v.data_ptr() + o, hi - lo,
+                lr, betas[0], betas[1], eps, weight_decay)
+        if self.guarded:
+            _lib.check(L.hg_adamw_step_guarded(*ptrs, self.step_dev.data_ptr(), self.lr_dev.data_ptr(), grad_scale,
+                                               self.clip_coef.data_ptr(), self.skip_flag.data_ptr(), _stream()),
+                       "hg_adamw_step_guarded")
+        else:
+            _lib.check(L.hg_adamw_step(*ptrs, 0, self.step_dev.data_ptr(), self.lr_dev.data_ptr(), grad_scale,
+                                       _stream()), "hg_adamw_step")
+
+    # ---- clip_grad_norm_ + skip of non-finite steps (the fork's manual-optimisation callback), inside the graph
+    @property
+    def guarded(self) -> bool:
+        return self.max_norm is not None
+
+    def enable_guard(self, max_norm: float, slots: int = 1) -> None:
+        """From now on every update of this network follows
+            total = clip_grad_norm_(params, max_norm);  if isfinite(total): optim.step()
+        grad_norm() fills `slots` partial sums (one per independently finished part of the buffer), finalize_norm()
+        decides, and adamw / adamw_slice read its coefficient and skip flag from device memory.  The results live in
+        static device buffers: grad_norm_dev (pre-clip norm, fp32), skipped_dev (int32, cumulative skipped steps)."""
+        max_norm = float(max_norm)
+        if not max_norm > 0.0:
+            raise ValueError(f"clip_grad_norm must be a positive number or inf, got {max_norm}")
+        dev = self.p.device
+        self.max_norm = max_norm
+        self.norm_slots = slots
+        self.norm_ws = torch.zeros(slots * _lib.lib().hg_grad_norm_slot_size(), dtype=torch.float64, device=dev)
+        self.grad_norm_dev = torch.zeros(1, dtype=torch.float32, device=dev)
+        self.clip_coef = torch.ones(1, dtype=torch.float32, device=dev)
+        self.skip_flag = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.skipped_dev = torch.zeros(1, dtype=torch.int32, device=dev)
+
+    def grad_norm(self, slot: int = 0, lo: int = 0, hi: Optional[int] = None) -> None:
+        """sum of squares of gradient elements [lo, hi) into partial-sum slot `slot` (on the current stream)"""
+        hi = self.numel if hi is None else hi
+        ws = self.norm_ws.data_ptr() + 8 * slot * _lib.lib().hg_grad_norm_slot_size()
+        _lib.check(_lib.lib().hg_grad_sumsq(self.g.data_ptr() + 4 * lo, hi - lo, ws, _stream()), "hg_grad_sumsq")
+
+    def finalize_norm(self, grad_scale: float = 1.0) -> None:
+        """after every slot is written: the norm of grad_scale * g, the clip coefficient, the skip flag; advances
+        step_dev for an applied step and skipped_dev for a skipped one"""
+        _lib.check(_lib.lib().hg_grad_norm_finalize(
+            self.norm_ws.data_ptr(), self.norm_slots, self.max_norm, grad_scale, self.grad_norm_dev.data_ptr(),
+            self.clip_coef.data_ptr(), self.skip_flag.data_ptr(), self.step_dev.data_ptr(),
+            self.skipped_dev.data_ptr(), _stream()), "hg_grad_norm_finalize")
 
     def span_of(self, module: nn.Module) -> Tuple[int, int]:
         """[lo, hi) of the flat buffers covered by `module`'s parameters (they must be contiguous in the buffer)"""
@@ -1356,7 +1402,8 @@ class DiscriminatorTrainer:
         self.acc_d.zero_()
         self.acc_g.zero_()
         self.flat.g.zero_()                 # every parameter-gradient kernel of the sub-discriminators accumulates
-        if update:
+        guard = update and self.flat.guarded
+        if update and not guard:
             self.flat.bump_step()
         grads = [dy_audio] + [torch.zeros(b, p.shape[1], dtype=torch.float32, device=self.device)
                               for p in self.pooled[1:]]
@@ -1378,6 +1425,14 @@ class DiscriminatorTrainer:
                     # done: the collectives run in issue order on NCCL's stream while the later lanes still compute
                     allreduce(self.flat, self.spans[i])
                     mark(f"d{i}_allreduce_done")
+                if guard:
+                    self.flat.grad_norm(i, *self.spans[i])     # slot = sub-discriminator: a fixed summation order
+        if guard:
+            # the norm is global over every slice: the lanes meet once every gradient is final (the barrier torch's
+            # clip_grad_norm_ over optim_d's parameters implies), then fork again for the updates
+            self.lanes.join()
+            self.flat.finalize_norm(1.0 / world)
+            self.lanes.fork()
         for i in self.order:
             sd = self.subs[i]
             with self.lanes.lane(i):
@@ -1440,6 +1495,12 @@ class TrainStep:
         if torch.distributed.is_available() and torch.distributed.is_initialized():
             self.world = torch.distributed.get_world_size(process_group)
         self.stamps = LaneStamps(device)
+        # h.clip_grad_norm (optional; null / absent = off): each network's update follows the fork's callback,
+        # total = clip_grad_norm_(params, clip_grad_norm); optim.step() only if total is finite
+        self.clip_grad_norm = getattr(h, "clip_grad_norm", None)
+        if self.clip_grad_norm is not None:
+            self.G.flat.enable_guard(self.clip_grad_norm)
+            self.D.flat.enable_guard(self.clip_grad_norm, slots=len(self.D.subs))
 
     def _allreduce(self, flat: FlatParams, span: Optional[Tuple[int, int]] = None) -> None:
         allreduce_gradients(flat, self.pg, span)
@@ -1511,10 +1572,18 @@ class TrainStep:
         self._allreduce(self.G.flat)
         self.stamps.mark("g_allreduce_done")
         if update:
+            if self.G.flat.guarded:
+                self.G.flat.grad_norm()
+                self.G.flat.finalize_norm(1.0 / self.world)
             self.G.flat.adamw(self.lr, self.betas, grad_scale=1.0 / self.world)
             self.G.invalidate()
         self.stamps.mark("end")
         out["y_g_hat"] = y_g
+        if self.clip_grad_norm is not None:
+            # static device buffers (refreshed by every step and graph replay): read them before the next step
+            for name, flat in (("g", self.G.flat), ("d", self.D.flat)):
+                out[f"grad_norm_{name}"] = flat.grad_norm_dev[0]
+                out[f"skipped_steps_{name}"] = flat.skipped_dev[0]
         self.launches_per_step = _lib.launch_count() - launches0   # library kernels issued (or captured) per step
         return out
 

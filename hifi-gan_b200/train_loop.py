@@ -41,7 +41,8 @@ from .utils import load_checkpoint, save_checkpoint, scan_checkpoint
 # ------------------------------------------------------------------------------------- optimizer state <-> torch
 def optimizer_state_dict(flat: FlatParams, params: List[torch.nn.Parameter], lr: float, betas, eps: float = 1e-8,
                          weight_decay: float = 0.01) -> dict:
-    """The flat AdamW state of `flat` as a torch.optim.AdamW state_dict over `params` (in that order)."""
+    """The flat AdamW state of `flat` as a torch.optim.AdamW state_dict over `params` (in that order).  `step` is the
+    number of updates applied: with clip_grad_norm set, a skipped non-finite step does not count, as in torch."""
     where = {id(p): i for i, p in enumerate(flat.params)}
     step = float(flat.step_dev.item())
     state = {}
@@ -134,7 +135,8 @@ def train(rank: int, a, h, local_rank: int = None) -> Dict[str, float]:
         mpd.load_state_dict(state_dict_do['mpd'])
         msd.load_state_dict(state_dict_do['msd'])
         steps, last_epoch = state_dict_do['steps'] + 1, state_dict_do['epoch']
-    ts = TrainStep(generator, mpd, msd, h, device)
+    ts = TrainStep(generator, mpd, msd, h, device)       # reads h.clip_grad_norm (optional) like every hyper-parameter
+    guarded = ts.clip_grad_norm is not None
     g_params = list(generator.parameters())
     d_params = list(msd.parameters()) + list(mpd.parameters())      # UPSTREAM: chain(msd.parameters(), mpd.parameters())
     if state_dict_do is not None:
@@ -186,6 +188,14 @@ def train(rank: int, a, h, local_rank: int = None) -> Dict[str, float]:
                     last = {"steps": steps, "loss_gen_all": out["loss_gen_all"].item(), "mel_error": mel_error}
                     print('Steps : {:d}, Gen Loss Total : {:4.3f}, Mel-Spec. Error : {:4.3f}, s/b : {:4.3f}'.format(
                         steps, last["loss_gen_all"], mel_error, time.time() - start_b))
+                    if guarded:
+                        last.update(grad_norm_g=out["grad_norm_g"].item(), grad_norm_d=out["grad_norm_d"].item(),
+                                    skipped_steps_g=int(out["skipped_steps_g"].item()),
+                                    skipped_steps_d=int(out["skipped_steps_d"].item()))
+                        skips = '' if not (last["skipped_steps_g"] or last["skipped_steps_d"]) else \
+                            ', Skipped Steps G/D : {:d}/{:d}'.format(last["skipped_steps_g"], last["skipped_steps_d"])
+                        print('Steps : {:d}, Grad Norm G : {:4.3f}, Grad Norm D : {:4.3f}{}'.format(
+                            steps, last["grad_norm_g"], last["grad_norm_d"], skips))
                 if steps % a.checkpoint_interval == 0 and steps != 0:
                     save_checkpoint("{}/g_{:08d}".format(a.checkpoint_path, steps), {'generator': generator.state_dict()})
                     save_checkpoint("{}/do_{:08d}".format(a.checkpoint_path, steps),
@@ -196,6 +206,9 @@ def train(rank: int, a, h, local_rank: int = None) -> Dict[str, float]:
                 if sw is not None and steps % a.summary_interval == 0:
                     sw.add_scalar("training/gen_loss_total", out["loss_gen_all"].item(), steps)
                     sw.add_scalar("training/mel_spec_error", out["loss_mel"].item() / 45, steps)
+                    if guarded:
+                        sw.add_scalar("training/grad_norm_g", out["grad_norm_g"].item(), steps)
+                        sw.add_scalar("training/grad_norm_d", out["grad_norm_d"].item(), steps)
                 if steps % a.validation_interval == 0 and val:
                     ts.G.invalidate()       # the module API must re-pack: the last AdamW update ran inside the graph
                     last["val_mel_error"] = validate(generator, val, h, device, val_mels)

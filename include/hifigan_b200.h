@@ -434,6 +434,28 @@ int hg_adamw_step(float* p, const float* g, float* m, float* v, long long n, flo
                   float eps, float weight_decay, int step, const int* dev_step, const float* dev_lr, float grad_scale,
                   void* stream);
 
+/* Gradient-norm clipping with the skip of a non-finite step (torch.nn.utils.clip_grad_norm_ followed by
+ * `if torch.isfinite(total): optim.step()`), without a host sync:
+ *   hg_grad_sumsq          sum of squares of x fp32 [n] (x 4-byte aligned; 16-byte loads when 16-byte aligned) as
+ *                          per-block fp64 partials into ONE slot of hg_grad_norm_slot_size() doubles at `partials`
+ *                          (the whole slot is written).  Deterministic: the block partition depends on n only, no
+ *                          floating-point atomics; several calls on different streams may fill different slots.
+ *   hg_grad_norm_finalize  one block after every slot is written: norm = sqrt(sum of slots [0, nslots)) * grad_scale
+ *                          (grad_scale = 1/world after a sum all-reduce: the norm of the averaged gradient), summed in
+ *                          fp64 in a fixed order.  Writes *norm, *clip_coef = min(1, max_norm / (norm + 1e-6)) (fp32,
+ *                          as torch; max_norm may be +inf), *skip = !isfinite(norm); then *dev_step += 1 when the norm
+ *                          is finite, else *skipped += 1 (either pointer may be NULL).
+ *   hg_adamw_step_guarded  hg_adamw_step with the step counter on the device (dev_step required, NOT advanced here),
+ *                          that writes nothing when *skip != 0 and otherwise scales the gradient by
+ *                          grad_scale * *clip_coef (the product rounded to fp32). */
+int hg_grad_norm_slot_size(void);
+int hg_grad_sumsq(const float* x, long long n, double* partials, void* stream);
+int hg_grad_norm_finalize(const double* partials, int nslots, float max_norm, float grad_scale, float* norm,
+                          float* clip_coef, int* skip, int* dev_step, int* skipped, void* stream);
+int hg_adamw_step_guarded(float* p, const float* g, float* m, float* v, long long n, float lr, float beta1,
+                          float beta2, float eps, float weight_decay, const int* dev_step, const float* dev_lr,
+                          float grad_scale, const float* clip_coef, const int* skip, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
