@@ -95,7 +95,7 @@ class _DiscEngine:
     def __init__(self, disc, device):
         from .train import FlatParams, _SubDiscTrainer
         self.flat = FlatParams(disc, device, bind=False)
-        self.sd = _SubDiscTrainer(disc, device, self.flat)
+        self.sd = _SubDiscTrainer(disc, device, self.flat, nslots=_SLOTS)
         self.next_slot = 0
         self.slot_call = [0] * _SLOTS
         self.calls = 0
@@ -104,7 +104,7 @@ class _DiscEngine:
 def _disc_run(disc, x: torch.Tensor, differentiable: bool):
     """One call of a sub-discriminator: claim the next ring slot, run the forward, export the feature maps and
     assemble the logits.  Returns (feature maps fp32 [B,C,H,p] + logits [B,1,H,p],
-    (engine, slot, call id, G, W, x2d))."""
+    (engine, slot, call id, G, the slot's weights and banks, x2d))."""
     eng = _engine(disc, x.device, lambda: _DiscEngine(disc, x.device))
     sd = eng.sd
     L = _lib.lib()
@@ -116,7 +116,7 @@ def _disc_run(disc, x: torch.Tensor, differentiable: bool):
     eng.next_slot = (slot + 1) % _SLOTS
     eng.calls += 1
     eng.slot_call[slot] = eng.calls
-    G, W = sd.forward_single(x2d, slot, dgrad=differentiable)
+    G, cs = sd.forward_single(x2d, slot, dgrad=differentiable)
     period, st = sd.period, _stream()
     outs = []
     for (h, rows, ch), act in zip(G["geo"], G["act"]):
@@ -127,19 +127,19 @@ def _disc_run(disc, x: torch.Tensor, differentiable: bool):
     h_last = G["geo"][-1][0]
     post = G["logit"].view(b, period, h_last).permute(0, 2, 1).contiguous().unsqueeze(1)     # [B,1,H,p]
     outs.append(post)
-    return tuple(outs), (eng, slot, eng.calls, G, W, x2d)
+    return tuple(outs), (eng, slot, eng.calls, G, cs, x2d)
 
 
 class _DiscFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, disc, *params):
-        outs, (ctx.eng, ctx.slot, ctx.call, ctx.G, ctx.W, ctx.x2d) = _disc_run(disc, x, True)
+        outs, (ctx.eng, ctx.slot, ctx.call, ctx.G, ctx.cs, ctx.x2d) = _disc_run(disc, x, True)
         ctx.set_materialize_grads(False)
         return outs
 
     @staticmethod
     def backward(ctx, *douts):
-        eng, G, W = ctx.eng, ctx.G, ctx.W
+        eng, G = ctx.eng, ctx.G
         sd = eng.sd
         n_par = len(eng.flat.params)
         if all(d is None for d in douts):
@@ -173,7 +173,7 @@ class _DiscFn(torch.autograd.Function):
         dy = torch.zeros(b, t, dtype=torch.float32, device=ctx.x2d.device) if ctx.needs_input_grad[0] else None
         if want_w:
             eng.flat.g.zero_()
-        sd.backward_single(G, W, ctx.slot, ctx.x2d, dlogit, pre, want_w, dy)
+        sd.backward_single(G, ctx.cs, ctx.x2d, dlogit, pre, want_w, dy)
         grads = _grads_out(eng.flat, eng.flat.params, ctx.needs_input_grad[2:]) if want_w else [None] * n_par
         return (None if dy is None else dy.view(b, 1, t), None) + tuple(grads)
 

@@ -13,6 +13,7 @@ fp32 parameter gradients, fp32 master weights and optimizer state.
 """
 from __future__ import annotations
 
+import contextlib
 import os
 from ctypes import byref, c_int
 from typing import Dict, List, Optional, Tuple
@@ -297,13 +298,7 @@ class _GenLayerGrad:
         self.db = None                                    # padded bias gradient, only when cout_p != cout
         self.dgrad_pad = (pc.taps - 1) * pc.dil - pc.pad_left
 
-    def pack(self, L) -> None:
-        if self.wd is not None:
-            pc = self.pc
-            _lib.check(L.hg_pack_dgrad_weight(pc.w.data_ptr(), pc.taps, self.rows, pc.cin_p, self.wd.data_ptr(),
-                                              _stream()), "hg_pack_dgrad_weight")
-
-    def add_jobs(self, table, finish: str = "finish") -> None:
+    def add_jobs(self, table, finish: str) -> None:
         """this layer's share of the trainer's batched launches: phase "dgrad" = the data-gradient filter bank (tap
         flip + transpose of the forward bank), phase `finish` = packed dW -> parameter gradients (unpack +
         weight_norm backward, accumulating)"""
@@ -364,22 +359,6 @@ class _GenLayerGrad:
                                      pc.taps, pc.dil, self.dgrad_pad, _p(mask), slope, 0, 0, 0.0, _p(res0), _p(res1),
                                      _p(res2), scale, _p(out), 0, 0, 1, 0, 0, bd[0], bd[1], bd[2], 0, _stream()),
                    "hg_conv1d_dgrad")
-
-    def to_param_grads(self, L) -> None:
-        """packed dW -> (weight_g.grad, weight_v.grad) or weight.grad, one fused launch (hg_wgrad_finish_*)"""
-        pc = self.pc
-        m = pc.module
-        g, v = _g_v(m)
-        gp, dgp = (0, 0) if g is None else (g.data_ptr(), self.flat.grad(g).data_ptr())
-        dvp = self.flat.grad(v).data_ptr()
-        if pc.kind == "conv":
-            _lib.check(L.hg_wgrad_finish_conv(self.dwp.data_ptr(), pc.cout, pc.cin, pc.taps, self.rows, pc.cin_p,
-                                              pc.cout, 1, None, v.data_ptr(), gp, 1, dvp, dgp,
-                                              _stream()), "hg_wgrad_finish_conv")
-        else:
-            _lib.check(L.hg_wgrad_finish_convtr(self.dwp.data_ptr(), pc.cin, pc.cout, m.kernel_size[0], pc.stride,
-                                                m.padding[0], pc.cin_p, pc.cout_p, v.data_ptr(), gp, 1,
-                                                dvp, dgp, _stream()), "hg_wgrad_finish_convtr")
 
 
 def _route_weight_grad(L, flat: FlatParams, m: nn.Module, dw: torch.Tensor, d0: int, rest: int,
@@ -732,17 +711,77 @@ class _DiscBwdLayer:
                    "hg_conv1d_dgrad")
 
 
+class _DiscSlot:
+    """The weights one sub-discriminator call runs with and everything its backward reads: the effective fp32 weight
+    of every layer (`w0` / `wp`: the first / last one as the [cout][k] matrices the edge kernels take), the forward
+    banks, the spectral-norm (u, v, sigma, workspace) of every layer's power iteration, the data-gradient banks, and
+    the job table that fills them (batched.py): phase "fwd" = weight_norm fold -> effective weight + forward bank of
+    every layer (spectral-norm layers: forward bank from the effective weight their power iteration produced),
+    "dgrad" = the polyphase data-gradient banks; `untiled` lists the wide layers whose bank does not tile and is
+    packed per layer.  One launch per phase instead of one per layer."""
+
+    def __init__(self, sd: "_SubDiscTrainer"):
+        from . import batched
+        dev, nl = sd.device, len(sd.mids)
+        f32 = lambda *shape: torch.empty(*shape, dtype=torch.float32, device=dev)
+        self.eff, self.fwd, self.sn = [], [], []
+        for li, m in enumerate(sd.mods):
+            v = m.weight_orig if sd.spectral else _g_v(m)[1]
+            self.eff.append(f32(v.shape[0], v.shape[1], v.shape[2] if v.dim() > 2 else 1))
+            layer = sd.mids[li - 1] if 1 <= li <= nl else None
+            self.fwd.append(None if layer is None else
+                            torch.empty(layer.k, layer.cout, layer.cin_tile, dtype=torch.bfloat16, device=dev))
+            if sd.spectral:                       # u, v, sigma of this call; workspace
+                rows, cols = v.shape[0], v.numel() // v.shape[0]
+                self.sn.append((f32(rows), f32(cols), f32(1), f32(rows + cols + 4)))
+        self.bwd = [_DiscBwdLayer(l, dev) for l in sd.mids]
+        k0, _, _, c0 = sd.first
+        self.w0 = self.eff[0].view(c0, k0)
+        self.wp = self.eff[-1].view(-1, sd.kpost)
+        self.untiled: List[int] = []
+        t = self.table = batched.JobTable(dev)
+        for li, m in enumerate(sd.mods):
+            layer = sd.mids[li - 1] if 1 <= li <= nl else None
+            if sd.spectral and layer is None:
+                continue                          # first / last conv of the spectral-norm scale: eff is all they need
+            g, v = (None, self.eff[li]) if sd.spectral else _g_v(m)
+            cout = v.shape[0]
+            cin_g, k = (layer.cin // layer.groups, layer.k) if layer is not None else (v.shape[1], v.numel() // (v.shape[0] * v.shape[1]))
+            ints = (cout, cin_g, k, layer.merge if layer else 1, (layer.cout // layer.groups) if layer else cout,
+                    layer.cin_tile if layer else cin_g)
+            t.add("fwd", batched.DISC_ROW, cout, cin_g * k * 4 if layer is not None else 0, v, g,
+                  dst0=None if sd.spectral else self.eff[li], dst1=self.fwd[li], ints=ints,
+                  tab=layer.order if layer is not None else ())
+            if layer is None:
+                continue
+            bl = self.bwd[li - 1]
+            cout_tile = (layer.cout // layer.groups) * layer.merge
+            tci = 32 if layer.k <= 10 else 8
+            while tci > 2 and (cin_g % tci or layer.cin % tci):
+                tci >>= 1
+            smem = 32 * (tci * layer.k + 1) * 4
+            if cin_g % tci == 0 and layer.cin % tci == 0 and cout_tile % 32 == 0 and smem <= 48 * 1024:
+                t.add("dgrad", batched.DISC_DGRAD_TILE, (layer.cin // tci) * (cout_tile // 32), smem, self.eff[li],
+                      dst0=bl.w, ints=(layer.cout, cin_g, layer.k, layer.merge, layer.cout // layer.groups, layer.cin,
+                                       layer.stride, layer.pad, bl.nshift, bl.smin, cout_tile, tci, layer.cin // tci))
+            else:
+                self.untiled.append(li - 1)
+        t.finalize()
+
+
 class _SubDiscTrainer:
     """One DiscriminatorP / DiscriminatorS: batched (real ++ generated) forward with saved activations, losses on
     the internal layout, and the hand-written backward."""
 
     W_CHAINS = 4
 
-    def __init__(self, disc: nn.Module, device, flat: FlatParams, boost: int = 0):
+    def __init__(self, disc: nn.Module, device, flat: FlatParams, boost: int = 0, nslots: Optional[int] = None):
         """flat: the FlatParams whose gradient buffer receives this sub-discriminator's parameter gradients.
         boost: added to the CUDA stream priorities of every lane of this sub-discriminator (negative = more urgent):
         the sub-discriminator with the longest chain (the spectral-norm scale) is the step's critical path, so its
-        kernels — its weight-gradient lane included — are placed ahead of the other sub-discriminators'."""
+        kernels — its weight-gradient lane included — are placed ahead of the other sub-discriminators'.
+        nslots: call slots (_DiscSlot) to create; default: what the training step uses (one, or one per half of
+        the spectral-norm scale)."""
         self.disc, self.device, self.flat = disc, device, flat
         self.period = getattr(disc, "period", 1)
         convs = list(disc.convs)
@@ -752,16 +791,17 @@ class _SubDiscTrainer:
         groups = lambda m: getattr(m, "groups", 1)
         self.mids = [_DiscLayer(m.in_channels, m.out_channels, m.kernel_size[0], m.stride[0], m.padding[0], groups(m))
                      for m in convs[1:]]
-        self.bwd = [_DiscBwdLayer(l, device) for l in self.mids]
         self.kpost = disc.conv_post.kernel_size[0]
+        # DiscriminatorS / P apply one norm to every conv: all spectral-norm or all weight_norm
         self.spectral = hasattr(m0, "weight_orig")
-        # the spectral-norm scale runs its real / generated halves as two parts with their own sigma (and their own
-        # data-gradient filter banks), on two lanes; lane 0 is the parameter-gradient lane of this sub-discriminator
-        self.bwd_parts = [self.bwd] + ([[_DiscBwdLayer(l, device) for l in self.mids]] if self.spectral else [])
+        # the spectral-norm scale runs its real / generated halves as two parts with their own call slot (their own
+        # sigma and data-gradient filter banks), on two lanes; lane 0 is the parameter-gradient lane of this
+        # sub-discriminator
+        self.slots = [_DiscSlot(self) for _ in range(nslots or (2 if self.spectral else 1))]
         self.lanes = _Lanes(2, device, [0 + boost, -1 + boost])   # 0: parameter-gradient lane, 1: second data-gradient chain
         n_prep = 8 if self.spectral else 4                        # spectral norm: one power-iteration chain per layer
         self.prep = _Lanes(n_prep, device, [-1 + boost] * n_prep)  # weight preparation / data-gradient packs
-        self._prefetched = None
+        self._prefetched = False
         # spectral norm: every layer's parameter-gradient chain (wgrad -> unpack -> <dw,w> -> apply, for both halves)
         # is independent of the other layers': spread over W_CHAINS lanes instead of one.  (One lane made this the
         # longest dependent chain of the whole step: 3.9 ms for 2 x 8 layers, profiles/r02_summary.md section 2.)
@@ -779,16 +819,14 @@ class _SubDiscTrainer:
         for n in sizes:
             self.dwps.append(self.dwp_flat[off:off + n])
             off += n
-        self._tables = {}
         self.db = torch.zeros(1024, dtype=torch.float32, device=device)
         self.db_unused = torch.zeros(1024, dtype=torch.float32, device=device)    # the first conv's discarded bias column
-        self.wbufs = {}
-        self.fwd_valid = self.dgrad_valid = False
-        self.W_cached = None
+        # weight_norm: slot 0's weights and banks match the parameters (forward(); the spectral norm never caches)
+        self.cached = False
 
     def invalidate(self) -> None:
         """the parameters changed (optimizer update / load_state_dict): re-fold and re-pack on next use"""
-        self.fwd_valid = self.dgrad_valid = False
+        self.cached = False
 
     # ---- weights -------------------------------------------------------------------------------------------
     def _scratch_of(self, chain: int) -> torch.Tensor:
@@ -802,78 +840,32 @@ class _SubDiscTrainer:
             buf = self._scr[chain] = torch.empty(w.numel(), dtype=torch.float32, device=self.device)
         return buf
 
-    def _weights(self, part: int):
-        """per-part persistent buffers of every layer's effective fp32 weight and forward GEMM pack; _weights_layer
-        and the table's "fwd" launch fill them"""
-        bufs = self.wbufs.get(part)
-        if bufs is None:
-            bufs = {"eff": [], "fwd": []}
-            for li, m in enumerate(self.mods):
-                _, v = _g_v(m) if not hasattr(m, "weight_orig") else (None, m.weight_orig)
-                bufs["eff"].append(torch.empty(v.shape[0], v.shape[1], v.shape[2] if v.dim() > 2 else 1,
-                                               dtype=torch.float32, device=self.device))
-                if 1 <= li <= len(self.mids):
-                    layer = self.mids[li - 1]
-                    bufs["fwd"].append(torch.empty(layer.k, layer.cout, layer.cin_tile, dtype=torch.bfloat16,
-                                                   device=self.device))
-                else:
-                    bufs["fwd"].append(None)
-            self.wbufs[part] = bufs
-        return {"eff": bufs["eff"], "fwd": bufs["fwd"], "sn": [None] * len(self.mods)}
-
-    def _table(self, part: int):
-        """Job table of part / call slot `part` (batched.py): phase "fwd" = weight_norm fold -> effective fp32 weight +
-        forward bank of every layer (spectral-norm layers: forward bank from the effective weight their power
-        iteration produced), "dgrad" = the polyphase data-gradient banks.  One launch each instead of one per layer."""
-        t = self._tables.get(part)
-        if t is not None:
-            return t
-        from . import batched
+    def _power_iterate(self, slots: List[_DiscSlot], lanes: bool) -> None:
+        """Spectral norm: one power iteration per layer and slot (in train mode, like the reference's hook), u / v
+        updated in place (hg_spectral_norm_fwd), into each slot's effective weight; the slot keeps this call's u, v,
+        sigma for its backward.  Per layer the slots run in list order: a second call continues from the first's
+        u, v.  lanes: layer li on prep lane li, forked from the current stream and not joined back; otherwise
+        everything on the current stream."""
         L = _lib.lib()
-        bufs = self.wbufs[part]
-        t = batched.JobTable(self.device)
-        nl = len(self.mids)
-        self.untiled = []                         # layers whose data-gradient bank does not tile: packed per layer
+        if lanes:
+            self.prep.fork()
         for li, m in enumerate(self.mods):
-            layer = self.mids[li - 1] if 1 <= li <= nl else None
-            sn = hasattr(m, "weight_orig")
-            if sn and layer is None:
-                continue                          # first / last conv of the spectral-norm scale: eff is all they need
-            g, v = (None, bufs["eff"][li]) if sn else _g_v(m)
-            cout = v.shape[0]
-            cin_g, k = (layer.cin // layer.groups, layer.k) if layer is not None else (v.shape[1], v.numel() // (v.shape[0] * v.shape[1]))
-            ints = (cout, cin_g, k, layer.merge if layer else 1, (layer.cout // layer.groups) if layer else cout,
-                    layer.cin_tile if layer else cin_g)
-            t.add("fwd", batched.DISC_ROW, cout, cin_g * k * 4 if layer is not None else 0, v, g,
-                  dst0=None if sn else bufs["eff"][li], dst1=bufs["fwd"][li] if layer is not None else None,
-                  ints=ints, tab=layer.order if layer is not None else ())
-            if layer is None:
-                continue
-            bl = self._bwd_bank(part)[li - 1]
-            cout_tile = (layer.cout // layer.groups) * layer.merge
-            tci = 32 if layer.k <= 10 else 8
-            while tci > 2 and (cin_g % tci or layer.cin % tci):
-                tci >>= 1
-            smem = 32 * (tci * layer.k + 1) * 4
-            if cin_g % tci == 0 and layer.cin % tci == 0 and cout_tile % 32 == 0 and smem <= 48 * 1024:
-                t.add("dgrad", batched.DISC_DGRAD_TILE, (layer.cin // tci) * (cout_tile // 32), smem, bufs["eff"][li],
-                      dst0=bl.w, ints=(layer.cout, cin_g, layer.k, layer.merge, layer.cout // layer.groups, layer.cin,
-                                       layer.stride, layer.pad, bl.nshift, bl.smin, cout_tile, tci, layer.cin // tci))
-            else:
-                self.untiled.append(li - 1)
-        self._tables[part] = t.finalize()
-        return t
+            wo = m.weight_orig
+            rows, cols = wo.shape[0], wo.numel() // wo.shape[0]
+            with self.prep.lane(li) if lanes else contextlib.nullcontext():
+                for s in slots:
+                    u, v, sigma, ws = s.sn[li]
+                    _lib.check(L.hg_spectral_norm_fwd(wo.data_ptr(), m.weight_u.data_ptr(), m.weight_v.data_ptr(),
+                                                      rows, cols, 1 if m.training else 0, s.eff[li].data_ptr(),
+                                                      sigma.data_ptr(), u.data_ptr(), v.data_ptr(), ws.data_ptr(),
+                                                      _stream()), "hg_spectral_norm_fwd")
 
-    def _prepare_weights(self, part: int) -> dict:
-        """effective weights + forward banks of part `part` on the current stream: spectral-norm layers run their
-        power iteration (one per call in train mode, like the reference's hook), then ONE batched launch folds /
-        packs every layer"""
-        W = self._weights(part)
-        if self.spectral:
-            for li in range(len(self.mods)):
-                self._weights_layer(W, self.wbufs[part], li)
-        self._table(part).launch("fwd")
-        return W
+    def _pack_dgrad(self, slot: _DiscSlot) -> None:
+        """the data-gradient banks of the slot's effective weights, on the current stream"""
+        if slot.table.has("dgrad"):
+            slot.table.launch("dgrad")
+        for i in slot.untiled:
+            slot.bwd[i].pack(slot.eff[1 + i])
 
     def prefetch_weights(self) -> None:
         """Spectral norm only: queue the NEXT forward's power iterations (both halves) and forward banks on the prep
@@ -883,45 +875,14 @@ class _SubDiscTrainer:
         lanes' persistent tensor-core kernels (measured: 0.98 -> 3.0 ms for chains that take 0.2 ms on a quiet GPU)."""
         if not self.spectral:
             return
-        Ws = [self._weights(pi) for pi in range(2)]
-        self.prep.fork()
-        for li in range(len(self.mods)):
-            with self.prep.lane(li):
-                for pi, W in enumerate(Ws):
-                    self._weights_layer(W, self.wbufs[pi], li)
+        self._power_iterate(self.slots[:2], lanes=True)
         p0 = self.prep.streams[0]
         for s_ in self.prep.streams[1:]:
             p0.wait_stream(s_)
         with torch.cuda.stream(p0):
-            for pi in range(2):
-                self._table(pi).launch("fwd")
-        self._prefetched = Ws
-
-    def _weights_layer(self, ws, bufs, li: int) -> None:
-        """fold (weight norm) or power-iterate (spectral norm) layer li into its effective fp32 weight"""
-        L = _lib.lib()
-        st = _stream()
-        m = self.mods[li]
-        eff = bufs["eff"][li]
-        if hasattr(m, "weight_orig"):
-            wo = m.weight_orig
-            rows, cols = wo.shape[0], wo.numel() // wo.shape[0]
-            snb = bufs.setdefault("sn", {}).get(li)
-            if snb is None:
-                f32 = lambda n: torch.empty(n, dtype=torch.float32, device=self.device)
-                snb = (f32(rows), f32(cols), f32(1), f32(rows + cols + 4))     # u, v, sigma of this call; workspace
-                bufs["sn"][li] = snb
-            # one power iteration per call in train mode, u / v buffers updated in place (hg_spectral_norm_fwd);
-            # the copies are what the backward of THIS call's weights needs (the next call moves u, v on)
-            _lib.check(L.hg_spectral_norm_fwd(wo.data_ptr(), m.weight_u.data_ptr(), m.weight_v.data_ptr(), rows,
-                                              cols, 1 if m.training else 0, eff.data_ptr(), snb[2].data_ptr(),
-                                              snb[0].data_ptr(), snb[1].data_ptr(), snb[3].data_ptr(), st),
-                       "hg_spectral_norm_fwd")
-            ws["sn"][li] = snb
-        else:
-            g, v = _g_v(m)
-            _lib.check(L.hg_fold_weight_norm(v.data_ptr(), 0 if g is None else g.data_ptr(), v.shape[0],
-                                             v.numel() // v.shape[0], eff.data_ptr(), st), "hg_fold_weight_norm")
+            for s in self.slots[:2]:
+                s.table.launch("fwd")
+        self._prefetched = True
 
     def _geometry(self, nb: int, t: int, slot: int = 0):
         key = (nb, t, slot)
@@ -963,7 +924,7 @@ class _SubDiscTrainer:
             return ps
 
         def ok(ps):
-            for li, (layer, bl) in enumerate(zip(self.mids, self.bwd)):
+            for li, (layer, bl) in enumerate(zip(self.mids, self.slots[0].bwd)):
                 h_in, p_in, h_out, p_out, s = hs[li], ps[li], hs[li + 1], ps[li + 1], layer.stride
                 if p_in - h_in < layer.pad:                                   # left padding of the next sequence
                     return False
@@ -989,78 +950,64 @@ class _SubDiscTrainer:
         L = _lib.lib()
         nb, t = ycat.shape
         G = self._geometry(nb, t)
-        period = self.period
         parts = [(0, nb)] if not self.spectral else [(0, nreal), (nreal, nb - nreal)]
-        self.parts = []
+        slots = self.slots[:len(parts)]
+        here = torch.cuda.current_stream()
         # weight_norm layers: the packs stay valid until the next optimizer update (the G-step forward of one step
         # and the D-step forward of the next see the same weights); spectral norm moves on every call, and its
-        # second part's power iteration continues from the first's.  The layers are independent of each other, so
-        # their fold / power-iteration / pack chains are spread over the prep lanes (part 0 before part 1 per layer).
-        if self.spectral and self._prefetched is not None:
+        # second part's power iteration continues from the first's.
+        stale = self.spectral or not self.cached
+        if self._prefetched:
             # prefetch_weights() queued this call's power iterations and forward banks on the prep lanes
-            Ws, self._prefetched = self._prefetched, None
-            torch.cuda.current_stream().wait_stream(self.prep.streams[0])
-            self.W_cached = Ws[-1]
-            self.fwd_valid = True
-        elif self.spectral or not self.fwd_valid:
-            if self.spectral:
-                # the power iterations of the layers are independent chains of three small kernels (part 0 before part 1
-                # per layer: the second call continues from the first's u, v): side by side on the prep lanes.  (Batched
-                # per stage over all layers, or as one cluster launch, they were slower: a many-block launch on this
-                # lane waits for whole tensor-core kernels of the other lanes to drain — profiles/r02_summary.md.)
-                Ws = [self._weights(pi) for pi in range(len(parts))]
-                self.prep.fork()
-                for li in range(len(self.mods)):
-                    with self.prep.lane(li):
-                        for pi, W in enumerate(Ws):
-                            self._weights_layer(W, self.wbufs[pi], li)
-                self.prep.join()
-                for pi in range(len(parts)):
-                    self._table(pi).launch("fwd")
-            else:
-                Ws = [self._prepare_weights(0)]
-            self.W_cached = Ws[-1]
-            self.fwd_valid = True
-        else:
-            Ws = [self.W_cached]
-        here = torch.cuda.current_stream()
+            self._prefetched = False
+            here.wait_stream(self.prep.streams[0])
+        elif self.spectral:
+            # the power iterations of the layers are independent chains of three small kernels: side by side on the
+            # prep lanes.  (Batched per stage over all layers, or as one cluster launch, they were slower: a
+            # many-block launch on this lane waits for whole tensor-core kernels of the other lanes to drain —
+            # profiles/r02_summary.md.)
+            self._power_iterate(slots, lanes=True)
+            self.prep.join()
+            for s in slots:
+                s.table.launch("fwd")
+        elif stale:
+            slots[0].table.launch("fwd")
+        self.cached = not self.spectral
         # the data-gradient filter banks of these weights: one batched launch per part, on a high-priority lane beside
         # the forward chain (on the low-priority w-lane a many-block launch starves behind the other lanes' tensor-core
         # kernels and holds the backward up); the backward waits for it before its first data-gradient launch
         plane = self.prep.streams[0]
         plane.wait_stream(here)
         with torch.cuda.stream(plane):
-            for pi in range(len(parts)):
-                self._pack_dgrad(Ws[pi], pi)
+            if stale:
+                for s in slots:
+                    self._pack_dgrad(s)
         if len(parts) > 1:
             # the second part's chain forks HERE, before the first part's launches are queued on this stream: the
             # two halves run side by side (they wrote "wait_stream(here)" after part 0 once, and ran one after the
             # other: 300 us of the step's critical path per forward — profiles/r02_summary.md section 2)
             self.lanes.streams[1].wait_stream(here)
-        for pi, (b0, bn) in enumerate(parts):
-            W = Ws[pi]
-            self.parts.append((b0, bn, W))
+        self.parts = [(b0, bn, s) for (b0, bn), s in zip(parts, slots)]
+        for pi, (b0, bn, s) in enumerate(self.parts):
             if pi == 1:
                 with torch.cuda.stream(self.lanes.streams[1]):
-                    self._forward_part(L, G, W, ycat, b0, bn, t)
+                    self._forward_part(L, G, s, ycat, b0, bn, t)
             else:
-                self._forward_part(L, G, W, ycat, b0, bn, t)
+                self._forward_part(L, G, s, ycat, b0, bn, t)
         if len(parts) > 1:
             here.wait_stream(self.lanes.streams[1])
         self.G, self.nb, self.nreal, self.t, self.ycat = G, nb, nreal, t, ycat
         return G
 
-    def _forward_part(self, L, G, W, ycat, b0: int, bn: int, t: int) -> None:
+    def _forward_part(self, L, G, slot: _DiscSlot, ycat, b0: int, bn: int, t: int) -> None:
         period = self.period
         st = _stream()
         k0, s0, p0, c0 = self.first
         seq0, nseq = b0 * period, bn * period
-        w0 = W["eff"][0].reshape(c0, k0).contiguous()
-        W["w0"] = w0
         b0_bias = self.mods[0].bias
         act = G["act"][0]
         h, rows, _ = G["geo"][0]
-        _lib.check(L.hg_disc_first_conv_fwd(ycat[b0:].data_ptr(), w0.data_ptr(), b0_bias.data_ptr(), bn, t, period,
+        _lib.check(L.hg_disc_first_conv_fwd(ycat[b0:].data_ptr(), slot.w0.data_ptr(), b0_bias.data_ptr(), bn, t, period,
                                             k0, s0, p0, c0, rows, act[seq0:].data_ptr(), LRELU_SLOPE, st),
                    "hg_disc_first_conv_fwd")
         for li, layer in enumerate(self.mids):
@@ -1068,17 +1015,15 @@ class _SubDiscTrainer:
             bias = m.bias
             out = G["act"][1 + li]
             h_out, rows_out, _ = G["geo"][1 + li]
-            _lib.check(L.hg_conv1d_general_fwd(act[seq0:].data_ptr(), W["fwd"][1 + li].data_ptr(), bias.data_ptr(),
+            _lib.check(L.hg_conv1d_general_fwd(act[seq0:].data_ptr(), slot.fwd[1 + li].data_ptr(), bias.data_ptr(),
                                                1, nseq * rows, layer.cin, nseq * rows_out, nseq * rows_out,
                                                layer.groups_eff, layer.cout, layer.k, layer.stride, layer.pad,
                                                out[seq0:].data_ptr(), LRELU_SLOPE, 0, rows_out, h_out, st),
                        "hg_conv1d_general_fwd")
             act, h, rows = out, h_out, rows_out
         c_last = G["geo"][-1][2]
-        wp = W["eff"][-1].reshape(c_last, self.kpost).contiguous()
-        W["wp"] = wp
         bp = self.mods[-1].bias
-        _lib.check(L.hg_disc_last_conv_fwd(act[seq0:].data_ptr(), wp.data_ptr(), bp.data_ptr(), nseq, h, rows,
+        _lib.check(L.hg_disc_last_conv_fwd(act[seq0:].data_ptr(), slot.wp.data_ptr(), bp.data_ptr(), nseq, h, rows,
                                            c_last, self.kpost, G["logit"][seq0:].data_ptr(), st),
                    "hg_disc_last_conv_fwd")
 
@@ -1135,51 +1080,33 @@ class _SubDiscTrainer:
             self.dwp_flat.zero_()
         self.lanes.fork()     # both lanes join the capture here (a join of a never-forked stream would invalidate it)
         self.wl.fork()
-        for pi, (b0, bn, W) in enumerate(self.parts):
+        for pi, (b0, bn, slot) in enumerate(self.parts):
             if pi == 1:                       # spectral norm: the generated half's chain on the second lane,
                 with torch.cuda.stream(self.lanes.streams[1]):     # beside the real half's (forked just above)
-                    self._backward_part(L, G, W, b0, bn, want_wgrad=True, fm=False, dy_audio=None, accumulate=True,
-                                        part=pi)
+                    self._backward_part(L, G, slot, b0, bn, want_wgrad=True, fm=False, dy_audio=None)
             else:
-                self._backward_part(L, G, W, b0, bn, want_wgrad=True, fm=False, dy_audio=None, accumulate=True,
-                                    part=pi)
+                self._backward_part(L, G, slot, b0, bn, want_wgrad=True, fm=False, dy_audio=None)
         self.wl.join()
         self.lanes.join()
 
-    def _bwd_bank(self, part: int):
-        """data-gradient filter banks of part / call slot `part` (created on first use)"""
-        while len(self.bwd_parts) <= part:
-            self.bwd_parts.append([_DiscBwdLayer(l, self.device) for l in self.mids])
-        return self.bwd_parts[part]
-
-    def _pack_dgrad(self, W, part: int = 0) -> None:
-        if self.spectral or not self.dgrad_valid:
-            t = self._table(part)
-            if t.has("dgrad"):
-                t.launch("dgrad")
-            for i in self.untiled:
-                self._bwd_bank(part)[i].pack(W["eff"][1 + i])
-            self.dgrad_valid = True
-
     # ---- one module call under torch autograd (autograd.py): forward with its own activation / weight slot ---------
     def forward_single(self, x2d: torch.Tensor, slot: int, dgrad: bool = True):
-        """x2d fp32 [B, T] -> (G, W) of call slot `slot`: activations, logits, the weights this call used (a train-mode
-        spectral-norm layer advances its power iteration per call, like the reference's hook) and, with `dgrad`
-        (the call can be differentiated), their data-gradient banks.  Everything on the current stream."""
+        """x2d fp32 [B, T] -> (G, call slot) of ring slot `slot`: activations, logits, the weights this call used (a
+        train-mode spectral-norm layer advances its power iteration per call, like the reference's hook) and, with
+        `dgrad` (the call can be differentiated), their data-gradient banks.  Everything on the current stream."""
         L = _lib.lib()
         nb, t = x2d.shape
         G = self._geometry(nb, t, slot)
-        W = self._prepare_weights(slot)
+        s = self.slots[slot]
+        if self.spectral:
+            self._power_iterate([s], lanes=False)
+        s.table.launch("fwd")
         if dgrad:
-            tb = self._table(slot)
-            if tb.has("dgrad"):
-                tb.launch("dgrad")
-            for i in self.untiled:
-                self._bwd_bank(slot)[i].pack(W["eff"][1 + i])
-        self._forward_part(L, G, W, x2d, 0, nb, t)
-        return G, W
+            self._pack_dgrad(s)
+        self._forward_part(L, G, s, x2d, 0, nb, t)
+        return G, s
 
-    def backward_single(self, G, W, slot: int, x2d: torch.Tensor, dlogit: torch.Tensor, pre_adds, want_wgrad: bool,
+    def backward_single(self, G, slot: _DiscSlot, x2d: torch.Tensor, dlogit: torch.Tensor, pre_adds, want_wgrad: bool,
                         dy_audio) -> None:
         """Backward of forward_single's call: dlogit fp32 [B*period][h] (internal order), pre_adds[l] bf16 gradient at
         feature map l in the internal layout (or None) -> parameter gradients ADDED into self.flat (want_wgrad)
@@ -1192,8 +1119,7 @@ class _SubDiscTrainer:
             self.dwp_flat.zero_()
         self.lanes.fork()
         self.wl.fork()
-        self._backward_part(L, G, W, 0, nb, want_wgrad=want_wgrad, fm=False, dy_audio=dy_audio, accumulate=True,
-                            part=slot, pre_adds=pre_adds)
+        self._backward_part(L, G, slot, 0, nb, want_wgrad=want_wgrad, fm=False, dy_audio=dy_audio, pre_adds=pre_adds)
         self.wl.join()
         self.lanes.join()
 
@@ -1209,14 +1135,13 @@ class _SubDiscTrainer:
         # d/dlg of mean((1 - lg)^2) + 2 * mean|lr - lg|
         _lib.check(L.hg_loss_grad(lg.data_ptr(), lr.data_ptr(), ng * h, 2, 1.0, 2.0 / (ng * h), nfm[-1], 0,
                                   G["dlogit"][nr:].data_ptr(), st))
-        b0, bn, W = self.parts[-1] if self.spectral else (self.nreal, self.nb - self.nreal, self.parts[0][2])
-        part = len(self.parts) - 1
+        slot = self.parts[-1][2]          # the generated half's weights
         torch.cuda.current_stream().wait_stream(self.prep.streams[0])     # data-gradient packs (see forward)
-        self._backward_part(L, G, W, self.nreal, self.nb - self.nreal, want_wgrad=False, fm=True,
-                            dy_audio=dy_audio, accumulate=False, nfm=nfm, part=part)
+        self._backward_part(L, G, slot, self.nreal, self.nb - self.nreal, want_wgrad=False, fm=True,
+                            dy_audio=dy_audio, nfm=nfm)
 
-    def _backward_part(self, L, G, W, b0: int, bn: int, want_wgrad: bool, fm: bool, dy_audio, accumulate: bool,
-                       nfm: Optional[List[float]] = None, part: int = 0, pre_adds=None) -> None:
+    def _backward_part(self, L, G, slot: _DiscSlot, b0: int, bn: int, want_wgrad: bool, fm: bool, dy_audio,
+                       nfm: Optional[List[float]] = None, pre_adds=None) -> None:
         """The data-gradient chain runs on the current stream; all parameter-gradient work (bias sums, wgrad,
         finish) goes to this sub-discriminator's w-lane, which also serialises the use of the shared scratch."""
         period = self.period
@@ -1224,7 +1149,7 @@ class _SubDiscTrainer:
         nr = self.nreal * period
         geo = G["geo"]
         nl = len(self.mids)
-        bwd = self._bwd_bank(part)
+        bwd = slot.bwd
         pre = pre_adds if pre_adds is not None else [None] * (nl + 1)   # incoming feature-map gradients (autograd path)
         h_last, rows_last, c_last = geo[-1]
         act_last = G["act"][-1]
@@ -1245,7 +1170,7 @@ class _SubDiscTrainer:
         # every data-gradient launch of the discriminator step also sums the bias gradient of the layer whose output
         # it differentiates, in fp32, straight into the flat gradient buffer (zeroed in run_phases)
         bias_of = (lambda li: self.flat.grad(self.mods[li].bias).data_ptr()) if want_wgrad else (lambda li: 0)
-        _lib.check(L.hg_disc_last_conv_bwd(act_last[seq0:].data_ptr(), W["wp"].data_ptr(), G["dlogit"][seq0:].data_ptr(),
+        _lib.check(L.hg_disc_last_conv_bwd(act_last[seq0:].data_ptr(), slot.wp.data_ptr(), G["dlogit"][seq0:].data_ptr(),
                                            nseq, h_last, rows_last, c_last, self.kpost, LRELU_SLOPE, fm_r_last,
                                            nfm[nl] if fm else 0.0, _p(pre[nl]), G["grad"][-1][seq0:].data_ptr(), 0, 0,
                                            bias_of(nl), _stream()), "hg_disc_last_conv_bwd")
@@ -1253,12 +1178,12 @@ class _SubDiscTrainer:
             def post_grads(scratch):
                 scratch[: c_last * self.kpost].zero_()
                 self.db.zero_()
-                _lib.check(L.hg_disc_last_conv_bwd(act_last[seq0:].data_ptr(), W["wp"].data_ptr(),
+                _lib.check(L.hg_disc_last_conv_bwd(act_last[seq0:].data_ptr(), slot.wp.data_ptr(),
                                                    G["dlogit"][seq0:].data_ptr(), nseq, h_last, rows_last, c_last,
                                                    self.kpost, LRELU_SLOPE, 0, 0.0, 0, 0, scratch.data_ptr(),
                                                    self.db.data_ptr(), 0, _stream()), "hg_disc_last_conv_bwd")
-                self._route(L, post, scratch, 1, c_last * self.kpost, W, len(self.mods) - 1, True)
-                self._bias(post, self.db[:1], True)
+                self._route(L, post, scratch, 1, c_last * self.kpost, slot, len(self.mods) - 1)
+                self.flat.grad(post.bias).add_(self.db[:1])
             side(post_grads, 0)
         for li in reversed(range(nl)):
             layer = self.mids[li]
@@ -1286,7 +1211,7 @@ class _SubDiscTrainer:
                                                           layer.cout, layer.cin_tile, layer.cout // layer.groups,
                                                           layer.merge, order, scratch.data_ptr(), st),
                                    "hg_unpack_wgrad_conv")
-                        self._route(L, m, scratch, layer.cout, cin_g * layer.k, W, 1 + li, True)
+                        self._route(L, m, scratch, layer.cout, cin_g * layer.k, slot, 1 + li)
                     else:
                         g, v = _g_v(m)          # unpack + weight_norm backward in one launch, accumulating
                         _lib.check(L.hg_wgrad_finish_conv(self.dwps[li].data_ptr(), layer.cout, cin_g, layer.k,
@@ -1306,33 +1231,27 @@ class _SubDiscTrainer:
                 scratch[: c0 * k0].zero_()
                 # the kernel's own bias column (summed from the bf16 gradient) lands in the db scratch and is not
                 # used: the first conv's bias gradient came from the fp32 sums of the launch that produced grad[0]
-                _lib.check(L.hg_disc_first_conv_bwd(self.ycat[b0:].data_ptr(), W["w0"].data_ptr(),
+                _lib.check(L.hg_disc_first_conv_bwd(self.ycat[b0:].data_ptr(), slot.w0.data_ptr(),
                                                     G["grad"][0][seq0:].data_ptr(), bn, self.t, period, k0, s0, p0, c0,
                                                     geo[0][1], scratch.data_ptr(), self.db_unused.data_ptr(), 0,
                                                     _stream()), "hg_disc_first_conv_bwd")
-                self._route(L, m0, scratch, c0, k0, W, 0, True)
+                self._route(L, m0, scratch, c0, k0, slot, 0)
             side(first_grads, nl + 1)
         if dy_audio is not None:
-            _lib.check(L.hg_disc_first_conv_bwd(self.ycat[b0:].data_ptr(), W["w0"].data_ptr(),
+            _lib.check(L.hg_disc_first_conv_bwd(self.ycat[b0:].data_ptr(), slot.w0.data_ptr(),
                                                 G["grad"][0][seq0:].data_ptr(), bn, self.t, period, k0, s0, p0, c0,
                                                 geo[0][1], 0, 0, _p(dy_audio), _stream()), "hg_disc_first_conv_bwd")
 
-    def _bias(self, m: nn.Module, db: torch.Tensor, accumulate: bool) -> None:
-        if accumulate:
-            self.flat.grad(m.bias).add_(db)
-        else:
-            self.flat.grad(m.bias).copy_(db)
-
-    def _route(self, L, m: nn.Module, dw: torch.Tensor, d0: int, rest: int, W, li: int, accumulate: bool) -> None:
+    def _route(self, L, m: nn.Module, dw: torch.Tensor, d0: int, rest: int, slot: _DiscSlot, li: int) -> None:
+        """dw fp32 (the layer's weight gradient, parameter layout) -> += its parameter gradients"""
         if hasattr(m, "weight_orig"):
             # spectral norm: w = W / sigma with sigma = u^T W v (u, v constants): dW = (dw - <dw, w> u v^T) / sigma
-            u, v, sigma, snws = W["sn"][li]
-            _lib.check(L.hg_spectral_norm_bwd(dw.data_ptr(), W["eff"][li].data_ptr(), u.data_ptr(), v.data_ptr(),
-                                              sigma.data_ptr(), d0, rest, 1 if accumulate else 0,
-                                              self.flat.grad(m.weight_orig).data_ptr(), snws.data_ptr(), _stream()),
-                       "hg_spectral_norm_bwd")
+            u, v, sigma, snws = slot.sn[li]
+            _lib.check(L.hg_spectral_norm_bwd(dw.data_ptr(), slot.eff[li].data_ptr(), u.data_ptr(), v.data_ptr(),
+                                              sigma.data_ptr(), d0, rest, 1, self.flat.grad(m.weight_orig).data_ptr(),
+                                              snws.data_ptr(), _stream()), "hg_spectral_norm_bwd")
         else:
-            _route_weight_grad(L, self.flat, m, dw, d0, rest, accumulate)
+            _route_weight_grad(L, self.flat, m, dw, d0, rest, accumulate=True)
 
 
 class DiscriminatorTrainer:
