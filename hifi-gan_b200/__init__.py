@@ -2,7 +2,7 @@
 from . import _lib  # noqa: F401
 from .configs import load_config  # noqa: F401
 from .env import AttrDict, build_env  # noqa: F401
-from .meldataset import MAX_WAV_VALUE, MelDataset, SegmentSampler, mel_spectrogram  # noqa: F401
+from .meldataset import MAX_WAV_VALUE, CorpusSampler, MelDataset, SegmentSampler, mel_spectrogram  # noqa: F401
 from .models import (LRELU_SLOPE, DiscriminatorP, DiscriminatorS, Generator,  # noqa: F401
                      MultiPeriodDiscriminator, MultiScaleDiscriminator, ResBlock1, ResBlock2,
                      discriminator_loss, feature_loss, generator_loss)

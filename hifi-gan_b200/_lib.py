@@ -140,6 +140,8 @@ _SIGNATURES = {
     "hg_float_to_int16": (c_int, [c_void_p, ctypes.c_longlong, c_float, c_void_p, c_void_p]),
     "hg_loss_sum": (c_int, [c_void_p, c_void_p, ctypes.c_longlong, c_int, c_float, c_void_p, c_void_p]),
     "hg_segment_gather": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
+    "hg_segment_stage_i16": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "hg_segment_stage_mel": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
     "hg_ncl_to_nlc": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_void_p]),
     "hg_nlc_to_ncl": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
     "hg_conv_post_tanh_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),

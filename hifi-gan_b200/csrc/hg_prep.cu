@@ -248,6 +248,63 @@ __global__ void segment_gather_kernel(const float* __restrict__ pool, const long
     out[static_cast<size_t>(b) * seg + i] = i < nv ? pool[s0 + i] : 0.f;
 }
 
+// One int16 sample -> the fp32 value the host pipeline gives it: q / 32768 (read_wav) / 32768 (MAX_WAV_VALUE, both
+// divisions exact), then the utterance's normalisation.  peak: (q / m) * 0.95f with m = max|q| over the utterance;
+// the two 2^-15 scales cancel exactly in the IEEE quotient.
+__device__ __forceinline__ float stage_sample(int q, int m, int mode) {
+  if (mode == HG_STAGE_PEAK) return m > 0 ? __fmul_rn(__fdiv_rn(static_cast<float>(q), static_cast<float>(m)), 0.95f) : 0.f;
+  if (mode == HG_STAGE_FORK) return q > 0 ? 0.95f : (q < 0 ? -0.95f : 0.f);
+  return __fmul_rn(static_cast<float>(q), 0x1p-30f);
+}
+
+// out[b][i] = i < valid[b] ? stage_sample(staged[b][i], peak[b]) : 0; kVec: 8 samples per thread in 16-byte accesses
+template <bool kVec>
+__global__ void __launch_bounds__(256)
+segment_stage_i16_kernel(const int16_t* __restrict__ staged, const int* __restrict__ peak,
+                         const int* __restrict__ valid, int seg, int mode, float* __restrict__ out) {
+  const int b = blockIdx.y;
+  const int i0 = (blockIdx.x * 256 + threadIdx.x) * 8;
+  if (i0 >= seg) return;
+  const int nv = valid[b], m = peak[b];
+  const int16_t* src = staged + static_cast<size_t>(b) * seg + i0;
+  float* dst = out + static_cast<size_t>(b) * seg + i0;
+  if (kVec) {
+    const int4 raw = *reinterpret_cast<const int4*>(src);
+    const int w[4] = {raw.x, raw.y, raw.z, raw.w};
+    float v[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const int q = static_cast<int16_t>(static_cast<uint32_t>(w[j >> 1]) >> ((j & 1) * 16));
+      v[j] = i0 + j < nv ? stage_sample(q, m, mode) : 0.f;
+    }
+    reinterpret_cast<float4*>(dst)[0] = make_float4(v[0], v[1], v[2], v[3]);
+    reinterpret_cast<float4*>(dst)[1] = make_float4(v[4], v[5], v[6], v[7]);
+  } else {
+    for (int j = 0; j < 8 && i0 + j < seg; ++j) dst[j] = i0 + j < nv ? stage_sample(src[j], m, mode) : 0.f;
+  }
+}
+
+// staged fp32 [B][fps][num_mels] -> out [B][num_mels][fps], frames >= valid_frames[b] zero; 32x32 smem transpose tiles
+__global__ void segment_stage_mel_kernel(const float* __restrict__ staged, const int* __restrict__ valid_frames,
+                                         int fps, int num_mels, float* __restrict__ out) {
+  __shared__ float tile[32][33];
+  const int b = blockIdx.z;
+  const int f0 = blockIdx.x * 32, m0 = blockIdx.y * 32;
+  const int tx = threadIdx.x, ty = threadIdx.y;  // 32 x 8
+  const int nv = valid_frames[b];
+  const float* src = staged + static_cast<size_t>(b) * fps * num_mels;
+  for (int i = ty; i < 32; i += 8) {
+    const int f = f0 + i, m = m0 + tx;
+    tile[i][tx] = (f < nv && f < fps && m < num_mels) ? src[static_cast<size_t>(f) * num_mels + m] : 0.f;
+  }
+  __syncthreads();
+  float* dst = out + static_cast<size_t>(b) * num_mels * fps;
+  for (int i = ty; i < 32; i += 8) {
+    const int m = m0 + i, f = f0 + tx;
+    if (m < num_mels && f < fps) dst[static_cast<size_t>(m) * fps + f] = tile[tx][i];
+  }
+}
+
 // mode 0: sum |a - b|     (feature_loss / mel L1, src/models.py:251-257)
 // mode 1: sum (c - a)^2   (LSGAN terms, src/models.py:260-282; c = 1 for "real", 0 for "generated")
 __global__ void __launch_bounds__(256)
@@ -300,6 +357,37 @@ extern "C" int hg_segment_gather(const float* pool, const long long* start, cons
              "hg_segment_gather: bad arguments");
   dim3 grid((seg + 1023) / 1024 < 64 ? (seg + 1023) / 1024 : 64, batch);
   segment_gather_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(pool, start, valid, seg, out);
+  HG_CHECK_CUDA(cudaGetLastError());
+  g_hg_launches.fetch_add(1, std::memory_order_relaxed);
+  return HG_OK;
+}
+
+extern "C" int hg_segment_stage_i16(const int16_t* staged, const int* peak, const int* valid, int batch, int seg,
+                                    int mode, float* out, void* stream) {
+  HG_REQUIRE(staged && peak && valid && out && batch > 0 && batch <= 65535 && seg > 0 &&
+             (mode == HG_STAGE_PEAK || mode == HG_STAGE_FORK || mode == HG_STAGE_NONE),
+             "hg_segment_stage_i16: bad arguments");
+  dim3 grid((seg + 256 * 8 - 1) / (256 * 8), batch);
+  const bool vec = seg % 8 == 0 && reinterpret_cast<uintptr_t>(staged) % 16 == 0 &&
+                   reinterpret_cast<uintptr_t>(out) % 16 == 0;
+  if (vec)
+    segment_stage_i16_kernel<true><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(staged, peak, valid, seg,
+                                                                                        mode, out);
+  else
+    segment_stage_i16_kernel<false><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(staged, peak, valid, seg,
+                                                                                         mode, out);
+  HG_CHECK_CUDA(cudaGetLastError());
+  g_hg_launches.fetch_add(1, std::memory_order_relaxed);
+  return HG_OK;
+}
+
+extern "C" int hg_segment_stage_mel(const float* staged, const int* valid_frames, int batch, int fps, int num_mels,
+                                    float* out, void* stream) {
+  HG_REQUIRE(staged && valid_frames && out && batch > 0 && batch <= 65535 && fps > 0 && num_mels > 0 &&
+             (num_mels + 31) / 32 <= 65535, "hg_segment_stage_mel: bad arguments");
+  dim3 grid((fps + 31) / 32, (num_mels + 31) / 32, batch), block(32, 8);
+  segment_stage_mel_kernel<<<grid, block, 0, static_cast<cudaStream_t>(stream)>>>(staged, valid_frames, fps,
+                                                                                  num_mels, out);
   HG_CHECK_CUDA(cudaGetLastError());
   g_hg_launches.fetch_add(1, std::memory_order_relaxed);
   return HG_OK;

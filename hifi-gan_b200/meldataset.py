@@ -175,16 +175,16 @@ def spectral_de_normalize_torch(magnitudes):
     return dynamic_range_decompression_torch(magnitudes)
 
 
+def read_filelist(list_path, wavs_dir):
+    """One `name|text` list file -> wav paths under wavs_dir (reference meldataset.py:88-96)."""
+    import os
+    with open(list_path, 'r', encoding='utf-8') as fi:
+        return [os.path.join(wavs_dir, x.split('|')[0] + '.wav') for x in fi.read().split('\n') if len(x) > 0]
+
+
 def get_dataset_filelist(a):
     """reference meldataset.py:88-96: `name|text` list files -> wav paths under a.input_wavs_dir."""
-    import os
-    with open(a.input_training_file, 'r', encoding='utf-8') as fi:
-        training_files = [os.path.join(a.input_wavs_dir, x.split('|')[0] + '.wav')
-                          for x in fi.read().split('\n') if len(x) > 0]
-    with open(a.input_validation_file, 'r', encoding='utf-8') as fi:
-        validation_files = [os.path.join(a.input_wavs_dir, x.split('|')[0] + '.wav')
-                            for x in fi.read().split('\n') if len(x) > 0]
-    return training_files, validation_files
+    return read_filelist(a.input_training_file, a.input_wavs_dir), read_filelist(a.input_validation_file, a.input_wavs_dir)
 
 
 class MelDataset(torch.utils.data.Dataset):
@@ -336,30 +336,128 @@ class SegmentSampler:
                 picks.append((self.offsets[i], n, self.mel_offsets[i], min(fps, f)))
         return picks
 
-    def _gather_audio(self, starts, valid):
+    def _gather(self, indices, picks):
+        """The [B, seg] audio crops of drawn `picks` (from draw / draw_fine_tuning for utterances `indices`) and, in
+        fine-tuning mode, the [B, num_mels, frames_per_seg] input-mel crops (else None)."""
         seg = self.segment_length
-        starts = torch.tensor(starts, dtype=torch.int64).to(self.device, non_blocking=True)
-        valid = torch.tensor(valid, dtype=torch.int32).to(self.device, non_blocking=True)
+        starts = torch.tensor([p[0] for p in picks], dtype=torch.int64).to(self.device, non_blocking=True)
+        valid = torch.tensor([p[1] for p in picks], dtype=torch.int32).to(self.device, non_blocking=True)
         audio = torch.empty(starts.numel(), seg, dtype=torch.float32, device=self.device)
         _lib.check(_lib.lib().hg_segment_gather(self.pool.data_ptr(), starts.data_ptr(), valid.data_ptr(), starts.numel(),
                                                 seg, audio.data_ptr(), torch.cuda.current_stream().cuda_stream),
                    "hg_segment_gather")
-        return audio
+        if not self.fine_tuning:
+            return audio, None
+        fps = self.frames_per_seg
+        col0 = torch.tensor([p[2] for p in picks], dtype=torch.int64, device=self.device)
+        nval = torch.tensor([p[3] for p in picks], dtype=torch.int64, device=self.device)
+        ar = torch.arange(fps, device=self.device)
+        cols = (col0[:, None] + ar[None, :]).clamp_(max=self.mel_pool.shape[1] - 1)      # [B, fps]
+        mel = self.mel_pool[:, cols].permute(1, 0, 2) * (ar[None, :] < nval[:, None])[:, None, :]   # zero padding
+        return audio, mel.contiguous()
 
     def batch(self, indices):
-        if self.fine_tuning:
-            picks = self.draw_fine_tuning(indices)
-            audio = self._gather_audio([p[0] for p in picks], [p[1] for p in picks])
-            fps = self.frames_per_seg
-            col0 = torch.tensor([p[2] for p in picks], dtype=torch.int64, device=self.device)
-            nval = torch.tensor([p[3] for p in picks], dtype=torch.int64, device=self.device)
-            ar = torch.arange(fps, device=self.device)
-            cols = (col0[:, None] + ar[None, :]).clamp_(max=self.mel_pool.shape[1] - 1)      # [B, fps]
-            mel = self.mel_pool[:, cols].permute(1, 0, 2) * (ar[None, :] < nval[:, None])[:, None, :]   # zero padding
-            mel = mel.contiguous()
-        else:
-            picks = self.draw(indices)
-            audio = self._gather_audio([p[0] for p in picks], [p[1] for p in picks])
+        picks = self.draw_fine_tuning(indices) if self.fine_tuning else self.draw(indices)
+        audio, mel = self._gather(indices, picks)
+        if mel is None:
             mel = mel_spectrogram(audio, *self.mel_args, self.fmax, center=False)
         mel_loss = mel_spectrogram(audio, *self.mel_args, self.fmax_loss, center=False)
         return mel, audio, mel_loss
+
+
+_STAGE_MODES = {"peak": 0, "fork": 1, None: 2}         # HG_STAGE_PEAK / _FORK / _NONE
+
+
+class _StagingSlot:
+    """A pinned host buffer, its device twin, and the event recorded after the last copy out of the host buffer."""
+
+    def __init__(self, nbytes, device):
+        self.host = torch.empty(nbytes, dtype=torch.uint8).pin_memory()
+        self.dev = torch.empty(nbytes, dtype=torch.uint8, device=device)
+        self.copied = None
+
+
+class CorpusSampler(SegmentSampler):
+    """`SegmentSampler` over a packed int16 corpus (`hifigan_b200.corpus.Corpus`) that stays on the host: the same
+    attributes, the same draw rule (`draw` / `draw_fine_tuning`) and the same two mel calls, but only each batch's
+    crops reach the GPU, so the device footprint is O(batch x segment) whatever the corpus size.
+
+    Per batch the host copies the B crops (int16 samples, and in fine-tuning mode the frame-major fp32 mel crops) from
+    the memory-mapped corpus into one of two pinned staging slots, one copy moves the slot to the device, and
+    hg_segment_stage_i16 / hg_segment_stage_mel turn it into exactly the tensors `SegmentSampler` gathers from its
+    in-memory pool over `normalize(read_wav(f) / MAX_WAV_VALUE)`.  An event recorded after each copy guards the slot's
+    reuse, so the host prepares batch i + 1 while the device still works on batch i.
+
+    normalize: 'peak' (train_loop.normalize_peak), 'fork' (normalize_fork) or None (fine-tuning, no normalisation).
+    order: the corpus entries the sampler's utterance indices 0..n-1 stand for (default: all, in file order)."""
+
+    def __init__(self, corpus, segment_length, n_fft, num_mels, hop_size, win_size, sampling_rate, fmin, fmax,
+                 fmax_loss=None, seed=1234, device="cuda", normalize="peak", fine_tuning=False, order=None):
+        if normalize not in _STAGE_MODES:
+            raise ValueError(f"CorpusSampler: normalize must be 'peak', 'fork' or None, not {normalize!r}")
+        if corpus.sampling_rate != sampling_rate:
+            raise ValueError("{} SR doesn't match target {} SR".format(corpus.sampling_rate, sampling_rate))
+        self.corpus = corpus
+        self.device = torch.device(device)
+        self.segment_length = segment_length
+        self.hop_size = hop_size
+        self.num_mels = num_mels
+        self.mel_args = (n_fft, num_mels, sampling_rate, hop_size, win_size, fmin)
+        self.fmax, self.fmax_loss = fmax, fmax_loss
+        self.mode = _STAGE_MODES[normalize]
+        order = list(range(len(corpus))) if order is None else list(order)
+        self.lengths = corpus.lengths[order].tolist()
+        self.offsets = corpus.offsets[order].tolist()          # into corpus.pcm: draw() returns corpus sample offsets
+        self.peaks = corpus.peaks[order].tolist()
+        self.rng = random.Random(seed)
+        self.fine_tuning = fine_tuning
+        if fine_tuning:
+            if corpus.mels is None:
+                raise ValueError(f"CorpusSampler: {corpus.path} holds no fine-tuning mels (pack it with mels_dir)")
+            if corpus.num_mels != num_mels:
+                raise ValueError(f"CorpusSampler: the corpus mels have {corpus.num_mels} bands, not {num_mels}")
+            self.mel_frames = corpus.mel_frames[order].tolist()
+            self.mel_offsets = corpus.mel_offsets[order].tolist()
+            self.frames_per_seg = math.ceil(segment_length / hop_size)
+        self._slots = [None, None]
+        self._next = 0
+
+    def _gather(self, indices, picks):
+        import numpy as np
+        b, seg = len(picks), self.segment_length
+        fps = self.frames_per_seg if self.fine_tuning else 0
+        audio_bytes = (b * seg * 2 + 255) // 256 * 256
+        mel_at = audio_bytes + (3 * b * 4 + 255) // 256 * 256
+        total = mel_at + b * fps * self.num_mels * 4
+        slot = self._slots[self._next]
+        if slot is not None and slot.copied is not None:
+            slot.copied.synchronize()                   # the copy that last read this slot has finished
+        if slot is None or slot.host.numel() < total:
+            slot = self._slots[self._next] = _StagingSlot(total, self.device)
+        self._next ^= 1
+        host = slot.host.numpy()
+        audio_h = host[:b * seg * 2].view(np.int16).reshape(b, seg)
+        meta = host[audio_bytes:audio_bytes + 3 * b * 4].view(np.int32).reshape(3, b)     # valid, peak, valid frames
+        pcm = self.corpus.pcm
+        for j, (i, p) in enumerate(zip(indices, picks)):
+            audio_h[j, :p[1]] = pcm[p[0]:p[0] + p[1]]
+            meta[0, j], meta[1, j] = p[1], self.peaks[i]
+        if self.fine_tuning:
+            mel_h = host[mel_at:total].view(np.float32).reshape(b, fps, self.num_mels)
+            for j, p in enumerate(picks):
+                mel_h[j, :p[3]] = self.corpus.mels[p[2]:p[2] + p[3]]
+                meta[2, j] = p[3]
+        slot.dev[:total].copy_(slot.host[:total], non_blocking=True)
+        slot.copied = torch.cuda.Event()
+        slot.copied.record()
+        st = torch.cuda.current_stream().cuda_stream
+        base = slot.dev.data_ptr()
+        audio = torch.empty(b, seg, dtype=torch.float32, device=self.device)
+        _lib.check(_lib.lib().hg_segment_stage_i16(base, base + audio_bytes + 4 * b, base + audio_bytes, b, seg,
+                                                   self.mode, audio.data_ptr(), st), "hg_segment_stage_i16")
+        if not self.fine_tuning:
+            return audio, None
+        mel = torch.empty(b, self.num_mels, fps, dtype=torch.float32, device=self.device)
+        _lib.check(_lib.lib().hg_segment_stage_mel(base + mel_at, base + audio_bytes + 8 * b, b, fps, self.num_mels,
+                                                   mel.data_ptr(), st), "hg_segment_stage_mel")
+        return audio, mel

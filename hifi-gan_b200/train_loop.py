@@ -17,6 +17,10 @@ What differs from UPSTREAM, deliberately: the DataLoader workers computing mels 
 GPU-resident `SegmentSampler` (the kernels have no CPU path); audio is peak-normalised per utterance to 0.95 (the
 UPSTREAM rule — this fork's `[1, L]` call of librosa.util.normalize normalises per SAMPLE, SURVEY §8a row S);
 TensorBoard scalars are written only if tensorboard is installed.
+
+`--input_corpus PATH` trains from a packed int16 corpus (`hifigan_b200.corpus`, packed from --input_training_file)
+instead of the wav files: it stays on the host and `CorpusSampler` stages each batch's crops to the GPU, with the same
+utterance order, shuffle, crops and values as the in-memory path.  Validation reads its wav files as before.
 """
 from __future__ import annotations
 
@@ -32,7 +36,8 @@ import torch
 
 from . import _lib
 from .env import AttrDict, build_env
-from .meldataset import MAX_WAV_VALUE, SegmentSampler, get_dataset_filelist, mel_spectrogram
+from .corpus import Corpus, utterance_name
+from .meldataset import MAX_WAV_VALUE, CorpusSampler, SegmentSampler, get_dataset_filelist, mel_spectrogram
 from .models import Generator, MultiPeriodDiscriminator, MultiScaleDiscriminator
 from .train import FlatParams, TrainStep, shard_batch
 from .utils import load_checkpoint, save_checkpoint, scan_checkpoint
@@ -143,18 +148,30 @@ def train(rank: int, a, h, local_rank: int = None) -> Dict[str, float]:
         load_optimizer_state_dict(ts.G.flat, g_params, state_dict_do['optim_g'])
         load_optimizer_state_dict(ts.D.flat, d_params, state_dict_do['optim_d'])
 
-    training_files, validation_files = get_dataset_filelist(a)
+    listed, validation_files = get_dataset_filelist(a)
+    order = list(range(len(listed)))
     random.seed(1234)                                                # MelDataset.__init__ (meldataset.py:104-106)
-    random.shuffle(training_files)
+    random.shuffle(order)                                            # the permutation depends on the length only
+    training_files = [listed[k] for k in order]
     # meldataset.py:126-130: `/ MAX_WAV_VALUE` (quirk kept), then peak normalisation unless fine-tuning
-    prep = (lambda a_: a_) if a.fine_tuning else (normalize_fork if getattr(a, "normalize", "peak") == "fork"
-                                                   else normalize_peak)
-    utts = [prep(read_wav(f, h.sampling_rate) / MAX_WAV_VALUE) for f in training_files]
+    normalize = None if a.fine_tuning else getattr(a, "normalize", "peak")
+    prep = {None: lambda a_: a_, "fork": normalize_fork, "peak": normalize_peak}[normalize]
     npy = lambda f: np.load(os.path.join(a.input_mels_dir, os.path.splitext(os.path.split(f)[-1])[0] + '.npy'))
-    sampler = SegmentSampler(utts, h.segment_size, h.n_fft, h.num_mels, h.hop_size, h.win_size, h.sampling_rate, h.fmin,
-                             h.fmax, h.fmax_for_loss, seed=1234 + steps, device=device,   # a resumed run draws new crops
-                             mels=[npy(f) for f in training_files] if a.fine_tuning else None)   # meldataset.py:155-161
-    del utts                                    # the sampler holds the pool on the device; drop the host copy
+    if getattr(a, "input_corpus", None):
+        # the packed int16 corpus stays on the host (page cache); CorpusSampler stages each batch's crops to the GPU
+        corpus = Corpus(a.input_corpus)
+        if corpus.names != [utterance_name(f) for f in listed]:
+            raise ValueError(f"{a.input_corpus} was not packed from {a.input_training_file} (names or order differ)")
+        sampler = CorpusSampler(corpus, h.segment_size, h.n_fft, h.num_mels, h.hop_size, h.win_size, h.sampling_rate,
+                                h.fmin, h.fmax, h.fmax_for_loss, seed=1234 + steps, device=device, normalize=normalize,
+                                fine_tuning=a.fine_tuning, order=order)
+    else:
+        utts = [prep(read_wav(f, h.sampling_rate) / MAX_WAV_VALUE) for f in training_files]
+        sampler = SegmentSampler(utts, h.segment_size, h.n_fft, h.num_mels, h.hop_size, h.win_size, h.sampling_rate,
+                                 h.fmin, h.fmax, h.fmax_for_loss, seed=1234 + steps, device=device,   # a resumed run
+                                 mels=[npy(f) for f in training_files] if a.fine_tuning else None)    # draws new crops
+        # (fine-tuning mels: meldataset.py:155-161)
+        del utts                                # the sampler holds the pool on the device; drop the host copy
     val = [prep(read_wav(f, h.sampling_rate) / MAX_WAV_VALUE) for f in validation_files] if rank == 0 else []
     val_mels = [torch.from_numpy(npy(f)).float() for f in validation_files] if (rank == 0 and a.fine_tuning) else None
     sw = None
@@ -262,6 +279,9 @@ def main(argv=None) -> Dict[str, float]:
     parser.add_argument('--validation_interval', default=1000, type=int)
     parser.add_argument('--fine_tuning', default=False, type=bool)
     parser.add_argument('--normalize', default='peak', choices=['peak', 'fork'])   # see normalize_fork
+    # a corpus packed from --input_training_file (python -m hifigan_b200.corpus): no training wav is read, each batch's
+    # crops are staged from the host instead of the whole corpus living on every GPU
+    parser.add_argument('--input_corpus', default=None)
     a = parser.parse_args(argv)
     with open(a.config) as f:
         h = AttrDict(json.loads(f.read()))

@@ -198,6 +198,24 @@ int hg_loss_sum(const float* a, const float* b, long long n, int mode, float c, 
 int hg_segment_gather(const float* pool, const long long* start, const int* valid, int batch, int seg,
                       float* out, void* stream);
 
+/* Staging of a packed int16 corpus's crops (hifigan_b200.corpus, CorpusSampler): the host copies a batch's crops into
+ * one buffer that moves to the device in one copy; these kernels turn them into what hg_segment_gather produces from
+ * the in-memory fp32 pool, bit for bit.
+ * hg_segment_stage_i16: staged int16 [B][seg] -> out fp32 [B][seg], zero for i >= valid[b].  Sample q of an utterance
+ *   whose peak is peak[b] = max|q| over the whole utterance becomes what the host pipeline q / 32768 (read_wav)
+ *   / 32768 (MAX_WAV_VALUE) followed by the normalisation gives:
+ *     HG_STAGE_PEAK  (q / m) * 0.95f, IEEE division (normalize_peak; m = 0 gives 0)
+ *     HG_STAGE_FORK  sign(q) * 0.95f                (normalize_fork)
+ *     HG_STAGE_NONE  q * 2^-30                      (fine-tuning: no normalisation)
+ *   peak, valid int32 [B].
+ * hg_segment_stage_mel: staged fp32 [B][fps][num_mels] (frame-major fine-tuning mel crops) -> out fp32
+ *   [B][num_mels][fps], zero for frames >= valid_frames[b] (int32 [B]). */
+enum { HG_STAGE_PEAK = 0, HG_STAGE_FORK = 1, HG_STAGE_NONE = 2 };
+int hg_segment_stage_i16(const int16_t* staged, const int* peak, const int* valid, int batch, int seg, int mode,
+                         float* out, void* stream);
+int hg_segment_stage_mel(const float* staged, const int* valid_frames, int batch, int fps, int num_mels, float* out,
+                         void* stream);
+
 /* hg_conv_post_tanh_fwd — conv_post + tanh (src/models.py:113-114).  x bf16 [B][T][C] already
  * holds leaky_relu(., 0.01) (models.py:112, fused into the producer's epilogue).  w fp32 [C][k]
  * (folded weight of the single output channel), y fp32 [B][T] == the reference's [B,1,T].
