@@ -160,10 +160,7 @@ _SIGNATURES = {
     "hg_unpack_wgrad_conv": (c_int, [c_void_p] + [c_int] * 7 + [POINTER(c_int), c_void_p, c_void_p]),
     "hg_wgrad_finish_conv": (c_int, [c_void_p] + [c_int] * 7 + [POINTER(c_int), c_void_p, c_void_p, c_int, c_void_p,
                                                                   c_void_p, c_void_p]),
-    "hg_wgrad_finish_convtr": (c_int, [c_void_p] + [c_int] * 7 + [c_void_p, c_void_p, c_int, c_void_p, c_void_p,
-                                                                    c_void_p]),
     "hg_weight_norm_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
-    "hg_fold_weight_norm": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "hg_pack_disc_weight": (c_int, [c_void_p] + [c_int] * 7 + [c_void_p, c_void_p, c_void_p]),
     "hg_spectral_norm_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
                                      c_void_p, c_void_p, c_void_p]),
@@ -207,7 +204,7 @@ def lib() -> ctypes.CDLL:
                 fn = getattr(handle, name)
                 fn.restype = res
                 fn.argtypes = args
-            if handle.hg_abi_version() != 3:
+            if handle.hg_abi_version() != 4:
                 raise HgError("libhifigan_b200.so ABI mismatch")
             _lib = handle
     return _lib

@@ -1,4 +1,4 @@
-// hg_batched.cu — weight preparation and weight-gradient finishing for MANY layers in one launch.
+// hg_batched.cu — weight preparation and weight-gradient finishing, for one layer or for MANY layers in one launch.
 //
 // The training step re-derives every GEMM-ready filter bank after each optimizer update (weight_norm fold — the
 // reference's hook recomputes w = g * v / ||v|| on every forward, src/models.py:16-31,56-59,81,86-88,96,132-140,196-204 —
@@ -6,9 +6,9 @@
 // layer those are 3-4 tiny launches; a V1 step has ~80 generator convs and ~55 discriminator convs, so they were 650
 // of its 1 300 launches and a fifth of its SM-time.  Here a launch covers a whole network: the host describes each
 // layer once in a device-resident job table (hg_prep_job), a second table maps every block of the grid to
-// (job, block-within-job), and one generic kernel dispatches on the job kind.  The per-row / per-tile arithmetic is
-// the same as in the single-layer kernels (hg_prep.cu, hg_train.cu), which stay as the reference implementations the
-// tests compare against.
+// (job, block-within-job), and one generic kernel dispatches on the job kind.  The job bodies below are the only
+// implementation of these folds, packs and finishes: the single-layer entry points (hg_pack_conv1d_weight,
+// hg_pack_disc_weight, hg_wgrad_finish_conv, ...) fill one job and launch it on its own (hg_prep_launch_one).
 #include "hg_common.cuh"
 
 #include <atomic>
@@ -18,18 +18,6 @@
 extern std::atomic<int64_t> g_hg_launches;
 
 namespace {
-
-__device__ __forceinline__ float block_sum256(float v, float* red) {
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
-  if (l == 0) red[w] = v;
-  __syncthreads();
-  float s = 0.f;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) s += red[i];
-  __syncthreads();
-  return s;
-}
 
 // ---- HG_JOB_GEN_CONV: one block per (padded) output channel --------------------------------------------------
 // v fp32 [cout][cin][k] (+ g [cout]) -> w bf16 [k][cout_p][cin_p]; bias_out[co] = bias[co] (0 for padding rows)
@@ -44,7 +32,7 @@ __device__ void job_gen_conv(const hg_prep_job& j, int co, float* red) {
   if (g && real) {                                   // block-uniform branch
     float ss = 0.f;
     for (int i = threadIdx.x; i < cin * k; i += 256) ss += vc[i] * vc[i];
-    ss = block_sum256(ss, red);
+    ss = hg::block_sum(ss, red);
     scale = ss > 0.f ? g[co] / sqrtf(ss) : 0.f;
   }
   for (int idx = threadIdx.x; idx < k * cin_p; idx += 256) {
@@ -72,7 +60,7 @@ __device__ void job_gen_convtr(const hg_prep_job& j, int ci, float* red) {
   if (g && real) {
     float ss = 0.f;
     for (int i = threadIdx.x; i < cout * k; i += 256) ss += vc[i] * vc[i];
-    ss = block_sum256(ss, red);
+    ss = hg::block_sum(ss, red);
     scale = ss > 0.f ? g[ci] / sqrtf(ss) : 0.f;
   }
   const int n_total = stride * cout_p;
@@ -102,7 +90,7 @@ __device__ void job_gen_post(const hg_prep_job& j, float* red) {
   if (g) {
     float ss = 0.f;
     for (int i = threadIdx.x; i < cin * k; i += 256) ss += v[i] * v[i];
-    ss = block_sum256(ss, red);
+    ss = hg::block_sum(ss, red);
     scale = ss > 0.f ? g[0] / sqrtf(ss) : 0.f;
   }
   float* out = static_cast<float*>(j.dst0);
@@ -122,7 +110,7 @@ __device__ void job_disc_row(const hg_prep_job& j, int co, float* red, float* ro
   if (g) {
     float ss = 0.f;
     for (int i = threadIdx.x; i < n; i += 256) ss += vr[i] * vr[i];
-    ss = block_sum256(ss, red);
+    ss = hg::block_sum(ss, red);
     scale = ss > 0.f ? g[co] / sqrtf(ss) : 0.f;
   }
   float* eff = static_cast<float*>(j.dst0);
@@ -197,9 +185,12 @@ __device__ void job_disc_dgrad_tile(const hg_prep_job& j, int lb, float* sm) {
   }
 }
 
-// ---- HG_JOB_FINISH_ROW: packed weight gradient -> parameter gradients (unpack + weight_norm backward), one block
-// per dim-0 index of the parameter (hg_wgrad_finish_conv / _convtr for many layers at once) --------------------
-__device__ __forceinline__ float packed_dw(const float* __restrict__ p, const hg_prep_job& j, int i0, int i1, int t) {
+// ---- HG_JOB_FINISH_ROW: weight gradient -> parameter gradients (unpack + weight_norm backward), one block per
+// dim-0 index of the parameter.  Modes 0 / 1 gather the row from the packed layout of a conv / polyphase convtr into
+// shared memory tap plane by tap plane (a conv's plane is contiguous along d1, so the reads coalesce; the transposing
+// writes go to shared memory); mode 2 reads a dense [d0][d1 * k] gradient in place.  weight_norm backward (dim 0):
+// dg = <dw, v> / ||v||, dv = g / ||v|| * (dw - v * <dw, v> / ||v||^2); g == NULL: plain weight, dv (+)= dw ---------
+__device__ __forceinline__ float gather_packed(const float* __restrict__ p, const hg_prep_job& j, int i0, int i1, int t) {
   const int mode = j.i[0], d1 = j.i[2], rows_p = j.i[4], cin_tile = j.i[5];
   if (mode == 0) {
     const int cout_g = j.i[6], merge = j.i[7];
@@ -213,38 +204,45 @@ __device__ __forceinline__ float packed_dw(const float* __restrict__ p, const hg
 }
 
 __device__ void job_finish_row(const hg_prep_job& j, int r, float* red, float* sdw) {
-  const int d1 = j.i[2], k = j.i[3], accumulate = j.i[12];
+  const int mode = j.i[0], d1 = j.i[2], k = j.i[3], accumulate = j.i[12];
   const int rest = d1 * k;
   const float* p = static_cast<const float*>(j.src0);
   const float* g = static_cast<const float*>(j.src1);
   const float* vr = static_cast<const float*>(j.src2) + static_cast<size_t>(r) * rest;
   float* o = static_cast<float*>(j.dst0) + static_cast<size_t>(r) * rest;
   float* dg = static_cast<float*>(j.dst1);
-  for (int idx = threadIdx.x; idx < rest; idx += 256) {
-    const int t = idx / d1, i1 = idx - t * d1;
-    sdw[i1 * k + t] = packed_dw(p, j, r, i1, t);
+  const float* dw = sdw;                             // this row's gradient in parameter order [d1][k]
+  if (mode == 2) {                                   // block-uniform
+    dw = p + static_cast<size_t>(r) * rest;
+  } else {
+    for (int idx = threadIdx.x; idx < rest; idx += 256) {
+      const int t = idx / d1, i1 = idx - t * d1;
+      sdw[i1 * k + t] = gather_packed(p, j, r, i1, t);
+    }
+    __syncthreads();
   }
-  __syncthreads();
   if (!g) {
-    for (int i = threadIdx.x; i < rest; i += 256) o[i] = accumulate ? o[i] + sdw[i] : sdw[i];
+    for (int i = threadIdx.x; i < rest; i += 256) o[i] = accumulate ? o[i] + dw[i] : dw[i];
     return;
   }
   float ss = 0.f, dot = 0.f;
   for (int i = threadIdx.x; i < rest; i += 256) {
     const float vv = vr[i];
     ss += vv * vv;
-    dot += vv * sdw[i];
+    dot += vv * dw[i];
   }
-  ss = block_sum256(ss, red);
-  dot = block_sum256(dot, red);
+  ss = hg::block_sum(ss, red);
+  dot = hg::block_sum(dot, red);
   const float nrm = sqrtf(ss);
   const float inv = nrm > 0.f ? 1.f / nrm : 0.f;
   const float gg = g[r];
+  // accumulate: rounded explicitly (the product is never fused into the add, the dg update always is), so the
+  // batched and the single-job kernel, which inline this body in different contexts, give the same bits
   for (int i = threadIdx.x; i < rest; i += 256) {
-    const float val = gg * inv * (sdw[i] - vr[i] * dot * inv * inv);
-    o[i] = accumulate ? o[i] + val : val;
+    const float val = gg * inv * (dw[i] - vr[i] * dot * inv * inv);
+    o[i] = accumulate ? __fadd_rn(o[i], val) : val;
   }
-  if (threadIdx.x == 0) dg[r] = accumulate ? dg[r] + dot * inv : dot * inv;
+  if (threadIdx.x == 0) dg[r] = accumulate ? fmaf(dot, inv, dg[r]) : dot * inv;
 }
 
 // ---- HG_JOB_LOSS_SUM: one block per chunk of a reduction; *dst0 += partial sum (fp32 atomic) ------------------
@@ -276,8 +274,24 @@ __device__ void job_loss_sum(const hg_prep_job& j, int lb, float* red) {
       acc += mode == 0 ? fabsf(d) : d * d;
     }
   }
-  acc = block_sum256(acc, red);
+  acc = hg::block_sum(acc, red);
   if (threadIdx.x == 0) atomicAdd(static_cast<float*>(j.dst0), acc);
+}
+
+// kKind >= 0: the kind is known at compile time and only that body is compiled in
+template <int kKind = -1>
+__device__ __forceinline__ void run_job(const hg_prep_job& j, int lb, float* red, float* dyn) {
+  switch (kKind < 0 ? j.kind : kKind) {              // block-uniform
+    case HG_JOB_GEN_CONV: job_gen_conv(j, lb, red); break;
+    case HG_JOB_GEN_CONVTR: job_gen_convtr(j, lb, red); break;
+    case HG_JOB_GEN_POST: job_gen_post(j, red); break;
+    case HG_JOB_DISC_ROW: job_disc_row(j, lb, red, dyn); break;
+    case HG_JOB_TRANSPOSE_TILE: job_transpose_tile(j, lb, dyn); break;
+    case HG_JOB_DISC_DGRAD_TILE: job_disc_dgrad_tile(j, lb, dyn); break;
+    case HG_JOB_FINISH_ROW: job_finish_row(j, lb, red, dyn); break;
+    case HG_JOB_LOSS_SUM: job_loss_sum(j, lb, red); break;
+    default: break;
+  }
 }
 
 __global__ void __launch_bounds__(256)
@@ -285,18 +299,29 @@ prep_batched_kernel(const hg_prep_job* __restrict__ jobs, const int2* __restrict
   extern __shared__ __align__(16) float dyn[];
   __shared__ float red[8];
   const int2 bj = block_job[blockIdx.x];
-  const hg_prep_job& j = jobs[bj.x];
-  switch (j.kind) {                                  // block-uniform
-    case HG_JOB_GEN_CONV: job_gen_conv(j, bj.y, red); break;
-    case HG_JOB_GEN_CONVTR: job_gen_convtr(j, bj.y, red); break;
-    case HG_JOB_GEN_POST: job_gen_post(j, red); break;
-    case HG_JOB_DISC_ROW: job_disc_row(j, bj.y, red, dyn); break;
-    case HG_JOB_TRANSPOSE_TILE: job_transpose_tile(j, bj.y, dyn); break;
-    case HG_JOB_DISC_DGRAD_TILE: job_disc_dgrad_tile(j, bj.y, dyn); break;
-    case HG_JOB_FINISH_ROW: job_finish_row(j, bj.y, red, dyn); break;
-    case HG_JOB_LOSS_SUM: job_loss_sum(j, bj.y, red); break;
-    default: break;
-  }
+  run_job(jobs[bj.x], bj.y, red, dyn);
+}
+
+// One job of kind kKind, block b = block b of the job.  __grid_constant__: the job is read from the parameter space in
+// place; a by-value parameter bound to the job bodies' const reference would be copied into a local-memory frame per
+// thread.  One instantiation per kind: with every body inlined the kernel needs 40 registers (6 blocks of 256 threads
+// per SM), with one body 32 (8 blocks), so a 1 024-row discriminator finish runs as one wave on 148 SMs.
+template <int kKind>
+__global__ void __launch_bounds__(256) prep_one_kernel(const __grid_constant__ hg_prep_job j) {
+  extern __shared__ __align__(16) float dyn[];
+  __shared__ float red[8];
+  run_job<kKind>(j, blockIdx.x, red, dyn);
+}
+
+template <int kKind>
+int launch_one(const hg_prep_job& job, int nblocks, int smem_bytes, void* stream) {
+  static hg::PerDeviceOnce once;
+  if (smem_bytes > 48 * 1024 && once.need(static_cast<size_t>(smem_bytes)))
+    HG_CHECK_CUDA(cudaFuncSetAttribute(prep_one_kernel<kKind>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       kPrepMaxSmem));
+  prep_one_kernel<kKind><<<nblocks, 256, smem_bytes, static_cast<cudaStream_t>(stream)>>>(job);
+  HG_CHECK_CUDA(cudaGetLastError());
+  return HG_OK;
 }
 
 }  // namespace
@@ -305,14 +330,30 @@ extern "C" int hg_prep_job_size(void) { return static_cast<int>(sizeof(hg_prep_j
 
 extern "C" int hg_prep_batched(const hg_prep_job* jobs, const int* block_job, int first_block, int nblocks,
                                int smem_bytes, void* stream) {
-  HG_REQUIRE(jobs && block_job && first_block >= 0 && nblocks > 0 && smem_bytes >= 0 && smem_bytes <= 96 * 1024,
+  HG_REQUIRE(jobs && block_job && first_block >= 0 && nblocks > 0 && smem_bytes >= 0 && smem_bytes <= kPrepMaxSmem,
              "hg_prep_batched: bad arguments");
   static hg::PerDeviceOnce once;
   if (smem_bytes > 48 * 1024 && once.need(static_cast<size_t>(smem_bytes)))
-    HG_CHECK_CUDA(cudaFuncSetAttribute(prep_batched_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
+    HG_CHECK_CUDA(cudaFuncSetAttribute(prep_batched_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPrepMaxSmem));
   prep_batched_kernel<<<nblocks, 256, smem_bytes, static_cast<cudaStream_t>(stream)>>>(
       jobs, reinterpret_cast<const int2*>(block_job) + first_block);
   HG_CHECK_CUDA(cudaGetLastError());
+  g_hg_launches.fetch_add(1, std::memory_order_relaxed);
+  return HG_OK;
+}
+
+int hg_prep_launch_one(const hg_prep_job& job, int nblocks, int smem_bytes, void* stream) {
+  int rc;
+  switch (job.kind) {
+    case HG_JOB_GEN_CONV: rc = launch_one<HG_JOB_GEN_CONV>(job, nblocks, smem_bytes, stream); break;
+    case HG_JOB_GEN_CONVTR: rc = launch_one<HG_JOB_GEN_CONVTR>(job, nblocks, smem_bytes, stream); break;
+    case HG_JOB_DISC_ROW: rc = launch_one<HG_JOB_DISC_ROW>(job, nblocks, smem_bytes, stream); break;
+    case HG_JOB_TRANSPOSE_TILE: rc = launch_one<HG_JOB_TRANSPOSE_TILE>(job, nblocks, smem_bytes, stream); break;
+    case HG_JOB_DISC_DGRAD_TILE: rc = launch_one<HG_JOB_DISC_DGRAD_TILE>(job, nblocks, smem_bytes, stream); break;
+    case HG_JOB_FINISH_ROW: rc = launch_one<HG_JOB_FINISH_ROW>(job, nblocks, smem_bytes, stream); break;
+    default: HG_REQUIRE(false, "hg_prep_launch_one: no single-job kernel for job kind %d", job.kind);
+  }
+  if (rc) return rc;
   g_hg_launches.fetch_add(1, std::memory_order_relaxed);
   return HG_OK;
 }

@@ -347,6 +347,20 @@ __device__ __forceinline__ float warp_colsum(float (&v)[N], int lane, int& col) 
   return v[0];
 }
 
+// Sum of v over a 256-thread block, valid in every thread; red: >= 8 floats of shared memory.  The eight warp sums
+// are added in warp order, so a block's result does not depend on scheduling.
+__device__ __forceinline__ float block_sum(float v, float* red) {
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
+  if (l == 0) red[w] = v;
+  __syncthreads();
+  float s = 0.f;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) s += red[i];
+  __syncthreads();
+  return s;
+}
+
 // cudaFuncSetAttribute is per DEVICE: launchers remember, per device ordinal, whether (or with which size) they
 // already raised a kernel's dynamic shared-memory limit.  One process may drive several GPUs.
 struct PerDeviceOnce {
@@ -366,3 +380,10 @@ struct PerDeviceOnce {
 int hg_encode_tmap_bf16_3d(CUtensorMap* out, const void* base, uint64_t d0, uint64_t d1, uint64_t d2,
                            uint64_t stride1_bytes, uint64_t stride2_bytes, uint32_t box0,
                            uint32_t box1, uint32_t box2, int swizzle_bytes);
+
+// host-side: runs ONE weight-preparation job (include/hifigan_b200.h, hg_prep_batched) as its own launch of `nblocks`
+// blocks, block b being block b of the job; smem_bytes <= kPrepMaxSmem.  Counts one launch.  The single-layer entry
+// points (hg_pack_*, hg_wgrad_finish_conv, hg_unpack_wgrad_conv, hg_weight_norm_bwd) run through this.
+struct hg_prep_job;
+constexpr int kPrepMaxSmem = 96 * 1024;
+int hg_prep_launch_one(const hg_prep_job& job, int nblocks, int smem_bytes, void* stream);

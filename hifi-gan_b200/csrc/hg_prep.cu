@@ -1,5 +1,6 @@
 // hg_prep.cu — bandwidth-bound helpers around the implicit-GEMM conv:
-//   * weight_norm fold + GEMM-ready bf16 packing (Conv1d and polyphase ConvTranspose1d)
+//   * weight_norm fold + GEMM-ready bf16 packing (Conv1d and polyphase ConvTranspose1d), run as one job of
+//     hg_batched.cu
 //   * [B][C][T] fp32 <-> [B][T][C] bf16 layout edges
 //   * conv_post + tanh (src/models.py:113-114)
 #include "hg_common.cuh"
@@ -11,64 +12,6 @@
 extern std::atomic<int64_t> g_hg_launches;
 
 namespace {
-
-__device__ __forceinline__ float block_sum(float v, float* red) {
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  const int w = threadIdx.x >> 5, l = threadIdx.x & 31, nw = (blockDim.x + 31) >> 5;
-  if (l == 0) red[w] = v;
-  __syncthreads();
-  float s = 0.f;
-  for (int i = 0; i < nw; ++i) s += red[i];
-  __syncthreads();
-  return s;
-}
-
-// one block per output channel: w[co] = g[co] * v[co] / ||v[co]||  ->  out[j][co][ci]
-__global__ void pack_conv1d_weight_kernel(const float* __restrict__ v, const float* __restrict__ g,
-                                          int cout, int cin, int k, int cin_pad,
-                                          __nv_bfloat16* __restrict__ out) {
-  __shared__ float red[32];
-  const int co = blockIdx.x;
-  const float* vc = v + static_cast<size_t>(co) * cin * k;
-  float scale = 1.f;
-  if (g) {
-    float ss = 0.f;
-    for (int i = threadIdx.x; i < cin * k; i += blockDim.x) ss += vc[i] * vc[i];
-    ss = block_sum(ss, red);
-    scale = ss > 0.f ? g[co] / sqrtf(ss) : 0.f;  // all-zero rows only exist as channel padding
-  }
-  for (int j = 0; j < k; ++j) {
-    __nv_bfloat16* o = out + (static_cast<size_t>(j) * cout + co) * cin_pad;
-    for (int ci = threadIdx.x; ci < cin_pad; ci += blockDim.x)
-      o[ci] = __float2bfloat16(ci < cin ? vc[ci * k + j] * scale : 0.f);
-  }
-}
-
-// one block per input channel (weight_norm dim 0 of ConvTranspose1d): polyphase scatter
-__global__ void pack_convtr1d_weight_kernel(const float* __restrict__ v, const float* __restrict__ g,
-                                            int cin, int cout, int k, int stride, int padding,
-                                            int nshift, int shift_min,
-                                            __nv_bfloat16* __restrict__ out) {
-  __shared__ float red[32];
-  const int ci = blockIdx.x;
-  const float* vc = v + static_cast<size_t>(ci) * cout * k;
-  float scale = 1.f;
-  if (g) {
-    float ss = 0.f;
-    for (int i = threadIdx.x; i < cout * k; i += blockDim.x) ss += vc[i] * vc[i];
-    ss = block_sum(ss, red);
-    scale = ss > 0.f ? g[ci] / sqrtf(ss) : 0.f;
-  }
-  const int n_total = stride * cout;
-  for (int idx = threadIdx.x; idx < nshift * n_total; idx += blockDim.x) {
-    const int s = idx / n_total;
-    const int n = idx % n_total;
-    const int p = n / cout, co = n % cout;
-    const int j = p + padding - (shift_min + s) * stride;
-    const float w = (j >= 0 && j < k) ? vc[co * k + j] * scale : 0.f;
-    out[(static_cast<size_t>(s) * n_total + n) * cin + ci] = __float2bfloat16(w);
-  }
-}
 
 // fp32 [B][C][T] -> bf16 [B][T][c_pad]; 32x32 smem transpose tiles
 __global__ void ncl_to_nlc_kernel(const float* __restrict__ x, int c, int t, int c_pad,
@@ -316,7 +259,7 @@ loss_sum_kernel(const float* __restrict__ a, const float* __restrict__ b, long l
     const float d = mode == 0 ? a[i] - b[i] : c - a[i];
     acc += mode == 0 ? fabsf(d) : d * d;
   }
-  acc = block_sum(acc, red);
+  acc = hg::block_sum(acc, red);
   if (threadIdx.x == 0) atomicAdd(out, acc);
 }
 
@@ -397,11 +340,12 @@ extern "C" int hg_pack_conv1d_weight(const float* v, const float* g, int cout, i
                                      int cin_pad, void* w_packed, void* stream) {
   HG_REQUIRE(v && w_packed, "hg_pack_conv1d_weight: null pointer");
   HG_REQUIRE(cout > 0 && cin > 0 && k > 0 && cin_pad >= cin, "hg_pack_conv1d_weight: bad shape");
-  pack_conv1d_weight_kernel<<<cout, 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      v, g, cout, cin, k, cin_pad, static_cast<__nv_bfloat16*>(w_packed));
-  HG_CHECK_CUDA(cudaGetLastError());
-  g_hg_launches.fetch_add(1, std::memory_order_relaxed);
-  return HG_OK;
+  hg_prep_job j{};
+  j.kind = HG_JOB_GEN_CONV;
+  j.src0 = v; j.src1 = g; j.dst0 = w_packed;
+  const int ints[] = {cout, cin, k, cout, cin_pad};
+  for (int n = 0; n < 5; ++n) j.i[n] = ints[n];
+  return hg_prep_launch_one(j, cout, 0, stream);
 }
 
 extern "C" int hg_convtr1d_geometry(int k, int stride, int padding, int* host_nshift,
@@ -422,12 +366,12 @@ extern "C" int hg_pack_convtr1d_weight(const float* v, const float* g, int cin, 
   int nshift = 0, shift_min = 0;
   int rc = hg_convtr1d_geometry(k, stride, padding, &nshift, &shift_min);
   if (rc) return rc;
-  pack_convtr1d_weight_kernel<<<cin, 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      v, g, cin, cout, k, stride, padding, nshift, shift_min,
-      static_cast<__nv_bfloat16*>(w_packed));
-  HG_CHECK_CUDA(cudaGetLastError());
-  g_hg_launches.fetch_add(1, std::memory_order_relaxed);
-  return HG_OK;
+  hg_prep_job j{};
+  j.kind = HG_JOB_GEN_CONVTR;
+  j.src0 = v; j.src1 = g; j.dst0 = w_packed;
+  const int ints[] = {cin, cout, k, cin, cout, stride, padding, nshift, shift_min};
+  for (int n = 0; n < 9; ++n) j.i[n] = ints[n];
+  return hg_prep_launch_one(j, cin, 0, stream);
 }
 
 extern "C" int hg_ncl_to_nlc(const float* x, int batch, int c, int t, int c_pad, void* out,

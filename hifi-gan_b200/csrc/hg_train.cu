@@ -1,11 +1,12 @@
 // hg_train.cu — the bandwidth-bound pieces of the training step (UPSTREAM train.py restated in SURVEY.md §3.3;
 // every op below is what torch autograd / torch.optim would run for the reference's src/models.py modules):
-//   * dgrad weight packing (tap flip + filter transpose), bias gradients (column sums)
+//   * bias gradients (column sums)
 //   * conv_post + tanh backward (src/models.py:112-114), the Cin = 1 / Cout = 1 discriminator ends' backward
 //     (src/models.py:134,141,146-151,196,204), AvgPool1d(4,2,2) backward (:227-230)
 //   * loss gradients (src/models.py:251-282 + the mel L1), L1 sums over internal bf16 feature maps
-//   * unpacking of hg_conv1d_wgrad results to the parameter layout, weight_norm backward
-//     (torch._weight_norm_interface_backward; reparametrisation at src/models.py:16-31,81,86-88,96,132-140)
+//   * the single-layer weight preparation and weight-gradient finishes (dgrad / discriminator packs, unpacking of
+//     hg_conv1d_wgrad results to the parameter layout, weight_norm backward = torch._weight_norm_interface_backward;
+//     reparametrisation at src/models.py:16-31,81,86-88,96,132-140): one job of hg_batched.cu each
 //   * AdamW (torch.optim.AdamW semantics, decoupled weight decay), and the gradient norm of
 //     torch.nn.utils.clip_grad_norm_ with the skip of a non-finite step that guards it
 #include "hg_common.cuh"
@@ -25,32 +26,7 @@ __device__ __forceinline__ float warp_sum(float v) {
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
 }
-__device__ __forceinline__ float block_sum(float v, float* red) {
-  v = warp_sum(v);
-  const int w = threadIdx.x >> 5, l = threadIdx.x & 31, nw = (blockDim.x + 31) >> 5;
-  if (l == 0) red[w] = v;
-  __syncthreads();
-  float s = 0.f;
-  for (int i = 0; i < nw; ++i) s += red[i];
-  __syncthreads();
-  return s;
-}
 __device__ __forceinline__ float sgn(float d) { return d > 0.f ? 1.f : (d < 0.f ? -1.f : 0.f); }
-
-// bf16 [k][n][c] -> bf16 [k][c][n] with the taps reversed: the filter bank of the data gradient
-__global__ void pack_dgrad_kernel(const __nv_bfloat16* __restrict__ w, int k, int n, int c,
-                                  __nv_bfloat16* __restrict__ out) {
-  __shared__ __nv_bfloat16 tile[32][33];
-  const int j = blockIdx.z;
-  const int c0 = blockIdx.x * 32, n0 = blockIdx.y * 32;
-  const int tx = threadIdx.x, ty = threadIdx.y;
-  for (int i = ty; i < 32; i += 8)
-    if (n0 + i < n && c0 + tx < c) tile[i][tx] = w[(static_cast<size_t>(j) * n + n0 + i) * c + c0 + tx];
-  __syncthreads();
-  for (int i = ty; i < 32; i += 8)
-    if (c0 + i < c && n0 + tx < n)
-      out[(static_cast<size_t>(k - 1 - j) * c + c0 + i) * n + n0 + tx] = tile[tx][i];
-}
 
 // out[c] (+)= sum over (b, t < t_valid) of x[b][t][c];  x bf16 [B][t_rows][C]
 // thread = (row lane, 8-channel vector); a block reduces its rows in registers, then across row lanes through
@@ -175,7 +151,7 @@ conv_post_bwd_dw_kernel(const __nv_bfloat16* __restrict__ x, const float* __rest
     bsum += v;
   }
   __syncthreads();
-  bsum = block_sum(bsum, red);
+  bsum = hg::block_sum(bsum, red);
   if (threadIdx.x == 0 && db) atomicAdd(db, bsum);
   for (int idx = threadIdx.x; idx < c * k; idx += blockDim.x) {
     const int j = idx / c, cc = idx % c;             // adjacent threads read adjacent channels
@@ -464,113 +440,6 @@ __global__ void loss_grad_kernel(const float* __restrict__ a, const float* __res
   }
 }
 
-struct UnpackArgs {
-  int mode;          // 0: Conv1d, 1: ConvTranspose1d (polyphase)
-  int d0, d1, k;     // parameter shape [d0][d1][k]  (conv: cout, cin/groups; convtr: cin, cout)
-  int rows_p;        // rows of the packed tensor per tap (cout_p, or stride * cout_p)
-  int cin_tile;      // inner dimension of the packed tensor
-  int cout_g, merge; // conv: output channels per group, groups merged per tile
-  int stride, padding, shift_min, cout_p;   // convtr
-  int pos[64];       // conv: packed position of original tap j
-};
-
-// packed fp32 [taps][rows_p][cin_tile] -> dense parameter-layout gradient [d0][d1][k]
-__global__ void unpack_wgrad_kernel(const float* __restrict__ p, const UnpackArgs a, float* __restrict__ dw) {
-  const long long n = static_cast<long long>(a.d0) * a.d1 * a.k;
-  for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n; i += 256LL * gridDim.x) {
-    const int j = static_cast<int>(i % a.k);
-    const int i1 = static_cast<int>((i / a.k) % a.d1);
-    const int i0 = static_cast<int>(i / (static_cast<long long>(a.k) * a.d1));
-    float v;
-    if (a.mode == 0) {
-      const int slot = (i0 / a.cout_g) % a.merge;
-      v = p[(static_cast<size_t>(a.pos[j]) * a.rows_p + i0) * a.cin_tile + slot * a.d1 + i1];
-    } else {
-      const int ph = (((j - a.padding) % a.stride) + a.stride) % a.stride;
-      const int s = (ph + a.padding - j) / a.stride - a.shift_min;
-      v = p[(static_cast<size_t>(s) * a.rows_p + ph * a.cout_p + i1) * a.cin_tile + i0];
-    }
-    dw[i] = v;
-  }
-}
-
-__device__ __forceinline__ float packed_dw(const float* __restrict__ p, const UnpackArgs& a, int i0, int i1, int j) {
-  if (a.mode == 0) {
-    const int slot = (i0 / a.cout_g) % a.merge;
-    return p[(static_cast<size_t>(a.pos[j]) * a.rows_p + i0) * a.cin_tile + slot * a.d1 + i1];
-  }
-  const int ph = (((j - a.padding) % a.stride) + a.stride) % a.stride;
-  const int s = (ph + a.padding - j) / a.stride - a.shift_min;
-  return p[(static_cast<size_t>(s) * a.rows_p + ph * a.cout_p + i1) * a.cin_tile + i0];
-}
-
-// packed weight gradient -> parameter gradients in ONE pass (unpack + weight_norm backward): one block per dim-0
-// index.  g == NULL: plain weight, dv (+)= dw.  Results are ADDED to dv / dg when accumulate != 0.
-__global__ void __launch_bounds__(256)
-wgrad_finish_kernel(const float* __restrict__ p, const UnpackArgs a, const float* __restrict__ v,
-                    const float* __restrict__ g, int accumulate, float* __restrict__ dv, float* __restrict__ dg) {
-  extern __shared__ float sdw[];                 // this row's gradient in parameter order [d1][k]
-  __shared__ float red[32];
-  const int r = blockIdx.x;
-  const int rest = a.d1 * a.k;
-  const float* vr = v + static_cast<size_t>(r) * rest;
-  float* o = dv + static_cast<size_t>(r) * rest;
-  // gather tap plane by tap plane: the packed layout is contiguous along d1 inside a plane (conv), so the reads
-  // coalesce; the transposing writes go to shared memory (stride k words)
-  for (int idx = threadIdx.x; idx < rest; idx += blockDim.x) {
-    const int j = idx / a.d1, i1 = idx - j * a.d1;
-    sdw[i1 * a.k + j] = packed_dw(p, a, r, i1, j);
-  }
-  __syncthreads();
-  if (!g) {
-    for (int i = threadIdx.x; i < rest; i += blockDim.x) o[i] = accumulate ? o[i] + sdw[i] : sdw[i];
-    return;
-  }
-  float ss = 0.f, dot = 0.f;
-  for (int i = threadIdx.x; i < rest; i += blockDim.x) {
-    const float vv = vr[i];
-    ss += vv * vv;
-    dot += vv * sdw[i];
-  }
-  ss = block_sum(ss, red);
-  dot = block_sum(dot, red);
-  const float nrm = sqrtf(ss);
-  const float inv = nrm > 0.f ? 1.f / nrm : 0.f;
-  const float gg = g[r];
-  for (int i = threadIdx.x; i < rest; i += blockDim.x) {
-    const float val = gg * inv * (sdw[i] - vr[i] * dot * inv * inv);
-    o[i] = accumulate ? o[i] + val : val;
-  }
-  if (threadIdx.x == 0) dg[r] = accumulate ? dg[r] + dot * inv : dot * inv;
-}
-
-// weight_norm backward (dim 0): w = g * v / ||v||;  dg = <dw, v> / ||v||;  dv = g/||v|| * (dw - v * <dw,v>/||v||^2)
-// one block per dim-0 index; dv, dg are ACCUMULATED into (+=) when accumulate != 0
-__global__ void __launch_bounds__(256)
-weight_norm_bwd_kernel(const float* __restrict__ dw, const float* __restrict__ v, const float* __restrict__ g,
-                       int rest, int accumulate, float* __restrict__ dv, float* __restrict__ dg) {
-  __shared__ float red[32];
-  const int r = blockIdx.x;
-  const float* vr = v + static_cast<size_t>(r) * rest;
-  const float* dr = dw + static_cast<size_t>(r) * rest;
-  float ss = 0.f, dot = 0.f;
-  for (int i = threadIdx.x; i < rest; i += blockDim.x) {
-    ss += vr[i] * vr[i];
-    dot += vr[i] * dr[i];
-  }
-  ss = block_sum(ss, red);
-  dot = block_sum(dot, red);
-  const float nrm = sqrtf(ss);
-  const float inv = nrm > 0.f ? 1.f / nrm : 0.f;
-  const float gg = g[r];
-  float* o = dv + static_cast<size_t>(r) * rest;
-  for (int i = threadIdx.x; i < rest; i += blockDim.x) {
-    const float val = gg * inv * (dr[i] - vr[i] * dot * inv * inv);
-    o[i] = accumulate ? o[i] + val : val;
-  }
-  if (threadIdx.x == 0) dg[r] = accumulate ? dg[r] + dot * inv : dot * inv;
-}
-
 // torch.optim.AdamW step on one flat fp32 tensor.  kGuard: the clip_grad_norm_ / non-finite-skip flavour — nothing
 // is written when *skip is set, otherwise the gradient scale is multiplied by *clip_coef (hg_grad_norm_finalize).
 // The guard arguments come last so the unguarded instantiation keeps its parameter offsets.
@@ -601,53 +470,12 @@ __global__ void adamw_kernel(float* __restrict__ p, const float* __restrict__ g,
   }
 }
 
-// w_eff[r][:] = g[r] * v[r][:] / ||v[r]||   (weight_norm fold, fp32; g == NULL copies)
-__global__ void __launch_bounds__(256)
-fold_weight_kernel(const float* __restrict__ v, const float* __restrict__ g, int rest, float* __restrict__ out) {
-  __shared__ float red[32];
-  const int r = blockIdx.x;
-  const float* vr = v + static_cast<size_t>(r) * rest;
-  float scale = 1.f;
-  if (g) {
-    float ss = 0.f;
-    for (int i = threadIdx.x; i < rest; i += blockDim.x) ss += vr[i] * vr[i];
-    ss = block_sum(ss, red);
-    scale = ss > 0.f ? g[r] / sqrtf(ss) : 0.f;
-  }
-  for (int i = threadIdx.x; i < rest; i += blockDim.x) out[static_cast<size_t>(r) * rest + i] = vr[i] * scale;
-}
-
-struct DiscPackArgs {
-  int cout, cin_g, k, merge, cout_g, cin_tile;      // forward pack
-  int cin, groups, stride, pad, nshift, shift_min, cout_tile;   // dgrad pack
-  int order[64];
-};
-
-// forward pack: fp32 [cout][cin_g][k] -> bf16 [q][cout][cin_tile] (taps in kernel order, groups merged block-diagonally)
-// One block per output channel: its [cin_g][k] row is read once, coalesced, into shared memory; every tap plane is
-// then written as one contiguous run of cin_tile bf16 values (two per thread).
-__global__ void __launch_bounds__(256)
-pack_disc_fwd_kernel(const float* __restrict__ w, const DiscPackArgs a, __nv_bfloat16* __restrict__ out) {
-  extern __shared__ float row[];
-  const int co = blockIdx.x;
-  const int n = a.cin_g * a.k;
-  const float* wr = w + static_cast<size_t>(co) * n;
-  for (int i = threadIdx.x; i < n; i += 256) row[i] = wr[i];
-  __syncthreads();
-  const int lo = ((co / a.cout_g) % a.merge) * a.cin_g;       // this channel's slot inside the merged group tile
-  const int half = a.cin_tile >> 1;
-  for (int idx = threadIdx.x; idx < a.k * half; idx += 256) {
-    const int q = idx / half, ct = (idx - q * half) * 2;
-    const int cl = ct - lo, tap = a.order[q];
-    const float v0 = (cl >= 0 && cl < a.cin_g) ? row[cl * a.k + tap] : 0.f;
-    const float v1 = (cl + 1 >= 0 && cl + 1 < a.cin_g) ? row[(cl + 1) * a.k + tap] : 0.f;
-    *reinterpret_cast<uint32_t*>(out + (static_cast<size_t>(q) * a.cout + co) * a.cin_tile + ct) = hg::pack_bf16x2(v0, v1);
-  }
-}
-
 // dgrad (polyphase) pack: fp32 [cout][cin_g][k] -> bf16 [m][rho * cin + ci][cc], cc = dy channel inside the
 // (merged) group tile of ci;  j = rho + pad - stride * (m + shift_min)
-// Generic form (one thread per output element); used when a layer's shape does not tile.
+// One thread per output element; used when a layer's shape does not tile (HG_JOB_DISC_DGRAD_TILE covers the others).
+struct DiscPackArgs {
+  int cin_g, k, merge, cout_g, cin, stride, pad, nshift, shift_min, cout_tile;
+};
 __global__ void pack_disc_dgrad_kernel(const float* __restrict__ w, const DiscPackArgs a, __nv_bfloat16* __restrict__ out) {
   const long long n = static_cast<long long>(a.nshift) * a.stride * a.cin * a.cout_tile;
   for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n; i += 256LL * gridDim.x) {
@@ -664,39 +492,6 @@ __global__ void pack_disc_dgrad_kernel(const float* __restrict__ w, const DiscPa
     out[i] = __float2bfloat16(v);
   }
 }
-// Tiled form: a block owns [tci input channels of one group] x [32 dy channels].  The 32 source runs (tci * k
-// contiguous floats each) are read coalesced into shared memory (odd pitch); every (shift, phase) plane is then
-// written as 64-byte runs along cc, two bf16 per thread, conflict-free.
-__global__ void __launch_bounds__(256)
-pack_disc_dgrad_tiled_kernel(const float* __restrict__ w, const DiscPackArgs a, int tci, __nv_bfloat16* __restrict__ out) {
-  extern __shared__ float sm[];                               // [32][tci * k + 1]
-  const int ci0 = blockIdx.x * tci, cc0 = blockIdx.y * 32;
-  const int g = ci0 / a.cin_g, cil0 = ci0 - g * a.cin_g;
-  const int co_base = (g / a.merge) * a.cout_tile + cc0;
-  const int run = tci * a.k, pitch = run + 1;
-  for (int idx = threadIdx.x; idx < 32 * run; idx += 256) {
-    const int ccl = idx / run, r = idx - ccl * run;
-    const int co = co_base + ccl;
-    sm[ccl * pitch + r] = (co / a.cout_g == g) ? w[(static_cast<size_t>(co) * a.cin_g + cil0) * a.k + r] : 0.f;
-  }
-  __syncthreads();
-  const int planes = a.nshift * a.stride;
-  for (int idx = threadIdx.x; idx < planes * tci * 16; idx += 256) {
-    const int cc2 = (idx & 15) * 2;
-    const int t = idx >> 4;
-    const int ms = t / tci, cil = t - ms * tci;
-    const int m = ms / a.stride, rho = ms - m * a.stride;
-    const int j = rho + a.pad - a.stride * (m + a.shift_min);
-    float v0 = 0.f, v1 = 0.f;
-    if (j >= 0 && j < a.k) {
-      v0 = sm[cc2 * pitch + cil * a.k + j];
-      v1 = sm[(cc2 + 1) * pitch + cil * a.k + j];
-    }
-    *reinterpret_cast<uint32_t*>(out + (static_cast<size_t>(ms) * a.cin + ci0 + cil) * a.cout_tile + cc0 + cc2) =
-        hg::pack_bf16x2(v0, v1);
-  }
-}
-
 // ---- spectral norm (torch.nn.utils.spectral_norm, dim 0, one power iteration, eps 1e-12; src/models.py:194) ----
 // K1: t[j] += sum_{i in row chunk} W[i][j] * u[i]            (W^T u, rows split over blockIdx.y, t zeroed before)
 __global__ void __launch_bounds__(256)
@@ -718,7 +513,7 @@ sn_wv_kernel(const float* __restrict__ w, const float* __restrict__ t, float* __
   if (iterate) {
     float ss = 0.f;
     for (int j = threadIdx.x; j < cols; j += 256) ss += t[j] * t[j];
-    ss = block_sum(ss, red);
+    ss = hg::block_sum(ss, red);
     inv = 1.f / fmaxf(sqrtf(ss), eps);
   }
   const float* src = iterate ? t : v;
@@ -748,7 +543,7 @@ sn_scale_kernel(const float* __restrict__ w, const float* __restrict__ s, float*
   if (iterate) {
     float ss = 0.f;
     for (int i = threadIdx.x; i < rows; i += 256) ss += s[i] * s[i];
-    ss = block_sum(ss, red);
+    ss = hg::block_sum(ss, red);
     const float inv = 1.f / fmaxf(sqrtf(ss), eps);
     sigma = ss * inv;
     if (blockIdx.x == 0)
@@ -760,7 +555,7 @@ sn_scale_kernel(const float* __restrict__ w, const float* __restrict__ s, float*
   } else {
     float d = 0.f;
     for (int i = threadIdx.x; i < rows; i += 256) d += u[i] * s[i];
-    sigma = block_sum(d, red);
+    sigma = hg::block_sum(d, red);
     if (blockIdx.x == 0 && u_copy)
       for (int i = threadIdx.x; i < rows; i += 256) u_copy[i] = u[i];
   }
@@ -774,7 +569,7 @@ sn_bwd_dot_kernel(const float* __restrict__ d, const float* __restrict__ w_eff, 
   __shared__ float red[32];
   float a = 0.f;
   for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n; i += 256LL * gridDim.x) a += d[i] * w_eff[i];
-  a = block_sum(a, red);
+  a = hg::block_sum(a, red);
   if (threadIdx.x == 0) atomicAdd(dot, a);
 }
 __global__ void __launch_bounds__(256)
@@ -870,6 +665,20 @@ grad_norm_finalize_kernel(const double* __restrict__ partial, int nslots, float 
   }
 }
 
+// HG_JOB_FINISH_ROW mode 0 for a conv's packed gradient [k][rows_p][cin_tile]; tab[packed position] = original tap
+hg_prep_job finish_conv_job(const float* dw_packed, int cout, int cin_g, int k, int rows_p, int cin_tile, int cout_g,
+                            int merge, const int* host_tap_order, const float* v, const float* g, int accumulate,
+                            float* dv, float* dg) {
+  hg_prep_job j{};
+  j.kind = HG_JOB_FINISH_ROW;
+  j.src0 = dw_packed; j.src1 = g; j.src2 = v; j.dst0 = dv; j.dst1 = dg;
+  const int ints[] = {0, cout, cin_g, k, rows_p, cin_tile, cout_g, merge};
+  for (int q = 0; q < 8; ++q) j.i[q] = ints[q];
+  j.i[12] = accumulate;
+  for (int q = 0; q < k; ++q) j.tab[host_tap_order ? host_tap_order[q] : q] = q;
+  return j;
+}
+
 int blocks_for(long long n, int per = 256) {
   long long b = (n + per - 1) / per;
   if (b > 148 * 16) b = 148 * 16;
@@ -880,12 +689,13 @@ int blocks_for(long long n, int per = 256) {
 
 extern "C" int hg_pack_dgrad_weight(const void* w_packed, int ktaps, int n, int c, void* out, void* stream) {
   HG_REQUIRE(w_packed && out && ktaps > 0 && n > 0 && c > 0 && ktaps <= 65535, "hg_pack_dgrad_weight: bad arguments");
-  dim3 grid((c + 31) / 32, (n + 31) / 32, ktaps), block(32, 8);
-  pack_dgrad_kernel<<<grid, block, 0, S(stream)>>>(static_cast<const __nv_bfloat16*>(w_packed), ktaps, n, c,
-                                                    static_cast<__nv_bfloat16*>(out));
-  HG_CHECK_CUDA(cudaGetLastError());
-  count();
-  return HG_OK;
+  hg_prep_job j{};
+  j.kind = HG_JOB_TRANSPOSE_TILE;
+  j.src0 = w_packed; j.dst0 = out;
+  const int tiles_c = (c + 31) / 32, tiles_n = (n + 31) / 32;
+  const int ints[] = {ktaps, n, c, tiles_c, tiles_n};
+  for (int q = 0; q < 5; ++q) j.i[q] = ints[q];
+  return hg_prep_launch_one(j, ktaps * tiles_c * tiles_n, 32 * 34 * 2, stream);
 }
 
 extern "C" int hg_colsum_bf16(const void* x, int batch, int t_valid, int t_rows, int c, int accumulate, float* out,
@@ -1006,23 +816,21 @@ extern "C" int hg_unpack_wgrad_conv(const float* dw_packed, int cout, int cin_g,
                                     int cout_g, int merge, const int* host_tap_order, float* dw, void* stream) {
   HG_REQUIRE(dw_packed && dw && k > 0 && k <= 64 && cout > 0 && cin_g > 0 && merge >= 1 && cout_g >= 1,
              "hg_unpack_wgrad_conv: bad arguments");
-  UnpackArgs a{};
-  a.mode = 0; a.d0 = cout; a.d1 = cin_g; a.k = k; a.rows_p = rows_p; a.cin_tile = cin_tile;
-  a.cout_g = cout_g; a.merge = merge;
-  for (int q = 0; q < k; ++q) a.pos[host_tap_order ? host_tap_order[q] : q] = q;
-  unpack_wgrad_kernel<<<blocks_for(static_cast<long long>(cout) * cin_g * k), 256, 0, S(stream)>>>(dw_packed, a, dw);
-  HG_CHECK_CUDA(cudaGetLastError());
-  count();
-  return HG_OK;
+  HG_REQUIRE(static_cast<size_t>(cin_g) * k * 4 <= kPrepMaxSmem, "hg_unpack_wgrad_conv: row of %d values does not fit",
+             cin_g * k);
+  const hg_prep_job j = finish_conv_job(dw_packed, cout, cin_g, k, rows_p, cin_tile, cout_g, merge, host_tap_order,
+                                        nullptr, nullptr, 0, dw, nullptr);
+  return hg_prep_launch_one(j, cout, cin_g * k * 4, stream);
 }
 
 extern "C" int hg_weight_norm_bwd(const float* dw, const float* v, const float* g, int dim0, int rest, int accumulate,
                                   float* dv, float* dg, void* stream) {
   HG_REQUIRE(dw && v && g && dv && dg && dim0 > 0 && rest > 0, "hg_weight_norm_bwd: bad arguments");
-  weight_norm_bwd_kernel<<<dim0, 256, 0, S(stream)>>>(dw, v, g, rest, accumulate, dv, dg);
-  HG_CHECK_CUDA(cudaGetLastError());
-  count();
-  return HG_OK;
+  hg_prep_job j{};
+  j.kind = HG_JOB_FINISH_ROW;
+  j.src0 = dw; j.src1 = g; j.src2 = v; j.dst0 = dv; j.dst1 = dg;
+  j.i[0] = 2; j.i[1] = dim0; j.i[2] = rest; j.i[3] = 1; j.i[12] = accumulate;
+  return hg_prep_launch_one(j, dim0, 0, stream);
 }
 
 extern "C" int hg_adamw_step(float* p, const float* g, float* m, float* v, long long n, float lr, float beta1,
@@ -1075,46 +883,47 @@ extern "C" int hg_grad_norm_finalize(const double* partials, int nslots, float m
   return HG_OK;
 }
 
-extern "C" int hg_fold_weight_norm(const float* v, const float* g, int dim0, int rest, float* w_eff, void* stream) {
-  HG_REQUIRE(v && w_eff && dim0 > 0 && rest > 0, "hg_fold_weight_norm: bad arguments");
-  fold_weight_kernel<<<dim0, 256, 0, S(stream)>>>(v, g, rest, w_eff);
-  HG_CHECK_CUDA(cudaGetLastError());
-  count();
-  return HG_OK;
-}
-
 extern "C" int hg_pack_disc_weight(const float* w_eff, int cout, int cin, int groups, int merge, int k, int stride,
                                    int pad, void* w_fwd, void* w_dgrad, void* stream) {
   HG_REQUIRE(w_eff && (w_fwd || w_dgrad), "hg_pack_disc_weight: null pointer");
   HG_REQUIRE(cout > 0 && cin > 0 && groups >= 1 && merge >= 1 && groups % merge == 0 && k >= 1 && k <= 64 && stride >= 1,
              "hg_pack_disc_weight: bad arguments");
   DiscPackArgs a{};
-  a.cout = cout; a.cin = cin; a.groups = groups; a.merge = merge; a.k = k; a.stride = stride; a.pad = pad;
+  a.cin = cin; a.merge = merge; a.k = k; a.stride = stride; a.pad = pad;
   a.cin_g = cin / groups; a.cout_g = cout / groups;
-  a.cin_tile = a.cin_g * merge; a.cout_tile = a.cout_g * merge;
-  int rc = hg_conv1d_tap_order(k, stride, pad, a.order);
+  a.cout_tile = a.cout_g * merge;
+  const int cin_tile = a.cin_g * merge;
+  hg_prep_job j{};
+  int rc = hg_conv1d_tap_order(k, stride, pad, j.tab);
   if (rc) return rc;
   rc = hg_convtr1d_geometry(k, stride, pad, &a.nshift, &a.shift_min);
   if (rc) return rc;
   if (w_fwd) {
     const size_t smem = static_cast<size_t>(a.cin_g) * k * sizeof(float);
-    HG_REQUIRE(smem <= 48 * 1024 && a.cin_tile % 2 == 0, "hg_pack_disc_weight: filter row does not fit (cin/groups * k = %d)",
+    HG_REQUIRE(smem <= 48 * 1024 && cin_tile % 2 == 0, "hg_pack_disc_weight: filter row does not fit (cin/groups * k = %d)",
                a.cin_g * k);
-    pack_disc_fwd_kernel<<<cout, 256, smem, S(stream)>>>(w_eff, a, static_cast<__nv_bfloat16*>(w_fwd));
-    HG_CHECK_CUDA(cudaGetLastError());
-    count();
+    j.kind = HG_JOB_DISC_ROW;
+    j.src0 = w_eff; j.dst1 = w_fwd;                  // src1 (g) NULL: w_eff is the weight, scaled by 1
+    const int ints[] = {cout, a.cin_g, k, merge, a.cout_g, cin_tile};
+    for (int q = 0; q < 6; ++q) j.i[q] = ints[q];
+    rc = hg_prep_launch_one(j, cout, static_cast<int>(smem), stream);
+    if (rc) return rc;
   }
   if (w_dgrad) {
     int tci = k <= 10 ? 32 : 8;
     while (tci > 2 && (a.cin_g % tci || cin % tci)) tci >>= 1;
     const size_t smem = 32 * (static_cast<size_t>(tci) * k + 1) * sizeof(float);
     if (a.cin_g % tci == 0 && cin % tci == 0 && a.cout_tile % 32 == 0 && smem <= 48 * 1024) {
-      dim3 grid(cin / tci, a.cout_tile / 32);
-      pack_disc_dgrad_tiled_kernel<<<grid, 256, smem, S(stream)>>>(w_eff, a, tci, static_cast<__nv_bfloat16*>(w_dgrad));
-    } else {
-      pack_disc_dgrad_kernel<<<blocks_for(static_cast<long long>(a.nshift) * stride * cin * a.cout_tile), 256, 0,
-                               S(stream)>>>(w_eff, a, static_cast<__nv_bfloat16*>(w_dgrad));
+      hg_prep_job d{};
+      d.kind = HG_JOB_DISC_DGRAD_TILE;
+      d.src0 = w_eff; d.dst0 = w_dgrad;
+      const int ints[] = {cout, a.cin_g, k, merge, a.cout_g, cin, stride, pad, a.nshift, a.shift_min, a.cout_tile,
+                          tci, cin / tci};
+      for (int q = 0; q < 13; ++q) d.i[q] = ints[q];
+      return hg_prep_launch_one(d, (cin / tci) * (a.cout_tile / 32), static_cast<int>(smem), stream);
     }
+    pack_disc_dgrad_kernel<<<blocks_for(static_cast<long long>(a.nshift) * stride * cin * a.cout_tile), 256, 0,
+                             S(stream)>>>(w_eff, a, static_cast<__nv_bfloat16*>(w_dgrad));
     HG_CHECK_CUDA(cudaGetLastError());
     count();
   }
@@ -1162,38 +971,15 @@ extern "C" int hg_spectral_norm_bwd(const float* dw_eff, const float* w_eff, con
   return HG_OK;
 }
 
-// hg_wgrad_finish_*: the packed-gradient unpack + hg_weight_norm_bwd fused (one launch per layer).  v, g: the module's
-// weight_v / weight_g (g == NULL: plain `weight`, dv receives the unpacked gradient).
+// hg_wgrad_finish_conv: the packed-gradient unpack + hg_weight_norm_bwd fused (one launch per layer).  v, g: the
+// module's weight_v / weight_g (g == NULL: plain `weight`, dv receives the unpacked gradient).
 extern "C" int hg_wgrad_finish_conv(const float* dw_packed, int cout, int cin_g, int k, int rows_p, int cin_tile,
                                     int cout_g, int merge, const int* host_tap_order, const float* v, const float* g,
                                     int accumulate, float* dv, float* dg, void* stream) {
   HG_REQUIRE(dw_packed && v && dv && (!g || dg) && k > 0 && k <= 64 && cout > 0 && cin_g > 0 && merge >= 1 && cout_g >= 1,
              "hg_wgrad_finish_conv: bad arguments");
-  UnpackArgs a{};
-  a.mode = 0; a.d0 = cout; a.d1 = cin_g; a.k = k; a.rows_p = rows_p; a.cin_tile = cin_tile;
-  a.cout_g = cout_g; a.merge = merge;
-  for (int q = 0; q < k; ++q) a.pos[host_tap_order ? host_tap_order[q] : q] = q;
   HG_REQUIRE(static_cast<size_t>(cin_g) * k * 4 <= 48 * 1024, "hg_wgrad_finish_conv: row of %d values does not fit", cin_g * k);
-  wgrad_finish_kernel<<<cout, 256, static_cast<size_t>(cin_g) * k * 4, S(stream)>>>(dw_packed, a, v, g, accumulate, dv, dg);
-  HG_CHECK_CUDA(cudaGetLastError());
-  count();
-  return HG_OK;
-}
-
-extern "C" int hg_wgrad_finish_convtr(const float* dw_packed, int cin, int cout, int k, int stride, int padding,
-                                      int cin_p, int cout_p, const float* v, const float* g, int accumulate,
-                                      float* dv, float* dg, void* stream) {
-  HG_REQUIRE(dw_packed && v && dv && (!g || dg) && k > 0 && cin > 0 && cout > 0 && stride > 0,
-             "hg_wgrad_finish_convtr: bad arguments");
-  int nshift = 0, smin = 0;
-  int rc = hg_convtr1d_geometry(k, stride, padding, &nshift, &smin);
-  if (rc) return rc;
-  UnpackArgs a{};
-  a.mode = 1; a.d0 = cin; a.d1 = cout; a.k = k; a.rows_p = stride * cout_p; a.cin_tile = cin_p;
-  a.stride = stride; a.padding = padding; a.shift_min = smin; a.cout_p = cout_p;
-  HG_REQUIRE(static_cast<size_t>(cout) * k * 4 <= 48 * 1024, "hg_wgrad_finish_convtr: row of %d values does not fit", cout * k);
-  wgrad_finish_kernel<<<cin, 256, static_cast<size_t>(cout) * k * 4, S(stream)>>>(dw_packed, a, v, g, accumulate, dv, dg);
-  HG_CHECK_CUDA(cudaGetLastError());
-  count();
-  return HG_OK;
+  const hg_prep_job j = finish_conv_job(dw_packed, cout, cin_g, k, rows_p, cin_tile, cout_g, merge, host_tap_order,
+                                        v, g, accumulate, dv, dg);
+  return hg_prep_launch_one(j, cout, cin_g * k * 4, stream);
 }

@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define HG_ABI_VERSION 3
+#define HG_ABI_VERSION 4
 
 /* Library identity / diagnostics. */
 const char* hg_version(void);
@@ -313,20 +313,17 @@ int hg_conv1d_wgrad(const void* x, const void* dy, int batch, int t_in_rows, int
 
 /* Packed weight gradient -> parameter layout: dw fp32 [cout][cin_g][k] from [k][rows_p][cin_tile]
  * (host_tap_order = hg_conv1d_tap_order or NULL for identity; merge = groups merged per block-diagonal tile,
- * cout_g = output channels per original group). */
+ * cout_g = output channels per original group).  A row of cin_g * k floats is staged in shared memory: at most
+ * 24 576 values (96 KB). */
 int hg_unpack_wgrad_conv(const float* dw_packed, int cout, int cin_g, int k, int rows_p, int cin_tile, int cout_g,
                          int merge, const int* host_tap_order, float* dw, void* stream);
 
-/* hg_wgrad_finish_conv / _convtr — the unpack to parameter layout and hg_weight_norm_bwd in ONE launch per layer:
- * packed weight gradient -> (weight_v.grad, weight_g.grad), or -> weight.grad when g == NULL.  conv: the layout of
- * hg_unpack_wgrad_conv; convtr: dw [cin][cout][k] from the polyphase [nshift][stride*cout_p][cin_p].  Added to the
- * existing values when accumulate != 0. */
+/* hg_wgrad_finish_conv — the unpack to parameter layout and hg_weight_norm_bwd in ONE launch per layer: packed
+ * weight gradient (the layout of hg_unpack_wgrad_conv; cin_g * k <= 12 288) -> (weight_v.grad, weight_g.grad), or
+ * -> weight.grad when g == NULL.  Added to the existing values when accumulate != 0. */
 int hg_wgrad_finish_conv(const float* dw_packed, int cout, int cin_g, int k, int rows_p, int cin_tile, int cout_g,
                          int merge, const int* host_tap_order, const float* v, const float* g, int accumulate,
                          float* dv, float* dg, void* stream);
-int hg_wgrad_finish_convtr(const float* dw_packed, int cin, int cout, int k, int stride, int padding, int cin_p,
-                           int cout_p, const float* v, const float* g, int accumulate, float* dv, float* dg,
-                           void* stream);
 
 /* hg_weight_norm_bwd — backward of w = g * v / ||v|| (norm over all dims but 0): dw, v fp32 [dim0][rest],
  * g fp32 [dim0] -> dv, dg (added to the existing values when accumulate != 0). */
@@ -334,12 +331,10 @@ int hg_weight_norm_bwd(const float* dw, const float* v, const float* g, int dim0
                        float* dv, float* dg, void* stream);
 
 /* Discriminator weight preparation (replaces torch.nn.utils.weight_norm's per-forward recompute for
- * src/models.py:132-141,194-204).  hg_fold_weight_norm: w_eff fp32 [dim0][rest] = g * v / ||v|| (g == NULL copies).
- * hg_pack_disc_weight: w_eff fp32 [cout][cin/groups][k] -> w_fwd bf16 [k][cout][cin_tile] (taps in
+ * src/models.py:132-141,194-204).  hg_pack_disc_weight: w_eff fp32 [cout][cin/groups][k] -> w_fwd bf16 [k][cout][cin_tile] (taps in
  * hg_conv1d_tap_order order, `merge` adjacent groups merged into one block-diagonal tile) for
  * hg_conv1d_general_fwd, and / or w_dgrad bf16 [nshift][stride*cin][cout_tile] (polyphase data-gradient filter
  * bank, geometry of hg_convtr1d_geometry(k, stride, pad)) for hg_conv1d_dgrad. */
-int hg_fold_weight_norm(const float* v, const float* g, int dim0, int rest, float* w_eff, void* stream);
 int hg_pack_disc_weight(const float* w_eff, int cout, int cin, int groups, int merge, int k, int stride, int pad,
                         void* w_fwd, void* w_dgrad, void* stream);
 
@@ -358,7 +353,8 @@ int hg_spectral_norm_bwd(const float* dw_eff, const float* w_eff, const float* u
  * Batched weight preparation / weight-gradient finishing: ONE launch for many layers.
  *
  * The per-layer entry points above (hg_pack_conv1d_weight, hg_pack_convtr1d_weight, hg_pack_dgrad_weight,
- * hg_fold_weight_norm, hg_pack_disc_weight, hg_wgrad_finish_conv / _convtr) cost one launch per layer and call; a
+ * hg_pack_disc_weight, hg_wgrad_finish_conv, hg_unpack_wgrad_conv, hg_weight_norm_bwd) each run ONE of the jobs below
+ * in a launch of its own: one launch per layer and call; a
  * training step re-derives ~135 filter banks after every optimizer update (the reference's weight_norm hook recomputes
  * w = g * v / ||v|| on every forward, src/models.py:16-31,56-59,81,86-88,96,132-140,196-204).  hg_prep_batched runs any
  * mix of those per-layer jobs in one grid: `jobs` is a device array of hg_prep_job, `block_job` a device array of
@@ -384,10 +380,13 @@ int hg_spectral_norm_bwd(const float* dw_eff, const float* w_eff, const float* u
  *                          effective weight fp32 -> dst0 bf16 [nshift][stride*cin][cout_tile] (hg_pack_disc_weight's
  *                          w_dgrad).  i = {cout, cin_g, k, merge, cout_g, cin, stride, pad, nshift, shift_min, cout_tile,
  *                          tci, cin / tci}; blocks = (cin / tci) * (cout_tile / 32)
- *   HG_JOB_FINISH_ROW      one block per dim-0 index of the parameter; smem d1 * k floats.  src0 packed dW fp32, src1 g
- *                          (NULL: plain weight), src2 v -> dst0 dv, dst1 dg (hg_wgrad_finish_conv / _convtr).
- *                          i = {mode (0 conv, 1 convtr), d0, d1, k, rows_p, cin_tile, cout_g, merge, stride, padding,
- *                          shift_min, cout_p, accumulate}, tab = packed position of tap j (conv)
+ *   HG_JOB_FINISH_ROW      one block per dim-0 index of the parameter; smem d1 * k floats (mode 2: none).  src0 dW
+ *                          fp32, src1 g (NULL: plain weight), src2 v -> dst0 dv, dst1 dg (hg_wgrad_finish_conv,
+ *                          hg_unpack_wgrad_conv, hg_weight_norm_bwd).  Mode 0: dW packed like a conv's forward bank
+ *                          [k][rows_p][cin_tile]; 1: polyphase convtr [nshift][stride*cout_p][cin_p]; 2: dense, already in
+ *                          parameter layout [d0][d1 * k] and read in place (no row-size limit).
+ *                          i = {mode, d0, d1, k, rows_p, cin_tile, cout_g, merge, stride, padding, shift_min, cout_p,
+ *                          accumulate}, tab = packed position of tap j (mode 0)
  *   HG_JOB_LOSS_SUM        one block per `chunk` elements: *dst0 += partial sum (the reductions of hg_loss_sum and
  *                          of the bf16 feature maps, for many tensors at once).  src0 a, src1 b.  i = {mode (0: fp32
  *                          |a - b|, 1: fp32 (c - a)^2, 2: bf16 |a - b| counted in 16-byte groups), n low 32 bits,

@@ -126,7 +126,7 @@ def test_losses_have_no_cpu_path():
 
 
 # ------------------------------------------------------------------------------------------- C-ABI surface
-def test_library_exports_every_declared_symbol_at_abi_3():
+def test_library_exports_every_declared_symbol_at_abi_4():
     header = open(os.path.join(ROOT, "include", "hifigan_b200.h")).read()
     declared = set(re.findall(r"\b(hg_[a-z0-9_]+)\s*\(", header))
     declared -= {"hg_mel_plan"}
@@ -134,10 +134,22 @@ def test_library_exports_every_declared_symbol_at_abi_3():
     for name in sorted(declared):
         assert hasattr(lib, name), f"{name} declared in include/hifigan_b200.h but not exported"
     assert declared == set(_lib.EXPORTED_SYMBOLS)
-    # ABI 3 dropped these entry points (ABI 2 had them)
-    for name in ("hg_set_cta_limit", "hg_unpack_wgrad_convtr", "hg_l1_sum_bf16"):
+    # ABI 3 dropped the first three entry points (ABI 2 had them), ABI 4 the last two
+    for name in ("hg_set_cta_limit", "hg_unpack_wgrad_convtr", "hg_l1_sum_bf16", "hg_fold_weight_norm",
+                 "hg_wgrad_finish_convtr"):
         assert not hasattr(lib, name), f"{name} is still exported"
-    assert _lib.lib().hg_abi_version() == 3
+    assert _lib.lib().hg_abi_version() == 4
+
+
+def test_unpack_wgrad_rejects_a_row_larger_than_shared_memory():
+    """hg_unpack_wgrad_conv stages one [cin_g][k] row in shared memory (at most 96 KB): a larger row is refused
+    before anything reaches the device."""
+    from ctypes import c_int
+    L = _lib.lib()
+    order = (c_int * 41)(*range(41))
+    fake = 256                      # never dereferenced: the check comes first
+    assert L.hg_unpack_wgrad_conv(fake, 8, 600, 41, 8, 600, 8, 1, order, fake, None) != 0
+    assert b"hg_unpack_wgrad_conv: row of 24600 values does not fit" in L.hg_last_error()
 
 
 def test_convtr_geometry():
